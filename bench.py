@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the path-refinement hot path (BASELINE.json metric: waypoint FK+Jac+collision+LM evals/s).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config 5, SURVEY.md 8d): synthetic P = 8192 candidate paths x T = 300 waypoints of the 8-dof Fetch, the four
@@ -49,7 +49,14 @@ def parse():
     ap.add_argument("--chunks", type=int, default=0, help="path chunks (streams) of the pipelined LM iterations (0: ResidentPipeline's choice)")
     ap.add_argument("--cpu-sample-paths", type=int, default=24)
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (rank 0's shard; see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU path: use it with --impl ours")
+    return args
 
 
 class ClockSampler(threading.Thread):
@@ -290,6 +297,43 @@ def workload_config(args, n_gpus):
     }
 
 
+DUMP_BYTES = 60_000_000  # --dump-outputs stays under 64 MB: past that, a sample of the paths drawn with a fixed seed
+
+
+def dump_outputs(out_dir, x_out, metrics, best, P, T, D):
+    """What a caller of the timed path receives from its last step, as .npy files in `out_dir`:
+    x_out.npy [n, T, D] float32 refined joint paths and path_metrics.npy [n, 8] float32 (the per-path metrics the
+    cost argmin ranks, ops.METRIC_NAMES + tag) of n paths - all P, or a sorted sample drawn with seed 0 when they do not
+    fit DUMP_BYTES -, path_index.npy [n] float64 which paths those are, and argmin.npy float64 [cost, global index,
+    n_valid, valid, trajectory length] of the argmin over all paths.  The timed path computes sign-only metrics: its
+    min_self / min_env columns are the exact minimum distance when negative and an unspecified non-negative value
+    (+inf when every capsule pair was culled) otherwise, so they are written as min(d, 0): 0 = no collision, else the
+    exact depth.  The inputs are seeded, so two builds can be compared file by file.  Every array is written; the names
+    of those holding a NaN or inf are returned (and reported on stderr and in the result line)."""
+    import numpy as np
+    from cppflow_b200.ops import METRIC_NAMES
+
+    n = min(P, DUMP_BYTES // ((T * D + metrics.shape[1]) * 4))
+    idx = np.arange(P) if n == P else np.sort(np.random.default_rng(0).choice(P, n, replace=False))
+    sel = torch.from_numpy(idx).to(x_out.device)
+    path_metrics = metrics.index_select(0, sel)
+    for col in (METRIC_NAMES.index("min_self"), METRIC_NAMES.index("min_env")):
+        path_metrics[:, col].clamp_(max=0.0)
+    arrays = {
+        "x_out": x_out.view(P, T, D).index_select(0, sel).cpu().numpy(),
+        "path_metrics": path_metrics.cpu().numpy(),
+        "path_index": idx.astype(np.float64),
+        "argmin": np.array([best.cost, best.global_index, best.n_valid, best.valid, best.trajectory_length], np.float64),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    non_finite = [name for name, a in arrays.items() if not np.isfinite(a).all()]
+    if non_finite:
+        print(f"--dump-outputs: the timed path produced NaN or inf in {non_finite}", file=sys.stderr)
+    return non_finite
+
+
 # ------------------------------------------------------------------------------------------------------------------
 
 
@@ -414,11 +458,16 @@ def main():
     sampler = ClockSampler(physical_gpu_index(local_rank), period=float(os.environ.get("BENCH_CLOCK_PERIOD", "0.005")))
     sampler.start()
     ms_total, pending = time_pipeline(rpipe, x0, x_out, steps, barrier, metrics, argmin_tail)
+    timed_outputs = (x_out.clone(), metrics.clone()) if args.dump_outputs and rank == 0 else None
     # a 20-step region is ~10 ms: keep the sampler running over a few more identical regions so that it sees load
     for _ in range(3):
         time_pipeline(rpipe, x0, x_out, steps, barrier, metrics, argmin_tail)
     clocks = sampler.stop()
     best = pending.result()
+    dumped = None
+    if timed_outputs is not None:
+        dumped = {"dir": args.dump_outputs, "non_finite": dump_outputs(args.dump_outputs, *timed_outputs, best, P, T, D)}
+        del timed_outputs
     ms_total = max_over_ranks(ms_total)
     ms_per_step = ms_total / steps
     value = world * evals_per_step / (ms_per_step * 1e-3)
@@ -467,7 +516,7 @@ def main():
     with numa_local(dev):
         out_hosts = [torch.empty_like(x_host).pin_memory() for _ in range(pipe.depth)]
     out_host = out_hosts[0]
-    e2e_steps = max(3, min(steps, 20))
+    e2e_steps = steps
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     for i in range(2 * pipe.depth):
         pipe.refine_async(x_host, out_hosts[i % pipe.depth])
@@ -526,7 +575,7 @@ def main():
     del d_in, d_out
 
     # ---- the same iteration on ONE stream (assembly and solve back to back), for comparison
-    n_single = max(5, min(steps, 100))
+    n_single = steps
     barrier()
     e0.record()
     for _ in range(n_single):
@@ -536,7 +585,7 @@ def main():
     ms_single = e0.elapsed_time(e1) / n_single
 
     # ---- per-kernel durations (live, CUDA events on the launching stream) for the roofline
-    n_prof = max(5, min(steps, 50))
+    n_prof = steps
     ev = [[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(n_prof)]
     ws = ops._workspace(dev, lib.cppflow_lm_full_workspace_bytes(rid, P, T), "lm_full")
     cu, tc, no = ops._obs(ob)
@@ -785,6 +834,8 @@ def main():
                    "note": "headline workload: the reference joint path runs through a cuboid, so no path can be valid; "
                            "invalid paths are ranked by trajectory length (see `quality` for the feasible variant)"},
     }
+    if dumped is not None:
+        line["dump_outputs"] = dumped
     emit(line)
     if world > 1:
         dist.destroy_process_group()

@@ -1,19 +1,22 @@
 """The drop-in boundary (SURVEY.md 8b): every hot-path name keeps the reference's signature.
 
-The real `/root/reference/cppflow` is imported in a subprocess with jrl / klampt / ikflow / matplotlib stubbed (the
-stubs of tests/golden/make_golden.py) and `inspect.signature` of each boundary function is compared with the repo's:
-the reference's parameters must come first, in the same order, with the same names and defaults; anything the repo adds
+`tests/golden/reference_signatures.json` holds the reference's side: the parameters of each boundary function and the
+fields of each boundary dataclass of jstmn/cppflow (regenerated from a checkout of it by
+tests/golden/make_golden_signatures.py).  `inspect.signature` of the repo's functions is compared with it: the
+reference's parameters must come first, in the same order, with the same names and defaults; anything the repo adds
 (e.g. `mesh_validator=`, `native=`) must be optional.  Dataclasses of the boundary must have the reference's fields in
-the reference's order.  Skipped where /root/reference does not exist (the GPU box)."""
+the reference's order."""
+import dataclasses
+import importlib
+import inspect
 import json
+import numbers
 import os
-import subprocess
-import sys
 
 import pytest
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REFERENCE = "/root/reference"
+GOLDEN = os.path.join(REPO, "tests", "golden", "reference_signatures.json")
 
 FUNCTIONS = [  # (module, qualified name)
     ("search", "dp_search"), ("search", "joint_limit_almost_violations_3d"),
@@ -32,12 +35,6 @@ DATACLASSES = [
     ("data_types", "PlannerSettings"), ("data_types", "TimingData"),
 ]
 
-_SCRIPT = r'''
-import dataclasses, importlib, inspect, json, sys
-sys.path.insert(0, %(repo)r); sys.path.insert(0, %(repo)r + "/tests/golden")
-import make_golden as MG
-MG.install_stubs()
-import cppflow  # the real reference package
 
 def resolve(mod, qual):
     obj = importlib.import_module(mod)
@@ -45,32 +42,39 @@ def resolve(mod, qual):
         obj = getattr(obj, part)
     return obj
 
-def params(fn):
+
+def describe_params(fn):
+    """[name, kind, has default, repr of the default, the default as a number (numeric defaults only)] per parameter;
+    numeric defaults compare by value, so that a numpy scalar and a float of the same value agree whatever their repr."""
     out = []
     for p in inspect.signature(fn).parameters.values():
-        d = None if p.default is inspect._empty else repr(p.default)
-        out.append([p.name, str(p.kind), p.default is not inspect._empty, d])
+        has = p.default is not inspect.Parameter.empty
+        num = float(p.default) if has and isinstance(p.default, numbers.Real) and not isinstance(p.default, bool) else None
+        out.append([p.name, str(p.kind), has, repr(p.default) if has else None, num])
     return out
 
-res = {"functions": {}, "dataclasses": {}}
-for mod, qual in %(functions)r:
-    res["functions"][mod + "." + qual] = [params(resolve("cppflow." + mod, qual)), params(resolve("cppflow_b200." + mod, qual))]
-for mod, qual in %(dataclasses)r:
-    ref, ours = resolve("cppflow." + mod, qual), resolve("cppflow_b200." + mod, qual)
-    res["dataclasses"][mod + "." + qual] = [[f.name for f in dataclasses.fields(ref)], [f.name for f in dataclasses.fields(ours)]]
-print("RESULT" + json.dumps(res))
-'''
+
+def _same_default(r, o):
+    if r[4] is not None and o[4] is not None:
+        return r[4] == o[4]
+    return r[3] == o[3]
 
 
 @pytest.fixture(scope="module")
 def signatures():
-    if not os.path.isdir(os.path.join(REFERENCE, "cppflow")):
-        pytest.skip("/root/reference is not available here")
-    code = _SCRIPT % dict(repo=REPO, functions=FUNCTIONS, dataclasses=DATACLASSES)
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
-    assert out.returncode == 0, out.stderr[-2000:]
-    line = [l for l in out.stdout.splitlines() if l.startswith("RESULT")][-1]
-    return json.loads(line[len("RESULT"):])
+    with open(GOLDEN) as f:
+        ref = json.load(f)
+    assert sorted(ref["functions"]) == sorted(f"{m}.{q}" for m, q in FUNCTIONS)
+    assert sorted(ref["dataclasses"]) == sorted(f"{m}.{q}" for m, q in DATACLASSES)
+    res = {"functions": {}, "dataclasses": {}}
+    for mod, qual in FUNCTIONS:
+        name = f"{mod}.{qual}"
+        res["functions"][name] = [ref["functions"][name]["params"], describe_params(resolve("cppflow_b200." + mod, qual))]
+    for mod, qual in DATACLASSES:
+        name = f"{mod}.{qual}"
+        ours = [f.name for f in dataclasses.fields(resolve("cppflow_b200." + mod, qual))]
+        res["dataclasses"][name] = [ref["dataclasses"][name]["fields"], ours]
+    return res
 
 
 def test_function_signatures_keep_the_reference_prefix(signatures):
@@ -84,7 +88,7 @@ def test_function_signatures_keep_the_reference_prefix(signatures):
                 problems.append(f"{name}: parameter {i} is '{o[0]}', the reference calls it '{r[0]}'")
             elif r[2] != o[2] and r[2]:
                 problems.append(f"{name}: '{r[0]}' has a default in the reference, none here")
-            elif r[2] and o[2] and r[3] != o[3]:
+            elif r[2] and o[2] and not _same_default(r, o):
                 problems.append(f"{name}: default of '{r[0]}' is {o[3]}, the reference has {r[3]}")
         for o in ours[len(ref):]:
             if not o[2] and "VAR_" not in o[1]:
