@@ -104,6 +104,29 @@ class LmLoopJobC(C.Structure):
     ]
 
 
+class FlowDescC(C.Structure):
+    """cppflow_flow_desc"""
+
+    _fields_ = [
+        ("robot", C.c_int32),
+        ("width", C.c_int32),
+        ("ndof", C.c_int32),
+        ("dim_cond", C.c_int32),
+        ("nb_nodes", C.c_int32),
+        ("coeff_fn_config", C.c_int32),
+        ("coeff_fn_internal_size", C.c_int32),
+        ("rnvp_clamp", C.c_float),
+        ("d_w_in", C.c_void_p),
+        ("d_w_hidden", C.c_void_p),
+        ("d_b_hidden", C.c_void_p),
+        ("d_w_out", C.c_void_p),
+        ("d_b_out", C.c_void_p),
+        ("d_scale", C.c_void_p),
+        ("d_perm", C.c_void_p),
+        ("d_perm_inv", C.c_void_p),
+    ]
+
+
 ABI_VERSION = 4  # CPPFLOW_ABI_VERSION of include/cppflow_b200.h
 
 _VP, _I, _I64, _SZ, _F, _DBL = C.c_void_p, C.c_int, C.c_int64, C.c_size_t, C.c_float, C.c_double
@@ -141,6 +164,8 @@ _PROTOTYPES = {
     "cppflow_path_key_argmin": (_I, [_VP, _I64, C.POINTER(ConstraintsC), _I64, _VP, _VP]),
     "cppflow_path_metrics_ex": (_I, [_I, _VP, _VP, _I64, _I64, c_float_p, c_float_p, _I, _I, _VP, _VP]),
     "cppflow_sm_partition_create": (_I, [_I, _I, _I, _I, C.POINTER(_VP), C.POINTER(_VP), C.POINTER(_I), C.POINTER(_I)]),
+    "cppflow_flow_workspace_bytes": (_SZ, [C.POINTER(FlowDescC), _I64]),
+    "cppflow_flow_run": (_I, [C.POINTER(FlowDescC), _VP, _VP, _I64, _I64, _I, _VP, _SZ, _VP, _VP]),
     "cppflow_fp32_probe": (_I, [_I, _I, _VP, C.POINTER(C.c_double), _VP]),
     "cppflow_neighbour_probe": (_I, [_I, _I, _I, _I, _VP, _VP]),
 }

@@ -442,3 +442,32 @@ def lm_alternating_loss_many(jobs):
         outs.append((x_out, res))
     check(lib.cppflow_lm_alternating_loss_many(n, arr))
     return [(x, int(r.n_steps_taken), bool(r.is_valid), r.schedule.decode(), list(r.last_metrics)) for x, r in outs]
+
+
+FLOW_REVERSE, FLOW_CLAMP = 1, 2  # CPPFLOW_FLOW_REVERSE / _CLAMP (include/cppflow_b200.h)
+
+
+@_on_device
+def flow_run(desc: _lib.FlowDescC, x: torch.Tensor, cond: torch.Tensor, reverse: bool, clamp: bool = False,
+             out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """IKFlow's GLOW network over the rows of x [n, width] (csrc/k_flow.cu): z -> x with `reverse`, x -> z otherwise.
+    Row i is conditioned on cond[i % len(cond)] ([x, y, z, qw, qx, qy, qz]).  `clamp` (reverse only) clamps the
+    first ndof output columns to the joint limits.  Workspace from the per-stream scratch buffer; no host sync."""
+    import ctypes as C
+
+    x = require_cuda(x, "x")
+    cond = require_cuda(cond, "cond")
+    assert x.dim() == 2 and x.shape[1] == desc.width, f"x must be [n, {desc.width}], is {tuple(x.shape)}"
+    assert cond.dim() == 2 and cond.shape[1] == 7 and cond.shape[0] >= 1, f"cond must be [m, 7], is {tuple(cond.shape)}"
+    n = x.shape[0]
+    out = torch.empty_like(x) if out is None else out
+    assert out.is_cuda and out.dtype == torch.float32 and out.is_contiguous() and out.shape == x.shape
+    lib = _lib.load()
+    nbytes = lib.cppflow_flow_workspace_bytes(C.byref(desc), n)
+    if nbytes == 0:
+        check(-1)
+    ws = _workspace(x.device, nbytes, "flow")
+    flags = (FLOW_REVERSE if reverse else 0) | (FLOW_CLAMP if clamp else 0)
+    check(lib.cppflow_flow_run(C.byref(desc), ptr(x), ptr(cond), n, cond.shape[0], flags, ptr(ws), ws.numel(), ptr(out),
+                               stream_ptr(x.device)))
+    return out

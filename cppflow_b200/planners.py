@@ -1,8 +1,9 @@
 """Planner front-end with the reference's control flow (cppflow/planners.py: Planner._run_pipeline :191-292,
 PlannerSearcher :301-336, CppFlowPlanner.generate_plan :345-468).
 
-IKFlow (the conditional normalising flow that proposes the k candidate joint paths, planners.py:116-172) is out of
-scope - its pretrained weights are not available offline - so the candidate generator is a pluggable callable
+IKFlow (the conditional normalising flow that proposes the k candidate joint paths, planners.py:116-172) runs on the
+CUDA path as `IkflowCandidateGenerator` (cppflow_b200/ikflow.py) with a checkpoint's state dict or seeded random
+weights; its pretrained weights are not available offline.  The candidate generator is a pluggable callable
 `(problem, k) -> [k, T, ndof]`.  The default, `LatentIkCandidateGenerator`, keeps the reference's latent plumbing (one
 latent per path, tiled over the waypoints; sampling around the latent of an initial configuration) on top of
 `LatentIkSolver`, which traces one inverse-kinematics branch per latent by coarse-to-fine numerical continuation with
@@ -254,8 +255,44 @@ class LatentIkCandidateGenerator:
         if initial_q_latent is not None:
             batched = self._sample_latents_near(k, T, initial_q_latent)
         else:
-            batched = self._sample_latents(k, T, robot.ndof)
+            batched = self._sample_latents(k, T, self.solver(robot).network_width)
         return self._get_k_ikflow_qpaths(robot, problem.target_path, batched, k)
+
+
+class IkflowCandidateGenerator(LatentIkCandidateGenerator):
+    """`(problem, k) -> [k, T, ndof]` from IKFlow's network (cppflow_b200/ikflow.py, csrc/k_flow.cu), as the reference
+    does it (planners.py:116-189): the latent sampling of `LatentIkCandidateGenerator` at the flow's `network_width`,
+    the reverse pass with the joint-limit clamp, and the forward pass for the latent of an initial configuration.
+    `solver_or_factory` is an `IkflowSolver` or a callable `robot -> IkflowSolver` (called once per robot).  Every
+    IKFlow sample is close to its target pose, so `last_converged` stays None: dp_search gets the collision flags only,
+    as in the reference."""
+
+    def __init__(self, solver_or_factory, seed: int = 0, latent_distribution: str = "uniform",
+                 latent_vector_scale: float = 2.0):
+        super().__init__(seed, latent_distribution, latent_vector_scale)
+        self._factory = solver_or_factory if callable(solver_or_factory) else None
+        self._fixed = None if callable(solver_or_factory) else solver_or_factory
+
+    def solver(self, robot):
+        if self._fixed is not None:
+            assert self._fixed.robot.name == robot.name, f"the IKFlow solver is for {self._fixed.robot.name}, not {robot.name}"
+            return self._fixed
+        if robot.name not in self._solvers:
+            self._solvers[robot.name] = self._factory(robot)
+        return self._solvers[robot.name]
+
+    def _get_configuration_corresponding_latent(self, robot, qs: torch.Tensor, ee_pose: torch.Tensor) -> torch.Tensor:
+        """planners.py:174-189: the forward pass of the flow at (qs, ee_pose)"""
+        return self.solver(robot).configuration_to_latent(qs.reshape(1, robot.ndof), ee_pose.reshape(1, 7))
+
+    def _get_k_ikflow_qpaths(self, robot, ee_path: torch.Tensor, batched_latent: torch.Tensor, k: int) -> torch.Tensor:
+        """planners.py:155-172 -> stacked [k, T, ndof]"""
+        n = ee_path.shape[0]
+        assert batched_latent.shape[0] == k * n, "one latent row per (path, waypoint), as _sample_latents lays them out"
+        solver = self.solver(robot)
+        latents = batched_latent.reshape(k, n, -1)[:, 0].to(ee_path.device)
+        self.last_converged = None
+        return solver.solve_paths(ee_path, latents, clamp_to_joint_limits=True)
 
 
 def _with_unreached_waypoints(env_v: torch.Tensor, generator) -> torch.Tensor:

@@ -280,6 +280,51 @@ int cppflow_path_key_argmin(const float* d_metrics, int64_t P, const cppflow_con
 int cppflow_sm_partition_create(int device, int min_sms_first, int n_streams_first, int n_streams_second,
                                 void** streams_first, void** streams_second, int* sms_first, int* sms_second);
 
+/* IKFlow's conditional GLOW network (ikflow/model.py: glow_cNF_model; restated in oracle/ikflow.py), the candidate
+ * generator of the reference (planners.py:116-189).  Forward (x -> z) or reverse (z -> x) pass over n rows; row i is
+ * conditioned on d_cond[i % n_cond] = [x, y, z, qw, qx, qy, qz] (the softflow scale, when dim_cond = 8, is 0).
+ * The first Linear of each subnet and its hidden Linears run on the tensor cores (tcgen05, BF16 operands, FP32
+ * accumulation); the subnet input [half | cond] and the hidden activations are stored in BF16.  The last Linear and
+ * the coupling arithmetic are FP32.  A row's result does not depend on n or on the other rows.
+ * Supported: ndof <= 8 (the robot's), ndof <= width <= 16, dim_cond 7 or 8, coeff_fn_config 1..4,
+ * coeff_fn_internal_size a multiple of 128 up to 1024, nb_nodes >= 1, n >= 1; anything else is CPPFLOW_E_INVALID.
+ * Packed weights, with s = 0 for subnet1 and 1 for subnet2 of each coupling block b, H = coeff_fn_internal_size and
+ * L = coeff_fn_config (rows beyond a layer's size are zero):
+ *   d_w_in     bf16 [nb_nodes, 2, H, 64]          first Linear, [out, in] with `in` zero-padded to 64
+ *   d_w_hidden bf16 [nb_nodes, 2, L - 1, H, H]    hidden Linears (NULL when L = 1)
+ *   d_b_hidden fp32 [nb_nodes, 2, L, H]           biases of the first and hidden Linears
+ *   d_w_out    fp32 [nb_nodes, 2, 16, H]          last Linear, [s | t] rows zero-padded to 16
+ *   d_b_out    fp32 [nb_nodes, 2, 16]
+ *   d_scale    fp32 [width]                       diagonal of FixedLinearTransform's M
+ *   d_perm, d_perm_inv int32 [nb_nodes, width]    PermuteRandom of block b and its inverse
+ * Workspace (cppflow_flow_workspace_bytes): four regions, each rounded up to 256 bytes: n x 16 fp32 (state),
+ * n x 64 bf16 (subnet input), and min(L, 2) buffers of n x H bf16 (hidden activations); 0 for an invalid desc.
+ * d_in, d_out [n, width]; with CPPFLOW_FLOW_CLAMP (reverse only) the first ndof columns of the output are clamped
+ * to the robot's joint limits. */
+#define CPPFLOW_FLOW_REVERSE 1
+#define CPPFLOW_FLOW_CLAMP 2
+typedef struct cppflow_flow_desc {
+    int32_t robot;
+    int32_t width; /* dim_latent_space */
+    int32_t ndof;
+    int32_t dim_cond;
+    int32_t nb_nodes;
+    int32_t coeff_fn_config;
+    int32_t coeff_fn_internal_size;
+    float rnvp_clamp;
+    const void* d_w_in;
+    const void* d_w_hidden;
+    const float* d_b_hidden;
+    const float* d_w_out;
+    const float* d_b_out;
+    const float* d_scale;
+    const int32_t* d_perm;
+    const int32_t* d_perm_inv;
+} cppflow_flow_desc;
+size_t cppflow_flow_workspace_bytes(const cppflow_flow_desc* desc, int64_t n);
+int cppflow_flow_run(const cppflow_flow_desc* desc, const float* d_in, const float* d_cond, int64_t n, int64_t n_cond,
+                     int flags, void* d_workspace, size_t workspace_bytes, float* d_out, void* stream);
+
 /* Measurement aid (no reference counterpart): dependent-free FP32 FMA loop on `blocks` x 1024 threads, used by
  * bench.py to measure the FP32 roofline denominator on the box.  *flops_out = FLOPs of the launch. */
 int cppflow_fp32_probe(int blocks, int iters, float* d_scratch, double* flops_out, void* stream);
