@@ -12,7 +12,7 @@ CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libcppflow_b200.so")
 OBJDIR = os.path.join(REPO, "build", "obj")
 
-SOURCES = ["capi.cu", "k_pose.cu", "k_collision.cu", "k_lm_full.cu", "k_search.cu", "k_metrics.cu", "k_probe.cu", "lm_loop.cu", "sm_partition.cu", "k_flow.cu"]
+SOURCES = ["capi.cu", "k_pose.cu", "k_collision.cu", "k_lm_full.cu", "k_search.cu", "k_metrics.cu", "k_probe.cu", "lm_loop.cu", "sm_partition.cu", "k_flow.cu", "k_flow_train.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-std=c++17", "-O3", "-lineinfo", "--expt-relaxed-constexpr",

@@ -127,6 +127,28 @@ class FlowDescC(C.Structure):
     ]
 
 
+class FlowTrainDescC(C.Structure):
+    """cppflow_flow_train_desc"""
+
+    _fields_ = [
+        ("flow", FlowDescC),
+        ("d_params", C.c_void_p),
+        ("d_adam_m", C.c_void_p),
+        ("d_adam_v", C.c_void_p),
+        ("d_w_in_t", C.c_void_p),
+        ("d_w_hidden_t", C.c_void_p),
+        ("d_w_out_t", C.c_void_p),
+        ("d_counters", C.c_void_p),
+        ("lr", C.c_double),
+        ("beta1", C.c_double),
+        ("beta2", C.c_double),
+        ("eps", C.c_double),
+        ("weight_decay", C.c_double),
+        ("lr_decay", C.c_double),
+        ("lr_decay_steps", C.c_int64),
+    ]
+
+
 ABI_VERSION = 4  # CPPFLOW_ABI_VERSION of include/cppflow_b200.h
 
 _VP, _I, _I64, _SZ, _F, _DBL = C.c_void_p, C.c_int, C.c_int64, C.c_size_t, C.c_float, C.c_double
@@ -166,6 +188,10 @@ _PROTOTYPES = {
     "cppflow_sm_partition_create": (_I, [_I, _I, _I, _I, C.POINTER(_VP), C.POINTER(_VP), C.POINTER(_I), C.POINTER(_I)]),
     "cppflow_flow_workspace_bytes": (_SZ, [C.POINTER(FlowDescC), _I64]),
     "cppflow_flow_run": (_I, [C.POINTER(FlowDescC), _VP, _VP, _I64, _I64, _I, _VP, _SZ, _VP, _VP]),
+    "cppflow_flow_train_workspace_bytes": (_SZ, [C.POINTER(FlowTrainDescC), _I64]),
+    "cppflow_flow_train_step": (_I, [C.POINTER(FlowTrainDescC), _VP, _VP, _I64, _I, _VP, _SZ, _VP, _VP, _VP]),
+    "cppflow_flow_train_batch": (_I, [C.POINTER(FlowTrainDescC), _VP, _VP, _I64, _I64, C.c_uint64, _F, _VP, _VP, _VP, _VP,
+                                      _VP]),
     "cppflow_fp32_probe": (_I, [_I, _I, _VP, C.POINTER(C.c_double), _VP]),
     "cppflow_neighbour_probe": (_I, [_I, _I, _I, _I, _VP, _VP]),
 }

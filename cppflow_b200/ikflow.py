@@ -36,6 +36,18 @@ def _split(width: int):
     return width // 2, width - width // 2
 
 
+def params_from_state_dict(sd: Dict[str, torch.Tensor], rnvp_clamp: float = 2.5) -> IkflowModelParameters:
+    """The IkflowModelParameters a GraphINN state dict was built with, read from its shapes (the clamp is not stored
+    in the state dict: it is an argument)."""
+    W = sd["module_list.0.M"].shape[0]
+    nb = sum(1 for k in sd if k.endswith(".perm"))
+    pre = "module_list.2.subnet1"
+    L = sum(1 for k in sd if k.startswith(pre + ".") and k.endswith(".weight")) - 1
+    H, c_in = sd[pre + ".0.weight"].shape
+    return IkflowModelParameters(nb_nodes=nb, dim_latent_space=W, coeff_fn_config=L, coeff_fn_internal_size=H,
+                                 rnvp_clamp=rnvp_clamp, softflow_enabled=c_in - W // 2 == 8)
+
+
 def random_state_dict(robot, params: IkflowModelParameters, seed: int = 0) -> Dict[str, torch.Tensor]:
     """Seeded weights in GraphINN's format: nn.Linear's default init (uniform +-1/sqrt(fan_in) for weight and bias),
     the FixedLinearTransform of the robot's joint limits and PermuteRandom(seed=b)."""
@@ -69,6 +81,52 @@ def random_state_dict(robot, params: IkflowModelParameters, seed: int = 0) -> Di
     return sd
 
 
+def pack_fp32(p: IkflowModelParameters, sd: Dict[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
+    """A GraphINN state dict -> the packed tables of include/cppflow_b200.h (cppflow_flow_desc), all FP32 on the CPU
+    but the int32 permutations."""
+    W, H, L, nb = p.dim_latent_space, p.coeff_fn_internal_size, p.coeff_fn_config, p.nb_nodes
+    dim_cond = 8 if p.softflow_enabled else 7
+    len1, len2 = _split(W)
+    w_in = torch.zeros((nb, 2, H, SUBNET_IN_WIDTH))
+    w_hidden = torch.zeros((nb, 2, max(L - 1, 0), H, H))
+    b_hidden = torch.zeros((nb, 2, L, H))
+    w_out = torch.zeros((nb, 2, OUT_ROWS, H))
+    b_out = torch.zeros((nb, 2, OUT_ROWS))
+    perm = torch.zeros((nb, W), dtype=torch.int32)
+    perm_inv = torch.zeros((nb, W), dtype=torch.int32)
+    M = sd["module_list.0.M"]
+    if tuple(M.shape) != (W, W):
+        raise ValueError(f"module_list.0.M is {tuple(M.shape)}, expected ({W}, {W})")
+    scale = torch.diagonal(M).float().clone()
+    for b in range(nb):
+        key = f"module_list.{2 * b + 1}.perm"
+        pb = sd[key].to(torch.int64) if key in sd else torch.as_tensor(np.random.RandomState(b).permutation(W))
+        if sorted(pb.tolist()) != list(range(W)):
+            raise ValueError(f"{key} is not a permutation of {W} elements")
+        perm[b] = pb.to(torch.int32)
+        perm_inv[b, pb] = torch.arange(W, dtype=torch.int32)
+        for s, (name, c_in, c_out) in enumerate((("subnet1", len1 + dim_cond, 2 * len2),
+                                                 ("subnet2", len2 + dim_cond, 2 * len1))):
+            pre = f"module_list.{2 * b + 2}.{name}"
+            dims = [c_in] + [H] * L + [c_out]
+            for j in range(L + 1):
+                w, bias = sd[f"{pre}.{2 * j}.weight"].float(), sd[f"{pre}.{2 * j}.bias"].float()
+                if tuple(w.shape) != (dims[j + 1], dims[j]) or tuple(bias.shape) != (dims[j + 1],):
+                    raise ValueError(f"{pre}.{2 * j}: weight {tuple(w.shape)} / bias {tuple(bias.shape)}, expected "
+                                     f"({dims[j + 1]}, {dims[j]}) / ({dims[j + 1]},)")
+                if j == 0:
+                    w_in[b, s, :, :c_in] = w
+                elif j < L:
+                    w_hidden[b, s, j - 1] = w
+                if j < L:
+                    b_hidden[b, s, j] = bias
+                else:
+                    w_out[b, s, :c_out] = w
+                    b_out[b, s, :c_out] = bias
+    return {"w_in": w_in, "w_hidden": w_hidden, "b_hidden": b_hidden, "w_out": w_out, "b_out": b_out, "scale": scale,
+            "perm": perm, "perm_inv": perm_inv}
+
+
 class IkflowSolver:
     """(end-effector poses, latents) -> joint configurations through IKFlow's network on the CUDA path.
 
@@ -97,49 +155,12 @@ class IkflowSolver:
             t["perm_inv"].data_ptr())
 
     def _pack(self, sd: Dict[str, torch.Tensor]) -> Dict[str, Optional[torch.Tensor]]:
-        p = self.params
-        W, H, L, nb = self.network_width, p.coeff_fn_internal_size, p.coeff_fn_config, p.nb_nodes
-        len1, len2 = _split(W)
-        w_in = torch.zeros((nb, 2, H, SUBNET_IN_WIDTH))
-        w_hidden = torch.zeros((nb, 2, max(L - 1, 0), H, H))
-        b_hidden = torch.zeros((nb, 2, L, H))
-        w_out = torch.zeros((nb, 2, OUT_ROWS, H))
-        b_out = torch.zeros((nb, 2, OUT_ROWS))
-        perm = torch.zeros((nb, W), dtype=torch.int32)
-        perm_inv = torch.zeros((nb, W), dtype=torch.int32)
-        M = sd["module_list.0.M"]
-        if tuple(M.shape) != (W, W):
-            raise ValueError(f"module_list.0.M is {tuple(M.shape)}, expected ({W}, {W})")
-        scale = torch.diagonal(M).float().clone()
-        for b in range(nb):
-            key = f"module_list.{2 * b + 1}.perm"
-            pb = sd[key].to(torch.int64) if key in sd else torch.as_tensor(np.random.RandomState(b).permutation(W))
-            if sorted(pb.tolist()) != list(range(W)):
-                raise ValueError(f"{key} is not a permutation of {W} elements")
-            perm[b] = pb.to(torch.int32)
-            perm_inv[b, pb] = torch.arange(W, dtype=torch.int32)
-            for s, (name, c_in, c_out) in enumerate((("subnet1", len1 + self.dim_cond, 2 * len2),
-                                                     ("subnet2", len2 + self.dim_cond, 2 * len1))):
-                pre = f"module_list.{2 * b + 2}.{name}"
-                dims = [c_in] + [H] * L + [c_out]
-                for j in range(L + 1):
-                    w, bias = sd[f"{pre}.{2 * j}.weight"].float(), sd[f"{pre}.{2 * j}.bias"].float()
-                    if tuple(w.shape) != (dims[j + 1], dims[j]) or tuple(bias.shape) != (dims[j + 1],):
-                        raise ValueError(f"{pre}.{2 * j}: weight {tuple(w.shape)} / bias {tuple(bias.shape)}, expected "
-                                         f"({dims[j + 1]}, {dims[j]}) / ({dims[j + 1]},)")
-                    if j == 0:
-                        w_in[b, s, :, :c_in] = w
-                    elif j < L:
-                        w_hidden[b, s, j - 1] = w
-                    if j < L:
-                        b_hidden[b, s, j] = bias
-                    else:
-                        w_out[b, s, :c_out] = w
-                        b_out[b, s, :c_out] = bias
-        dev = self.device
-        return {"w_in": w_in.to(torch.bfloat16).to(dev), "w_hidden": w_hidden.to(torch.bfloat16).to(dev) if L > 1 else None,
-                "b_hidden": b_hidden.to(dev), "w_out": w_out.to(dev), "b_out": b_out.to(dev), "scale": scale.to(dev),
-                "perm": perm.to(dev), "perm_inv": perm_inv.to(dev)}
+        t = pack_fp32(self.params, sd)
+        dev, L = self.device, self.params.coeff_fn_config
+        return {"w_in": t["w_in"].to(torch.bfloat16).to(dev),
+                "w_hidden": t["w_hidden"].to(torch.bfloat16).to(dev) if L > 1 else None,
+                "b_hidden": t["b_hidden"].to(dev), "w_out": t["w_out"].to(dev), "b_out": t["b_out"].to(dev),
+                "scale": t["scale"].to(dev), "perm": t["perm"].to(dev), "perm_inv": t["perm_inv"].to(dev)}
 
     def run(self, x: torch.Tensor, cond: torch.Tensor, reverse: bool, clamp: bool = False) -> torch.Tensor:
         """The network over x [n, network_width]; row i conditioned on cond[i % len(cond)] (poses [m, 7])."""

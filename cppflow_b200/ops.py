@@ -471,3 +471,51 @@ def flow_run(desc: _lib.FlowDescC, x: torch.Tensor, cond: torch.Tensor, reverse:
     check(lib.cppflow_flow_run(C.byref(desc), ptr(x), ptr(cond), n, cond.shape[0], flags, ptr(ws), ws.numel(), ptr(out),
                                stream_ptr(x.device)))
     return out
+
+
+FLOW_TRAIN_NO_UPDATE = 1  # CPPFLOW_FLOW_TRAIN_NO_UPDATE (include/cppflow_b200.h)
+
+
+def flow_train_workspace_bytes(desc: _lib.FlowTrainDescC, batch: int) -> int:
+    """Bytes of the workspace of flow_train_step; raises for a desc or batch the library rejects."""
+    import ctypes as C
+
+    nbytes = _lib.load().cppflow_flow_train_workspace_bytes(C.byref(desc), batch)
+    if nbytes == 0:
+        check(-1)
+    return nbytes
+
+
+def flow_train_step(desc: _lib.FlowTrainDescC, x: torch.Tensor, cond: torch.Tensor, workspace: torch.Tensor,
+                    loss: torch.Tensor, grad: Optional[torch.Tensor] = None, update: bool = True) -> None:
+    """One training step of IKFlow's network (csrc/k_flow_train.cu) on the current stream: x [n, width] and cond
+    [n, dim_cond] (n % 128 == 0) -> loss [1] (the batch's mean NLL), the packed gradient into `grad` when given, and
+    with `update` the Adam step on the tables `desc` points at.  No allocation and no host synchronisation."""
+    import ctypes as C
+
+    n = x.shape[0]
+    assert x.is_cuda and x.dtype == torch.float32 and x.is_contiguous() and x.shape == (n, desc.flow.width)
+    assert cond.is_cuda and cond.dtype == torch.float32 and cond.is_contiguous() and cond.shape == (n, desc.flow.dim_cond)
+    assert loss.is_cuda and loss.dtype == torch.float32 and loss.numel() >= 1
+    assert grad is None or (grad.is_cuda and grad.dtype == torch.float32 and grad.is_contiguous())
+    flags = 0 if update else FLOW_TRAIN_NO_UPDATE
+    check(_lib.load().cppflow_flow_train_step(C.byref(desc), ptr(x), ptr(cond), n, flags, ptr(workspace),
+                                              workspace.numel() * workspace.element_size(), ptr(loss), ptr(grad),
+                                              stream_ptr(x.device)))
+
+
+def flow_train_batch(desc: _lib.FlowTrainDescC, q: torch.Tensor, poses: torch.Tensor, seed: int, noise_scale: float,
+                     x: torch.Tensor, cond: torch.Tensor, idx: Optional[torch.Tensor] = None,
+                     noise: Optional[torch.Tensor] = None) -> None:
+    """Draws the training batch of the desc's current step counter into x [n, width] and cond [n, dim_cond] from the
+    dataset q [N, ndof], poses [N, 7] (include/cppflow_b200.h: cppflow_flow_train_batch).  No host synchronisation."""
+    import ctypes as C
+
+    n = x.shape[0]
+    assert q.is_cuda and q.dtype == torch.float32 and q.is_contiguous() and q.shape[1] == desc.flow.ndof
+    assert poses.is_cuda and poses.dtype == torch.float32 and poses.is_contiguous() and poses.shape == (q.shape[0], 7)
+    assert x.is_contiguous() and x.shape == (n, desc.flow.width) and cond.is_contiguous()
+    assert cond.shape == (n, desc.flow.dim_cond)
+    check(_lib.load().cppflow_flow_train_batch(C.byref(desc), ptr(q), ptr(poses), q.shape[0], n, seed & (2**64 - 1),
+                                               float(noise_scale), ptr(x), ptr(cond), ptr(idx), ptr(noise),
+                                               stream_ptr(x.device)))

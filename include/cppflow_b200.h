@@ -325,6 +325,51 @@ size_t cppflow_flow_workspace_bytes(const cppflow_flow_desc* desc, int64_t n);
 int cppflow_flow_run(const cppflow_flow_desc* desc, const float* d_in, const float* d_cond, int64_t n, int64_t n_cond,
                      int flags, void* d_workspace, size_t workspace_bytes, float* d_out, void* stream);
 
+/* Training of the network above: ikflow's train.py (the flow's negative log-likelihood of joint configurations given
+ * their poses, minimised with Adam; restated in oracle/ikflow_train.py: forward_with_logdet, nll, training_batch).
+ * One cppflow_flow_train_step runs, for a batch of n rows (n a multiple of 128, any network cppflow_flow_run accepts):
+ * the forward pass of d_x [n, width] conditioned on d_cond [n, dim_cond] (row i on row i, softflow scale included),
+ * whose z is bit-identical to cppflow_flow_run's; *d_loss = mean(0.5 |z|^2 - log|det dz/dx|); the gradient of the
+ * loss with respect to every packed FP32 parameter (tensor-core GEMMs on tcgen05 for the subnets' Linears, fixed-order
+ * reductions, no atomics: two runs are bit-identical); then, unless CPPFLOW_FLOW_TRAIN_NO_UPDATE, one step of
+ * torch.optim.Adam (weight decay added to the gradient) on the FP32 master weights, which also rewrites the BF16
+ * tables of flow and the transposed copies below.  If any gradient element is not finite the update is skipped:
+ * weights and moments stay, d_counters[1] counts it.  The learning rate is
+ * lr * lr_decay^floor(d_counters[2] / lr_decay_steps) (torch's ExponentialLR stepped every lr_decay_steps steps).
+ * No allocation, no host synchronisation; capturable in a CUDA graph.
+ * d_params, d_adam_m, d_adam_v: fp32 [P], the tables of cppflow_flow_desc concatenated in the order
+ *   w_in [nb, 2, H, 64] | w_hidden [nb, 2, L - 1, H, H] | b_hidden [nb, 2, L, H] | w_out [nb, 2, 16, H] | b_out [nb, 2, 16]
+ *   (padding zero); flow.d_b_hidden, d_w_out and d_b_out must point at their segments of d_params.
+ * d_grad: NULL, or fp32 [P] that receives the gradient (before weight decay) in the same layout.
+ * Rejected (CPPFLOW_E_INVALID): what cppflow_flow_run rejects, n % 128 != 0, width > ndof with dim_cond 7 (the padding
+ * columns have no density without softflow's noise), hyperparameters out of range. */
+#define CPPFLOW_FLOW_TRAIN_NO_UPDATE 1
+typedef struct cppflow_flow_train_desc {
+    cppflow_flow_desc flow;
+    float* d_params;
+    float* d_adam_m;
+    float* d_adam_v;
+    void* d_w_in_t;      /* bf16 [nb, 2, 64, H]: w_in transposed */
+    void* d_w_hidden_t;  /* bf16 [nb, 2, L - 1, H, H]: each hidden weight transposed (NULL when L = 1) */
+    void* d_w_out_t;     /* bf16 [nb, 2, H, 64]: w_out transposed, columns >= 16 zero */
+    int64_t* d_counters; /* [3]: Adam updates applied, steps skipped (non-finite gradient), steps taken */
+    double lr, beta1, beta2, eps, weight_decay, lr_decay;
+    int64_t lr_decay_steps;
+} cppflow_flow_train_desc;
+/* Workspace of cppflow_flow_train_step: all activations of the forward pass plus the backward's buffers; 0 for an
+ * invalid desc or batch. */
+size_t cppflow_flow_train_workspace_bytes(const cppflow_flow_train_desc* desc, int64_t batch);
+int cppflow_flow_train_step(const cppflow_flow_train_desc* desc, const float* d_x, const float* d_cond, int64_t batch,
+                            int flags, void* d_workspace, size_t workspace_bytes, float* d_loss, float* d_grad, void* stream);
+/* A training batch (jrl's sample_joint_angles_and_poses data, ikflow's softflow; oracle/ikflow_train.py: training_batch):
+ * row r takes sample idx of d_q [n_data, ndof] / d_poses [n_data, 7] and draws c ~ U(0, 1), eps ~ N(0, I_width) and a
+ * fair coin from a counter-based generator keyed on (seed, d_counters[2], r); then d_x[r] = [q | 0 ...] +
+ * softflow_noise_scale * c * eps and d_cond[r] = [pose with its quaternion negated on heads | c] (dim_cond 8).  With
+ * dim_cond 7, c = 0 and eps = 0.  Optional outputs: d_idx int64 [batch], d_noise fp32 [batch, width + 2] = [eps | c | coin]. */
+int cppflow_flow_train_batch(const cppflow_flow_train_desc* desc, const float* d_q, const float* d_poses, int64_t n_data,
+                             int64_t batch, uint64_t seed, float softflow_noise_scale, float* d_x, float* d_cond,
+                             int64_t* d_idx, float* d_noise, void* stream);
+
 /* Measurement aid (no reference counterpart): dependent-free FP32 FMA loop on `blocks` x 1024 threads, used by
  * bench.py to measure the FP32 roofline denominator on the box.  *flops_out = FLOPs of the launch. */
 int cppflow_fp32_probe(int blocks, int iters, float* d_scratch, double* flops_out, void* stream);
