@@ -149,6 +149,20 @@ class FlowTrainDescC(C.Structure):
     ]
 
 
+class IkRefineDescC(C.Structure):
+    """cppflow_ik_refine_desc"""
+
+    _fields_ = [
+        ("lambdas", C.c_float * 32),
+        ("n_steps", C.c_int32),
+        ("pos_tol", C.c_float),
+        ("rot_tol", C.c_float),
+        ("alpha_position", C.c_float),
+        ("alpha_rotation", C.c_float),
+        ("flags", C.c_int32),
+    ]
+
+
 ABI_VERSION = 4  # CPPFLOW_ABI_VERSION of include/cppflow_b200.h
 
 _VP, _I, _I64, _SZ, _F, _DBL = C.c_void_p, C.c_int, C.c_int64, C.c_size_t, C.c_float, C.c_double
@@ -192,6 +206,10 @@ _PROTOTYPES = {
     "cppflow_flow_train_step": (_I, [C.POINTER(FlowTrainDescC), _VP, _VP, _I64, _I, _VP, _SZ, _VP, _VP, _VP]),
     "cppflow_flow_train_batch": (_I, [C.POINTER(FlowTrainDescC), _VP, _VP, _I64, _I64, C.c_uint64, _F, _VP, _VP, _VP, _VP,
                                       _VP]),
+    "cppflow_ik_refine": (_I, [_I, C.POINTER(IkRefineDescC), _VP, _VP, _I64, _I64, _VP, _VP, _VP, _VP, _VP]),
+    "cppflow_ik_round_inputs": (_I, [_VP, _I64, _I, _VP, C.c_uint64, _I, _I, _F, _VP, _VP, _VP]),
+    "cppflow_ik_select_workspace_bytes": (_SZ, [_I64]),
+    "cppflow_ik_select": (_I, [_I, _VP, _VP, _VP, _I64, _I, _VP, _VP, _VP, _VP, _VP, _SZ, _VP]),
     "cppflow_fp32_probe": (_I, [_I, _I, _VP, C.POINTER(C.c_double), _VP]),
     "cppflow_neighbour_probe": (_I, [_I, _I, _I, _I, _VP, _VP]),
 }

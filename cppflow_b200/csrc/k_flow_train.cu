@@ -16,6 +16,7 @@
 // BF16 tables and their transposed copies.  No kernel uses atomics and every sum has a fixed order: two runs are
 // bit-identical.
 #include "flow.cuh"
+#include "rng.cuh"
 
 namespace cppflow {
 namespace flow {
@@ -314,15 +315,6 @@ __global__ void __launch_bounds__(256) flow_adam_kernel(AdamArgs a) {
 }
 
 // --------------------------------------------------------------------------------------------- batch sampling
-
-__device__ __forceinline__ uint64_t mix64(uint64_t z) {  // splitmix64's finaliser
-    z += 0x9E3779B97F4A7C15ull;
-    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-    return z ^ (z >> 31);
-}
-
-__device__ __forceinline__ float u01(uint64_t h) { return ((float)(h >> 40) + 0.5f) * (1.f / 16777216.f); }
 
 // One thread per batch row; the random numbers of (seed, step, row) do not depend on the batch size.
 __global__ void __launch_bounds__(256) flow_train_batch_kernel(const float* __restrict__ q, const float* __restrict__ poses,

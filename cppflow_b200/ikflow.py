@@ -7,7 +7,7 @@ oracle/ikflow.py) onto the device once; every call is then one library call on t
 state dict it draws seeded random weights with nn.Linear's default initialisation: the role of the reference's
 `Planner(..., is_mock=True)`.  Pretrained IKFlow weights are not bundled; loading a real checkpoint is unverified."""
 from dataclasses import dataclass
-from typing import Dict, Optional
+from typing import Dict, Optional, Tuple
 
 import numpy as np
 import torch
@@ -181,6 +181,50 @@ class IkflowSolver:
         z = latents.to(self.device, torch.float32).repeat_interleave(T, dim=0)
         q = self.run(z, ee_path, True, clamp_to_joint_limits)
         return q[:, : self.robot.ndof].reshape(k, T, self.robot.ndof)
+
+    def generate_exact_ik_solutions(self, poses: torch.Tensor, pos_tol: float = 1e-3, rot_tol: float = 1e-2,
+                                    repeat_counts=(1, 3, 10), lambdas=None, check_self_collision: bool = False,
+                                    seed: int = 0, latent_scale: float = 1.0) -> Tuple[torch.Tensor, torch.Tensor]:
+        """ikflow's IKFlowSolver.generate_exact_ik_solutions: poses [m, 7] -> (q [m, ndof], valid bool [m]).
+
+        Round r draws repeat_counts[r] latents per target still unsolved (gaussian, times latent_scale, from a generator
+        keyed on (seed, r, target, sample)), runs the reverse pass with the joint-limit clamp, refines every sample with
+        up to len(lambdas) pose-only LM steps that stop once |e_pos| < pos_tol (m) and |e_rot| < rot_tol (rad) - and,
+        with `check_self_collision`, no capsule self pair is at distance <= 0 - and keeps each target's first converged
+        sample (csrc/k_ik.cu).  Targets left unsolved after the last round come back with valid = False and their last
+        refined sample.  `lambdas` defaults to the far-seed damping schedule of `planners.LmIkCandidateGenerator`
+        (20 steps, 1e-1 -> 1e-6); the LM weights are those of ALT_LOSS_V2_1_POSE.
+
+        The tolerances, repeat counts, gaussian latents and latent_scale = 1 are ikflow's defaults as recalled from its
+        public code, not checked against it.  Between rounds the host reads the number of targets still unsolved once:
+        it sizes the next round's flow launch.  That read is the only host synchronisation."""
+        from .lm_hyper_parameters import ALT_LOSS_V2_1_POSE
+        from .planners import LmIkCandidateGenerator
+
+        rob, D = self.robot, self.robot.ndof
+        poses = poses.to(self.device, torch.float32).contiguous()
+        assert poses.dim() == 2 and poses.shape[1] == 7, f"poses must be [m, 7], is {tuple(poses.shape)}"
+        m = poses.shape[0]
+        desc = ops.ik_refine_desc(LmIkCandidateGenerator.LAMBDAS if lambdas is None else lambdas, pos_tol, rot_tol,
+                                  ops.make_params(ALT_LOSS_V2_1_POSE), clamp=True,
+                                  check_self_collision=check_self_collision)
+        solutions = torch.zeros((m, D), device=self.device, dtype=torch.float32)
+        valid = torch.zeros((m,), device=self.device, dtype=torch.uint8)
+        unsolved = torch.arange(m, device=self.device, dtype=torch.int32)
+        spare = torch.empty_like(unsolved)
+        count = torch.empty((1,), device=self.device, dtype=torch.int32)
+        n = m
+        for r, rep in enumerate(repeat_counts):
+            if n == 0:
+                break
+            z, cond = ops.ik_round_inputs(unsolved[:n], rep, poses, seed, r, self.network_width, latent_scale)
+            x = self.run(z, cond, True, True)[:, :D].contiguous()
+            q, status, _ = ops.ik_refine(rob.robot_id, D, desc, x, cond, out=x)
+            ops.ik_select(rob.robot_id, D, q, status, unsolved[:n], rep, solutions, valid, spare, count)
+            unsolved, spare = spare, unsolved
+            if r + 1 < len(repeat_counts):
+                n = int(count.item())
+        return solutions, valid.bool()
 
     def configuration_to_latent(self, q: torch.Tensor, pose: torch.Tensor) -> torch.Tensor:
         """The forward pass of the reference's _get_configuration_corresponding_latent (planners.py:174-189):

@@ -519,3 +519,88 @@ def flow_train_batch(desc: _lib.FlowTrainDescC, q: torch.Tensor, poses: torch.Te
     check(_lib.load().cppflow_flow_train_batch(C.byref(desc), ptr(q), ptr(poses), q.shape[0], n, seed & (2**64 - 1),
                                                float(noise_scale), ptr(x), ptr(cond), ptr(idx), ptr(noise),
                                                stream_ptr(x.device)))
+
+
+IK_CLAMP, IK_CHECK_SELF_COLLISION, IK_NO_EARLY_EXIT = 1, 2, 4  # CPPFLOW_IK_* (include/cppflow_b200.h)
+IK_MAX_STEPS = 32  # CPPFLOW_IK_MAX_STEPS
+
+
+def ik_refine_desc(lambdas, pos_tol: float, rot_tol: float, params: LmParamsC, clamp: bool = True,
+                   check_self_collision: bool = False, early_exit: bool = True) -> _lib.IkRefineDescC:
+    """cppflow_ik_refine_desc: step s damped with lambdas[s]; the alphas of `params` (its lm_lambda is not used)."""
+    lambdas = [float(v) for v in lambdas]
+    if len(lambdas) > IK_MAX_STEPS:
+        raise ValueError(f"at most {IK_MAX_STEPS} LM steps, got {len(lambdas)}")
+    desc = _lib.IkRefineDescC()
+    desc.lambdas[: len(lambdas)] = lambdas
+    desc.n_steps = len(lambdas)
+    desc.pos_tol, desc.rot_tol = float(pos_tol), float(rot_tol)
+    desc.alpha_position, desc.alpha_rotation = params.alpha_position, params.alpha_rotation
+    desc.flags = ((IK_CLAMP if clamp else 0) | (IK_CHECK_SELF_COLLISION if check_self_collision else 0)
+                  | (0 if early_exit else IK_NO_EARLY_EXIT))
+    return desc
+
+
+@_on_device
+def ik_refine(rid: int, ndof: int, desc: _lib.IkRefineDescC, q: torch.Tensor, target: torch.Tensor,
+              out: Optional[torch.Tensor] = None, with_errors: bool = False):
+    """Pose-only LM refinement with a per-row stop (csrc/k_ik.cu), one launch: row i of q [n, ndof] tracks
+    target[i % len(target)].  -> (q_out [n, ndof], status uint8 [n], steps int32 [n][, errors [n, 2] = (|e_pos| m,
+    |e_rot| rad)]).  `out` may be q (in place).  No host synchronisation."""
+    import ctypes as C
+
+    q = _check_q(q, ndof)
+    target = require_cuda(target, "target")
+    assert target.dim() == 2 and target.shape[1] == 7 and target.shape[0] > 0, f"target must be [m, 7], is {tuple(target.shape)}"
+    n = q.shape[0]
+    q_out = torch.empty_like(q) if out is None else out
+    assert q_out.is_cuda and q_out.dtype == torch.float32 and q_out.is_contiguous() and q_out.shape == q.shape
+    status = torch.empty((n,), device=q.device, dtype=torch.uint8)
+    steps = torch.empty((n,), device=q.device, dtype=torch.int32)
+    err = torch.empty((n, 2), device=q.device, dtype=torch.float32) if with_errors else None
+    check(_lib.load().cppflow_ik_refine(rid, C.byref(desc), ptr(q), ptr(target), n, target.shape[0], ptr(q_out),
+                                        ptr(status), ptr(steps), ptr(err), stream_ptr(q.device)))
+    return (q_out, status, steps, err) if with_errors else (q_out, status, steps)
+
+
+@_on_device
+def ik_round_inputs(unsolved: torch.Tensor, rep: int, poses: torch.Tensor, seed: int, round_index: int, width: int,
+                    latent_scale: float = 1.0) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Latents [n * rep, width] and conditions [n * rep, 7] of one exact-IK round for the targets unsolved (int32 [n],
+    indices into poses [m, 7]); row t * rep + j is sample j of target unsolved[t] (include/cppflow_b200.h:
+    cppflow_ik_round_inputs).  No host synchronisation."""
+    unsolved = require_cuda(unsolved, "unsolved", torch.int32)
+    poses = require_cuda(poses, "poses")
+    assert unsolved.dim() == 1 and poses.dim() == 2 and poses.shape[1] == 7
+    if rep < 1:
+        raise ValueError(f"rep must be >= 1, got {rep}")
+    rows = unsolved.shape[0] * rep
+    latents = torch.empty((rows, width), device=poses.device, dtype=torch.float32)
+    cond = torch.empty((rows, 7), device=poses.device, dtype=torch.float32)
+    check(_lib.load().cppflow_ik_round_inputs(ptr(unsolved), unsolved.shape[0], int(rep), ptr(poses),
+                                              int(seed) & (2**64 - 1), int(round_index), int(width), float(latent_scale),
+                                              ptr(latents), ptr(cond), stream_ptr(poses.device)))
+    return latents, cond
+
+
+@_on_device
+def ik_select(rid: int, ndof: int, q: torch.Tensor, status: torch.Tensor, unsolved: torch.Tensor, rep: int,
+              solutions: torch.Tensor, valid: torch.Tensor, unsolved_out: torch.Tensor, n_unsolved_out: torch.Tensor) -> None:
+    """The selection of one exact-IK round (include/cppflow_b200.h: cppflow_ik_select): writes solutions [m, ndof] and
+    valid uint8 [m] of the targets in unsolved (int32 [n]), the targets still unsolved to unsolved_out (int32, >= n
+    entries) and their count to n_unsolved_out (int32 [1]).  Workspace from the per-stream scratch buffer; no host
+    synchronisation."""
+    q = _check_q(q, ndof)
+    n = unsolved.shape[0]
+    assert q.shape[0] == n * rep, f"q must have {n} * {rep} rows, has {q.shape[0]}"
+    assert status.is_cuda and status.dtype == torch.uint8 and status.is_contiguous() and status.shape == (q.shape[0],)
+    assert unsolved.is_cuda and unsolved.dtype == torch.int32 and unsolved.is_contiguous()
+    assert solutions.is_cuda and solutions.dtype == torch.float32 and solutions.is_contiguous()
+    assert solutions.dim() == 2 and solutions.shape[1] == ndof
+    assert valid.is_cuda and valid.dtype == torch.uint8 and valid.is_contiguous() and valid.shape == (solutions.shape[0],)
+    assert unsolved_out.is_cuda and unsolved_out.dtype == torch.int32 and unsolved_out.numel() >= n
+    assert n_unsolved_out.is_cuda and n_unsolved_out.dtype == torch.int32 and n_unsolved_out.numel() >= 1
+    lib = _lib.load()
+    ws = _workspace(q.device, lib.cppflow_ik_select_workspace_bytes(n), "ik_select")
+    check(lib.cppflow_ik_select(rid, ptr(q), ptr(status), ptr(unsolved), n, int(rep), ptr(solutions), ptr(valid),
+                                ptr(unsolved_out), ptr(n_unsolved_out), ptr(ws), ws.numel(), stream_ptr(q.device)))

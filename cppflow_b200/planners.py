@@ -8,6 +8,7 @@ weights; its pretrained weights are not available offline.  The candidate genera
 latent per path, tiled over the waypoints; sampling around the latent of an initial configuration) on top of
 `LatentIkSolver`, which traces one inverse-kinematics branch per latent by coarse-to-fine numerical continuation with
 the pose-only LM steps of the CUDA kernel (SURVEY.md 8f, row f2)."""
+from dataclasses import dataclass
 from time import time
 from typing import Callable, Dict, Optional, Tuple
 
@@ -259,19 +260,40 @@ class LatentIkCandidateGenerator:
         return self._get_k_ikflow_qpaths(robot, problem.target_path, batched, k)
 
 
+@dataclass(frozen=True)
+class IkRefineSettings:
+    """Opt-in LM refinement of IKFlow's candidates (`IkflowCandidateGenerator(refine=...)`): up to len(lambdas)
+    pose-only LM steps per waypoint (step s damped with lambdas[s], at most 32), each waypoint stopping once its pose
+    error is inside pos_tol (m) and rot_tol (rad).  The default tolerances are the plan constraints that
+    `LatentIkSolver._converged` checks (0.1 mm, 0.1 deg)."""
+
+    lambdas: Tuple[float, ...]
+    pos_tol: float = 1e-4
+    rot_tol: float = 1.745e-3
+
+
 class IkflowCandidateGenerator(LatentIkCandidateGenerator):
     """`(problem, k) -> [k, T, ndof]` from IKFlow's network (cppflow_b200/ikflow.py, csrc/k_flow.cu), as the reference
     does it (planners.py:116-189): the latent sampling of `LatentIkCandidateGenerator` at the flow's `network_width`,
     the reverse pass with the joint-limit clamp, and the forward pass for the latent of an initial configuration.
     `solver_or_factory` is an `IkflowSolver` or a callable `robot -> IkflowSolver` (called once per robot).  Every
     IKFlow sample is close to its target pose, so `last_converged` stays None: dp_search gets the collision flags only,
-    as in the reference."""
+    as in the reference.
+
+    With `refine` (an `IkRefineSettings`), the k x T reverse-pass output goes through one LM refinement launch against
+    the [T, 7] path (csrc/k_ik.cu: cppflow_ik_refine, waypoint t of every candidate tracks pose t), and
+    `last_converged` [k, T] is the per-waypoint convergence status, so dp_search sees the waypoints that missed their
+    pose as violations.  No resampling and no host synchronisation happen here.  `refine=None` is the reference's
+    behaviour."""
 
     def __init__(self, solver_or_factory, seed: int = 0, latent_distribution: str = "uniform",
-                 latent_vector_scale: float = 2.0):
+                 latent_vector_scale: float = 2.0, refine: Optional[IkRefineSettings] = None):
         super().__init__(seed, latent_distribution, latent_vector_scale)
         self._factory = solver_or_factory if callable(solver_or_factory) else None
         self._fixed = None if callable(solver_or_factory) else solver_or_factory
+        self.refine = refine
+        self._refine_desc = None if refine is None else ops.ik_refine_desc(
+            refine.lambdas, refine.pos_tol, refine.rot_tol, ops.make_params(ALT_LOSS_V2_1_POSE), clamp=True)
 
     def solver(self, robot):
         if self._fixed is not None:
@@ -292,7 +314,14 @@ class IkflowCandidateGenerator(LatentIkCandidateGenerator):
         solver = self.solver(robot)
         latents = batched_latent.reshape(k, n, -1)[:, 0].to(ee_path.device)
         self.last_converged = None
-        return solver.solve_paths(ee_path, latents, clamp_to_joint_limits=True)
+        qs = solver.solve_paths(ee_path, latents, clamp_to_joint_limits=True)
+        if self.refine is None:
+            return qs
+        D = robot.ndof
+        flat = qs.reshape(k * n, D).contiguous()
+        flat, status, _ = ops.ik_refine(robot.robot_id, D, self._refine_desc, flat, ee_path.contiguous(), out=flat)
+        self.last_converged = status.bool().reshape(k, n)
+        return flat.reshape(k, n, D)
 
 
 def _with_unreached_waypoints(env_v: torch.Tensor, generator) -> torch.Tensor:

@@ -370,6 +370,59 @@ int cppflow_flow_train_batch(const cppflow_flow_train_desc* desc, const float* d
                              int64_t batch, uint64_t seed, float softflow_noise_scale, float* d_x, float* d_cond,
                              int64_t* d_idx, float* d_noise, void* stream);
 
+/* Exact inverse kinematics from IKFlow's samples: ikflow's IKFlowSolver.generate_exact_ik_solutions (sample the flow,
+ * refine every sample with batched Levenberg-Marquardt IK, resample the targets that did not converge with more samples
+ * per round), restated from memory of ikflow's public code, not checked against it.  The three calls below are one
+ * round; cppflow_b200/ikflow.py chains them with cppflow_flow_run.  None allocates or synchronises with the host, and
+ * each can be captured in a CUDA graph.
+ *
+ * cppflow_ik_refine: up to n_steps pose-only LM steps per row (jrl's batched LM IK step as the reference's
+ * levenberg_marquardt_only_pose + clamp_to_joint_limits, optimization.py:61-92), one thread per row with q and the
+ * target in registers.  Step s uses lambdas[s]; each step is the arithmetic of one cppflow_lm_pose_step launch.
+ * Before each step and after the last one the row computes its pose error (get_6d_pose_errors) and stops when
+ * |e_pos| < pos_tol (m) and |e_rot| < rot_tol (rad), the norms taken in FP32 as sqrt((e0^2 + e1^2) + e2^2) without
+ * fused multiply-adds.  With CPPFLOW_IK_CHECK_SELF_COLLISION it also needs every capsule self pair at distance > 0
+ * (Robot.self_collision_distances).  CPPFLOW_IK_NO_EARLY_EXIT: every row takes all n_steps and is checked once at
+ * the end.  CPPFLOW_IK_CLAMP clamps to the joint limits after every step.
+ * Row i tracks d_target[i % n_targets].  Out: d_q_out [n, ndof] (may be d_q), d_status uint8 [n] (1 = converged),
+ * d_steps int32 [n] (steps taken; NULL allowed), d_err [n, 2] = final (|e_pos|, |e_rot|) (NULL allowed).
+ * Rejected: n_steps outside [0, CPPFLOW_IK_MAX_STEPS], negative or NaN tolerances, unknown flags. */
+#define CPPFLOW_IK_MAX_STEPS 32
+#define CPPFLOW_IK_CLAMP 1
+#define CPPFLOW_IK_CHECK_SELF_COLLISION 2
+#define CPPFLOW_IK_NO_EARLY_EXIT 4
+typedef struct cppflow_ik_refine_desc {
+    float lambdas[CPPFLOW_IK_MAX_STEPS];
+    int32_t n_steps;
+    float pos_tol;
+    float rot_tol;
+    float alpha_position;
+    float alpha_rotation;
+    int32_t flags;
+} cppflow_ik_refine_desc;
+int cppflow_ik_refine(int robot, const cppflow_ik_refine_desc* desc, const float* d_q, const float* d_target, int64_t n,
+                      int64_t n_targets, float* d_q_out, uint8_t* d_status, int32_t* d_steps, float* d_err, void* stream);
+
+/* The latents and conditions of one round (IKFlowSolver.generate_ik_solutions' latent draw, latent_distribution =
+ * "gaussian" scaled by latent_scale): row r = t * rep + j, for t < n_unsolved and j < rep, is sample j of target
+ * d_unsolved[t].  d_latents [n_unsolved * rep, width] ~ latent_scale * N(0, I) from a counter-based generator keyed
+ * on (seed, round, target, j), so a row does not depend on which other targets are still unsolved;
+ * d_cond [n_unsolved * rep, 7] = d_poses[target], the condition layout of cppflow_flow_run. */
+int cppflow_ik_round_inputs(const int32_t* d_unsolved, int64_t n_unsolved, int rep, const float* d_poses, uint64_t seed, int round, int width, float latent_scale, float* d_latents, float* d_cond,
+                            void* stream);
+
+/* The selection of one round (generate_exact_ik_solutions' choice among a target's converged samples): d_q [n_unsolved *
+ * rep, ndof] and d_status [n_unsolved * rep] laid out as cppflow_ik_round_inputs lays out the rows.  For each target
+ * d_unsolved[t], the converged sample with the smallest j goes to d_solutions[target] and d_valid[target] = 1; with
+ * none, sample 0 goes there and d_valid[target] = 0.  The targets still unsolved are written to d_unsolved_out in
+ * ascending list order and their count to *d_n_unsolved_out (order-preserving compaction: deterministic, no atomics).
+ * Workspace: cppflow_ik_select_workspace_bytes(n_unsolved) bytes, 256-byte aligned (0: n_unsolved out of range or no
+ * device to size the compaction for). */
+size_t cppflow_ik_select_workspace_bytes(int64_t n_unsolved);
+int cppflow_ik_select(int robot, const float* d_q, const uint8_t* d_status, const int32_t* d_unsolved, int64_t n_unsolved,
+                      int rep, float* d_solutions, uint8_t* d_valid, int32_t* d_unsolved_out, int32_t* d_n_unsolved_out,
+                      void* d_workspace, size_t workspace_bytes, void* stream);
+
 /* Measurement aid (no reference counterpart): dependent-free FP32 FMA loop on `blocks` x 1024 threads, used by
  * bench.py to measure the FP32 roofline denominator on the box.  *flops_out = FLOPs of the launch. */
 int cppflow_fp32_probe(int blocks, int iters, float* d_scratch, double* flops_out, void* stream);

@@ -7,10 +7,14 @@ visualisation, no results directory).
     python tools/evaluate.py --planner PlannerSearcher --problem panda__1cube --k 64
     python tools/evaluate.py --problem_file my_problem.yaml            # a problem yaml in the reference's layout
     python tools/evaluate.py --all --ikflow_checkpoint panda_sd.pt     # candidates from a trained IKFlow
+    python tools/evaluate.py --all --ikflow_checkpoint panda_sd.pt --ikflow_refine   # ... refined by LM IK
 
 --ikflow_checkpoint takes a GraphINN state dict (tools/train_ikflow.py --state_dict, or an IKFlow checkpoint's); the
 planner then draws its candidates with IkflowCandidateGenerator.  The network's shape is read from the state dict,
-and problems of robots whose joint scale differs from the state dict's are skipped.
+and problems of robots whose joint scale differs from the state dict's are skipped.  --ikflow_refine passes the
+flow's candidates through the per-waypoint LM refinement (IkRefineSettings: the 20-step damping schedule of
+LmIkCandidateGenerator, stopping at 0.1 mm / 0.1 deg); waypoints that do not converge count as violations in
+dp_search.
 
 Errors come from plan_from_qpath (FK of the returned path against the target path); the validity flag is the
 capsule-model one (the reference's klampt mesh check is out of scope)."""
@@ -24,7 +28,8 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from cppflow_b200.data_type_utils import ALL_PROBLEM_FILENAMES, plan_from_qpath, problem_from_filename  # noqa: E402
 from cppflow_b200.data_types import Constraints, PlannerSettings  # noqa: E402
 from cppflow_b200.ikflow import IkflowSolver, params_from_state_dict  # noqa: E402
-from cppflow_b200.planners import CppFlowPlanner, IkflowCandidateGenerator, PlannerSearcher  # noqa: E402
+from cppflow_b200.planners import (CppFlowPlanner, IkflowCandidateGenerator, IkRefineSettings,  # noqa: E402
+                                   LmIkCandidateGenerator, PlannerSearcher)
 
 PLANNERS = {"CppFlow": CppFlowPlanner, "PlannerSearcher": PlannerSearcher}
 COLUMNS = ["Problem", "Robot", "Planner", "Valid plan", "time, total (s)", "time, ikflow (s)", "time, coll_checking (s)",
@@ -64,9 +69,13 @@ def main(argv=None):
     ap.add_argument("--device", default="cuda:0")
     ap.add_argument("--no_warmup", action="store_true")
     ap.add_argument("--ikflow_checkpoint", default=None, help="GraphINN state dict: plan with IkflowCandidateGenerator")
+    ap.add_argument("--ikflow_refine", action="store_true", help="LM-refine the IKFlow candidates (IkRefineSettings)")
     args = ap.parse_args(argv)
     if args.ikflow_checkpoint and args.planner != "CppFlow":
         ap.error("--ikflow_checkpoint needs --planner CppFlow")
+    if args.ikflow_refine and not args.ikflow_checkpoint:
+        ap.error("--ikflow_refine needs --ikflow_checkpoint")
+    refine = IkRefineSettings(LmIkCandidateGenerator.LAMBDAS) if args.ikflow_refine else None
     sd = torch.load(args.ikflow_checkpoint, map_location="cpu") if args.ikflow_checkpoint else None
     if args.all:
         problems = [problem_from_filename(CONSTRAINTS, n, device=args.device) for n in ALL_PROBLEM_FILENAMES]
@@ -89,7 +98,7 @@ def main(argv=None):
                 continue
             if rob.name not in solvers:
                 solvers[rob.name] = IkflowSolver(rob, params_from_state_dict(sd), state_dict=sd, device=args.device)
-            generator = IkflowCandidateGenerator(solvers[rob.name], seed=0)
+            generator = IkflowCandidateGenerator(solvers[rob.name], seed=0, refine=refine)
         try:
             row, ok = evaluate(args.planner, problem, settings, warmup=not args.no_warmup, generator=generator)
         except AssertionError as e:  # the reference's checks on the candidates, e.g. "too many env collisions"

@@ -1,7 +1,8 @@
 """Train IKFlow for one robot on one GPU (cppflow_b200/ikflow_training.py) and print one JSON line every --every steps:
 the mean NLL of those steps and the accuracy of the flow as an IK sampler at a fixed set of held-out poses (--k
 reverse-pass samples with z ~ N(0, 1) per pose; mean and median position and rotation error of their forward
-kinematics).
+kinematics), and the share of those poses that IkflowSolver.generate_exact_ik_solutions solves with its defaults
+(exact_ik_success: 1 mm and 0.01 rad after LM refinement, rounds of 1, 3 and 10 samples per unsolved pose).
 
     python tools/train_ikflow.py --robot panda --minutes 30 --out runs/panda.ckpt --state_dict runs/panda_sd.pt
     python tools/train_ikflow.py --resume runs/panda.ckpt --steps 10000 --out runs/panda.ckpt
@@ -60,10 +61,12 @@ def main(argv=None):
     def report(t_loop):
         hist = tr.loss_history()
         taken = int(tr.counters[2].item())
+        solver = tr.solver()
         recent = hist[-min(args.every, hist.numel()):] if hist.numel() else hist
         line = {"step": taken, "samples": taken * tr.batch_size, "train_seconds": round(t_loop, 2),
                 "nll": recent.mean().item() if recent.numel() else None,
-                "skipped": int(tr.counters[1].item()), **sample_accuracy(tr.solver(), held, args.k)}
+                "skipped": int(tr.counters[1].item()), **sample_accuracy(solver, held, args.k),
+                "exact_ik_success": solver.generate_exact_ik_solutions(held)[1].float().mean().item()}
         print(json.dumps(line), flush=True)
         if args.out:
             tr.save(args.out)
