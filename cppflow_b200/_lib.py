@@ -163,7 +163,7 @@ class IkRefineDescC(C.Structure):
     ]
 
 
-ABI_VERSION = 4  # CPPFLOW_ABI_VERSION of include/cppflow_b200.h
+ABI_VERSION = 5  # CPPFLOW_ABI_VERSION of include/cppflow_b200.h
 
 _VP, _I, _I64, _SZ, _F, _DBL = C.c_void_p, C.c_int, C.c_int64, C.c_size_t, C.c_float, C.c_double
 _PROTOTYPES = {
@@ -199,7 +199,6 @@ _PROTOTYPES = {
     "cppflow_path_metrics": (_I, [_I, _VP, _VP, _I64, _I64, c_float_p, c_float_p, _I, _VP, _VP]),
     "cppflow_path_key_argmin": (_I, [_VP, _I64, C.POINTER(ConstraintsC), _I64, _VP, _VP]),
     "cppflow_path_metrics_ex": (_I, [_I, _VP, _VP, _I64, _I64, c_float_p, c_float_p, _I, _I, _VP, _VP]),
-    "cppflow_sm_partition_create": (_I, [_I, _I, _I, _I, C.POINTER(_VP), C.POINTER(_VP), C.POINTER(_I), C.POINTER(_I)]),
     "cppflow_flow_workspace_bytes": (_SZ, [C.POINTER(FlowDescC), _I64]),
     "cppflow_flow_run": (_I, [C.POINTER(FlowDescC), _VP, _VP, _I64, _I64, _I, _VP, _SZ, _VP, _VP]),
     "cppflow_flow_train_workspace_bytes": (_SZ, [C.POINTER(FlowTrainDescC), _I64]),
@@ -211,7 +210,6 @@ _PROTOTYPES = {
     "cppflow_ik_select_workspace_bytes": (_SZ, [_I64]),
     "cppflow_ik_select": (_I, [_I, _VP, _VP, _VP, _I64, _I, _VP, _VP, _VP, _VP, _VP, _SZ, _VP]),
     "cppflow_fp32_probe": (_I, [_I, _I, _VP, C.POINTER(C.c_double), _VP]),
-    "cppflow_neighbour_probe": (_I, [_I, _I, _I, _I, _VP, _VP]),
 }
 EXPORTED_SYMBOLS = tuple(_PROTOTYPES)
 

@@ -17,8 +17,6 @@
 // thread and writes the packed (A_tt, b_t) block (44 floats for D = 8) to the workspace.
 // Kernel B (solve) runs a twisted block-Thomas elimination per path (two lanes per path, one from each end), streaming
 // the blocks in with TMA bulk copies, and writes clamp(x + dx).  Nothing of size (T*D)^2 is ever formed.
-#include <cstdlib>
-
 #include "common.cuh"
 #include "collision.cuh"
 #include "linalg.cuh"
@@ -118,54 +116,10 @@ struct BetaSel {
     }
 };
 
-#ifdef CPPFLOW_SOLVE_TIMING
-// debug build only (tools/probe_solve_phases.py): cycles of lane 0 of every warp per phase of the forward / backward loops
-__device__ unsigned long long g_solve_cycles[8];
-#define PHASE_T(var) const long long var = clock64()
-#define PHASE_DECL long long ph_acc[7] = {0, 0, 0, 0, 0, 0, 0}
-#define PHASE_ADD(i, a, b) ph_acc[i] += (b) - (a)
-#define PHASE_FLUSH if (lane == 0) { for (int i_ = 0; i_ < 7; ++i_) atomicAdd(&g_solve_cycles[i_], (unsigned long long)ph_acc[i_]); }
-extern "C" int cppflow_debug_solve_cycles(unsigned long long* h_out, int reset) {
-    if (reset) { unsigned long long z[8] = {}; cudaMemcpyToSymbol(g_solve_cycles, z, sizeof(z)); return 0; }
-    cudaMemcpyFromSymbol(h_out, g_solve_cycles, sizeof(unsigned long long) * 8);
-    return 0;
-}
-#else
-#define PHASE_T(var)
-#define PHASE_DECL
-#define PHASE_ADD(i, a, b)
-#define PHASE_FLUSH
-#endif
-
-// Fused elimination (CPPFLOW_LM_FUSED): the assembly CTA of waypoint t also takes the elimination step of that waypoint,
-// so the (A_tt, b_t) block never leaves registers - what goes to the workspace is (-S_t^-1, u_t) straight away, and the
-// solve that follows only back-substitutes (HBM traffic of an iteration 1.85 -> ~1.05 GB).  The chain S_t = A_t - E
-// S_{t-1}^-1 E runs from CTA to CTA: warp w of the CTA of (path block, side, step k) waits for flags[block][side][w]
-// >= k, reads the predecessor's result block (L2: it was written a few microseconds ago by another SM), eliminates,
-// stores, and publishes k + 1.  CTAs take their (row, path block) from a ticket counter in launch order, rows in the
-// order the twisted sweep consumes them (0, T-1, 1, T-2, ..., middle), so a CTA's predecessor always holds a smaller
-// ticket and is running or done: no deadlock whatever the number of resident CTAs.
-struct FuseParams {
-    int* flags;    // [path blocks][2 sides][ABLOCK / 32 warps] steps completed, zeroed before the launch
-    int* ticket;   // CTA counter, zeroed before the launch
-    int npb;       // path blocks
-    const float* q;
-    float* x_out;  // the middle waypoint's new configuration is written here
-    SolveParams sp;
-};
-__device__ __forceinline__ int ld_acquire_gpu(const int* p) {
-    int v;
-    asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void st_release_gpu(int* p, int v) {
-    asm volatile("st.release.gpu.global.s32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-
-template <class M, bool FUSE>
+template <class M>
 __global__ void __launch_bounds__(ABLOCK, 2)
 lm_assemble_kernel(const float* __restrict__ q, const float* __restrict__ xv, const float* __restrict__ target,
-                   int P, int T, const Obstacles ob, const AssembleParams prm, float* __restrict__ ws, const FuseParams fz) {
+                   int P, int T, const Obstacles ob, const AssembleParams prm, float* __restrict__ ws) {
     constexpr int D = M::NDOF;
     constexpr int NT = BlockLayout<D>::NT;
     constexpr int NW = BlockLayout<D>::NW;
@@ -174,22 +128,7 @@ lm_assemble_kernel(const float* __restrict__ q, const float* __restrict__ xv, co
     fill_coll_tables<M>(tb, ob, threadIdx.x, ABLOCK);
     // grid = (path blocks, waypoints): consecutive threads take consecutive PATHS at the same waypoint t, so the
     // target pose is block-uniform and the block stores below are fully coalesced in the [t][k][path] workspace
-    int t, pbx, f_side = 0, f_k = 0;
-    bool f_middle = false;
-    if constexpr (FUSE) {
-        __shared__ int s_ticket;
-        if (threadIdx.x == 0) s_ticket = atomicAdd(fz.ticket, 1);
-        __syncthreads();
-        const int row = s_ticket / fz.npb;  // rows in the order the twisted elimination consumes them
-        pbx = s_ticket - row * fz.npb;
-        const int m = T / 2, n1 = T - 1 - m;  // side 0 eliminates t = 0 .. m-1, side 1 t = T-1 .. m+1, then the middle
-        if (row < 2 * n1) { f_k = row >> 1; f_side = row & 1; t = f_side ? T - 1 - f_k : f_k; }
-        else if (row < T - 1) { f_k = n1; f_side = 0; t = n1; }  // m = n1 + 1: side 0's last step
-        else { f_middle = true; t = m; }
-    } else {
-        t = blockIdx.y;
-        pbx = blockIdx.x;
-    }
+    const int t = blockIdx.y, pbx = blockIdx.x;
     const int pth_raw = pbx * ABLOCK + threadIdx.x;
     const bool live = pth_raw < P;
     const int pth = live ? pth_raw : P - 1;  // idle lanes shadow the last path and skip the stores
@@ -367,96 +306,7 @@ lm_assemble_kernel(const float* __restrict__ q, const float* __restrict__ xv, co
 #pragma unroll
         for (int k = 0; k < NW / 4; ++k) out[k * 16] = make_float4(blk[4 * k], blk[4 * k + 1], blk[4 * k + 2], blk[4 * k + 3]);
     };
-    if constexpr (!FUSE) {
-        if (live) store_blk(t, A, b);
-    } else {
-        constexpr int NWARP = ABLOCK / 32;
-        const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-        const BetaSel<M> bs(fz.sp.b_rev, fz.sp.b_pri);
-        int* flags_pb = fz.flags + pbx * 2 * NWARP;
-        // lane 0 waits for the chain's predecessor, the warp follows (other SMs wrote the block: read it from L2)
-        auto wait_for = [&](const int* flag, int need) {
-            if (lane == 0) {
-                while (ld_acquire_gpu(flag) < need) __nanosleep(64);
-            }
-            __syncwarp();
-        };
-        auto load_blk = [&](int tt, float (&v)[NW]) {
-            const float4* src = block_at(tt);
-#pragma unroll
-            for (int k = 0; k < NW / 4; ++k) {
-                const float4 f = __ldcg(src + k * 16);
-                v[4 * k] = f.x; v[4 * k + 1] = f.y; v[4 * k + 2] = f.z; v[4 * k + 3] = f.w;
-            }
-        };
-        if (!f_middle) {
-            int* flag = flags_pb + f_side * NWARP + warp;
-            float u[D];
-            if (f_k > 0) {
-                wait_for(flag, f_k);
-                float pb_[NW];
-                load_blk(f_side ? t + 1 : t - 1, pb_);
-                static_for<D>([&](auto Ii) {
-                    constexpr int i = decltype(Ii)::value;
-                    u[i] = fmaf(bs.template b<i>(), pb_[NT + i], b[i]);
-                    static_for<i + 1>([&](auto Jj) {
-                        constexpr int j = decltype(Jj)::value;
-                        A[tri(i, j)] = fmaf(bs.template bb<i, j>(), pb_[tri(i, j)], A[tri(i, j)]);
-                    });
-                });
-            } else {  // first block of a side: S = A + (beta beta^T) . 0, y = b + beta . 0 (the same fmaf, for the same bits)
-                static_for<D>([&](auto Ii) {
-                    constexpr int i = decltype(Ii)::value;
-                    u[i] = fmaf(bs.template b<i>(), 0.f, b[i]);
-                    static_for<i + 1>([&](auto Jj) {
-                        constexpr int j = decltype(Jj)::value;
-                        A[tri(i, j)] = fmaf(bs.template bb<i, j>(), 0.f, A[tri(i, j)]);
-                    });
-                });
-            }
-            sweep_neg_inverse<D>(A, u, fz.sp.pivot_floor);
-            if (live) store_blk(t, A, u);
-            __threadfence();  // this lane's stores are visible device-wide ...
-            __syncwarp();     // ... for every lane of the warp, before lane 0 publishes the step
-            if (lane == 0) st_release_gpu(flag, f_k + 1);
-        } else {
-            const int m = t, n0 = m, n1 = T - 1 - m;
-            float dx[D];
-            float L[NW], Rb[NW];
-            if (n0 > 0) { wait_for(flags_pb + warp, n0); load_blk(m - 1, L); }
-            else {
-#pragma unroll
-                for (int k = 0; k < NW; ++k) L[k] = 0.f;
-            }
-            if (n1 > 0) { wait_for(flags_pb + NWARP + warp, n1); load_blk(m + 1, Rb); }
-            else {
-#pragma unroll
-                for (int k = 0; k < NW; ++k) Rb[k] = 0.f;
-            }
-            static_for<D>([&](auto Ii) {
-                constexpr int i = decltype(Ii)::value;
-                dx[i] = fmaf(bs.template b<i>(), L[NT + i] + Rb[NT + i], b[i]);
-                static_for<i + 1>([&](auto Jj) {
-                    constexpr int j = decltype(Jj)::value;
-                    A[tri(i, j)] = fmaf(bs.template bb<i, j>(), L[tri(i, j)] + Rb[tri(i, j)], A[tri(i, j)]);
-                });
-            });
-            sweep_neg_inverse<D>(A, dx, fz.sp.pivot_floor);
-            if (live) {
-                store_blk(m, A, dx);  // the back-substitution starts from dx_m (the u slot of the middle block)
-                float xn[D];
-                load_row<D>(fz.q + i * D, xn);
-                static_for<D>([&](auto Dd) {
-                    constexpr int d = decltype(Dd)::value;
-                    xn[d] += dx[d];
-                    if (fz.sp.do_clamp) xn[d] = fminf(fmaxf(xn[d], dof_lower<M>(d)), dof_upper<M>(d));
-                });
-                float* xo = fz.x_out + i * D;
-#pragma unroll
-                for (int d = 0; d < D; ++d) xo[d] = xn[d];
-            }
-        }
-    }
+    if (live) store_blk(t, A, b);
 }
 
 template <int NW>
@@ -583,9 +433,7 @@ __device__ __forceinline__ void cp_async4_a(unsigned dst, const void* gmem) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(gmem) : "memory");
 }
 
-// BACK_ONLY: the elimination and the middle block were done by the fused assembly (lm_assemble_kernel<M, true>): the
-// workspace already holds (-S_t^-1, u_t) and, in the middle block's u slot, dx_m; only the back-substitution runs.
-template <class M, int SOLVE_RING, int SOLVE_WARPS, bool BACK_ONLY = false>
+template <class M, int SOLVE_RING, int SOLVE_WARPS>
 __global__ void __launch_bounds__(32 * SOLVE_WARPS, 512 / (32 * SOLVE_WARPS))
 lm_block_solve_kernel(const float* __restrict__ q, int64_t P, int64_t T64, const SolveParams prm, float* __restrict__ ws,
                       float* __restrict__ x_out) {
@@ -692,7 +540,6 @@ lm_block_solve_kernel(const float* __restrict__ q, int64_t P, int64_t T64, const
         }
     };
 
-    PHASE_DECL;
     // running state of this side: nS = -S^-1 of the block eliminated last (packed lower triangle), u = S^-1 y
     float nS[NT], u[D];
 #pragma unroll
@@ -701,21 +548,15 @@ lm_block_solve_kernel(const float* __restrict__ q, int64_t P, int64_t T64, const
     for (int d = 0; d < D; ++d) u[d] = 0.f;
 
     // ---- elimination sweep (steps s = 0 .. n_iter-1):  S_t = A_t + (beta beta^T) . nS,  y_t = b_t + beta . u_in
-    if constexpr (!BACK_ONLY) {
 #pragma unroll
     for (int j = 0; j < SOLVE_RING; ++j)
         if (j < n_iter) issue(j, j < n0 ? j : -1, j < n1 ? T - 1 - j : -1, 0u);
     for (int k = 0; k < n_iter; ++k) {
         const bool mine = k < n_side;
         float blk[NW];
-        PHASE_T(c0);
         wait_slot();
-        PHASE_T(c1);
         if (mine) read_block(blk);
         const unsigned token = slot_read_token(blk, mine);  // every lane's reads of the slot have returned
-        PHASE_T(c2);
-        PHASE_ADD(0, c0, c1);
-        PHASE_ADD(1, c1, c2);
         if (mine) {
             static_for<D>([&](auto Ii) {
                 constexpr int i = decltype(Ii)::value;
@@ -727,8 +568,6 @@ lm_block_solve_kernel(const float* __restrict__ q, int64_t P, int64_t T64, const
             });
             sweep_neg_inverse<D>(nS, u, prm.pivot_floor);
         }
-        PHASE_T(c3);
-        PHASE_ADD(2, c2, c3);
         // refill the slot with step k + RING.  Issued AFTER the sweep: the elected lane's few instructions would
         // otherwise sit between the loads and the first pivot of every step; the slot is not needed for RING more steps.
         {
@@ -752,12 +591,8 @@ lm_block_solve_kernel(const float* __restrict__ q, int64_t P, int64_t T64, const
 #pragma unroll
             for (int i = 0; i < NV; ++i) dstg[i * 16] = make_float4(v[4 * i], v[4 * i + 1], v[4 * i + 2], v[4 * i + 3]);
         }
-        PHASE_T(c4);
-        PHASE_ADD(3, c3, c4);
         advance();
     }
-    }  // !BACK_ONLY
-    PHASE_T(cf0);
     __threadfence();                                  // the generic stores above are performed ...
     asm volatile("fence.proxy.async;" ::: "memory");  // ... and ordered before the async-proxy (TMA) reads below
     __syncwarp();
@@ -794,17 +629,7 @@ lm_block_solve_kernel(const float* __restrict__ q, int64_t P, int64_t T64, const
 
     // ---- middle block: S_m = A_m + (beta beta^T) . (nS_left + nS_right),  y_m = b_m + beta . (u_left + u_right)
     float dx[D];
-    if constexpr (BACK_ONLY) {
-        const float4* src = reinterpret_cast<const float4*>(wsg + m * SM::BLK_BYTES) + l;
-        float tail[NW - NT / 4 * 4];  // the float4s that hold the u slot (dx_m)
-#pragma unroll
-        for (int k = NT / 4; k < NV; ++k) {
-            const float4 f = src[k * 16];
-            tail[4 * (k - NT / 4)] = f.x; tail[4 * (k - NT / 4) + 1] = f.y; tail[4 * (k - NT / 4) + 2] = f.z; tail[4 * (k - NT / 4) + 3] = f.w;
-        }
-#pragma unroll
-        for (int i = 0; i < D; ++i) dx[i] = tail[NT - NT / 4 * 4 + i];
-    } else {
+    {
         float Sm[NT];
         float blk[NW];
         const float4* src = reinterpret_cast<const float4*>(wsg + m * SM::BLK_BYTES) + l;
@@ -839,10 +664,7 @@ lm_block_solve_kernel(const float* __restrict__ q, int64_t P, int64_t T64, const
         const int k = n_side - 1 - r;
         const bool mine = k >= 0;
         float blk[NW], xn[D];
-        PHASE_T(b0);
         wait_slot();
-        PHASE_T(b1);
-        PHASE_ADD(4, b0, b1);
         if (mine) {
             read_block(blk);
 #pragma unroll
@@ -878,15 +700,10 @@ lm_block_solve_kernel(const float* __restrict__ q, int64_t P, int64_t T64, const
         }
         if (mine && active) store_x(t_of(k), xn);
         cp_async_commit();
-        PHASE_T(b2);
-        PHASE_ADD(5, b1, b2);
         advance();
         if (++qslot == SOLVE_RING) qslot = 0;
     }
     cp_async_wait<0>();
-    PHASE_T(cf1);
-    PHASE_ADD(6, cf0, cf1);  // fence + middle block + whole back-substitution
-    PHASE_FLUSH;
 }
 
 // ----------------------------------------------------------------------------------------------------------------
@@ -1265,22 +1082,19 @@ static int launch_assemble(const cppflow_lm_params* p, const float* q, const flo
     AssembleParams ap;
     SolveParams sp;
     make_params<M>(p, ob.n, 0, ap, sp);
-    size_t sh = sizeof(float) * ABLOCK * SmemLayout<M>::N_FULL;
-    // experiment switch (profiles/r02_notes.md, occupancy curve): extra KB of shared memory per CTA, e.g. 90 -> one CTA per SM
-    static const char* pad_kb = std::getenv("CPPFLOW_ASM_SMEM_PAD_KB");
-    if (pad_kb) sh += (size_t)std::atoi(pad_kb) * 1024;
+    const size_t sh = sizeof(float) * ABLOCK * SmemLayout<M>::N_FULL;
     static SmemGrant granted;  // per template instantiation and device
-    if (int rc = ensure_dynamic_smem(lm_assemble_kernel<M, false>, sh, granted)) return rc;
+    if (int rc = ensure_dynamic_smem(lm_assemble_kernel<M>, sh, granted)) return rc;
     const dim3 grid(grid_for(P, ABLOCK), (unsigned)T);
-    lm_assemble_kernel<M, false><<<grid, ABLOCK, sh, st>>>(q, xv, target, (int)P, (int)T, ob, ap, ws, FuseParams{});
+    lm_assemble_kernel<M><<<grid, ABLOCK, sh, st>>>(q, xv, target, (int)P, (int)T, ob, ap, ws);
     return CPPFLOW_OK;
 }
 
-template <class M, int RING, int WARPS = SOLVE_WARPS_DEFAULT, bool BACK_ONLY = false>
+template <class M, int RING, int WARPS = SOLVE_WARPS_DEFAULT>
 static int launch_solve_variant(const SolveParams& sp, const float* q, int64_t P, int64_t T, bool high_priority,
                                 float* ws, float* x_out, cudaStream_t st) {
     const size_t sh = SolveSmem<M::NDOF, RING>::BYTES * WARPS;
-    auto kern = lm_block_solve_kernel<M, RING, WARPS, BACK_ONLY>;
+    auto kern = lm_block_solve_kernel<M, RING, WARPS>;
     static SmemGrant granted;  // per template instantiation and device
     if (int rc = ensure_dynamic_smem(kern, sh, granted)) return rc;
     int prio_high = 0;
@@ -1327,10 +1141,6 @@ template <class M>
 static size_t ws_block_bytes(int64_t P, int64_t T) {
     return ((size_t)((P + 15) / 16 * 16) * (size_t)T * BlockLayout<M::NDOF>::NW * sizeof(float) + 255) / 256 * 256;
 }
-// flags + ticket of the fused elimination, behind the blocks
-static size_t ws_tail_bytes(int64_t P) {
-    return ((size_t)grid_for(P, ABLOCK) * 2 * (ABLOCK / 32) + 64) * sizeof(int);
-}
 // segments of the segmented solve asked for by the flags (0 = the twisted solve): at least 4 waypoints per segment
 static int seg_count(int64_t T, int flags) {
     int64_t n = (flags >> CPPFLOW_LM_SEGMENTS_SHIFT) & 0xff;
@@ -1346,20 +1156,20 @@ template <class M>
 static size_t ws_seg_x_bytes(int64_t P, int S) {
     return ((size_t)((P + 15) / 16) * (S - 1) * SegLayout<M::NDOF>::x_f4() * 16 + 255) / 256 * 256;
 }
-// [blocks][flags + ticket of the fused elimination][segmented solve: factors | corners | separator solutions]
+// [blocks][segmented solve: factors | corners | separator solutions]; the blocks are a multiple of 256 bytes
 template <class M>
 static size_t ws_bytes(int64_t P, int64_t T, int flags = 0) {
-    const size_t n = ws_block_bytes<M>(P, T) + ws_tail_bytes(P);
-    const int S = (flags & CPPFLOW_LM_FUSED) ? 0 : seg_count(T, flags);
+    const size_t n = ws_block_bytes<M>(P, T);
+    const int S = seg_count(T, flags);
     if (S == 0) return n;
-    return (n + 255) / 256 * 256 + ws_block_bytes<M>(P, T) + ws_seg_corner_bytes<M>(P, S) + ws_seg_x_bytes<M>(P, S);
+    return 2 * n + ws_seg_corner_bytes<M>(P, S) + ws_seg_x_bytes<M>(P, S);
 }
 
 template <class M>
 static int launch_solve_segmented(const SolveParams& sp, const float* q, int64_t P, int64_t T, int S, bool high_priority,
                                   float* ws, float* x_out, cudaStream_t st) {
     unsigned char* base = reinterpret_cast<unsigned char*>(ws);
-    size_t off = (ws_block_bytes<M>(P, T) + ws_tail_bytes(P) + 255) / 256 * 256;
+    size_t off = ws_block_bytes<M>(P, T);
     float* fac = reinterpret_cast<float*>(base + off);
     off += ws_block_bytes<M>(P, T);
     float* corners = reinterpret_cast<float*>(base + off);
@@ -1368,10 +1178,6 @@ static int launch_solve_segmented(const SolveParams& sp, const float* q, int64_t
     const SegGeom geo{(int)T, S};
     const int64_t warps = (P + 15) / 16 * S;
     constexpr int W = 1;  // single-warp CTAs spread the chains over the SMs' schedulers (as the register-resident solve)
-    static const int passes = [] {  // debug (tools/probe_segsolve.py): stop after pass 1 / 2 to time the passes live
-        const char* e = std::getenv("CPPFLOW_SEG_PASSES");
-        return e ? std::atoi(e) : 3;
-    }();
     // CPPFLOW_LM_OVERLAP: the passes of one chunk run while another chunk's assembly fills the SMs; with the highest
     // launch priority their single-warp CTAs take the registers of every assembly CTA that retires
     cudaLaunchConfig_t cfg = {};
@@ -1391,7 +1197,6 @@ static int launch_solve_segmented(const SolveParams& sp, const float* q, int64_t
     cfg.dynamicSmemBytes = 0;
     const float* ws_c = ws;
     if (int rc = launched(cudaLaunchKernelEx(&cfg, lm_seg_eliminate_kernel<M, W>, P, geo, sp, ws_c, fac, corners), "lm_seg_eliminate")) return rc;
-    if (passes < 2) return CPPFLOW_OK;
     const size_t sh = seg_reduced_smem<M::NDOF>(S);
     static SmemGrant granted;  // per template instantiation and device
     if (int rc = ensure_dynamic_smem(lm_seg_reduced_kernel<M>, seg_reduced_smem<M::NDOF>(SEG_MAX_SEGMENTS), granted)) return rc;
@@ -1400,7 +1205,6 @@ static int launch_solve_segmented(const SolveParams& sp, const float* q, int64_t
     cfg.blockDim = dim3(32 * SEG_REDUCED_WARPS);
     cfg.dynamicSmemBytes = sh;
     if (int rc = launched(cudaLaunchKernelEx(&cfg, lm_seg_reduced_kernel<M>, P, geo, sp, ws_c, corners_c, sepx), "lm_seg_reduced")) return rc;
-    if (passes < 3) return CPPFLOW_OK;
     const float* sepx_c = sepx;
     // pass 3 out of shared memory when a half-segment's factors fit (T / S <= ~70): every load in flight at once
     int half = 0;
@@ -1409,8 +1213,7 @@ static int launch_solve_segmented(const SolveParams& sp, const float* q, int64_t
         half = len / 2 > half ? len / 2 : half;
     }
     const size_t stage_bytes = (size_t)(half > 0 ? half : 1) * seg_stage_floats<M::NDOF>() * sizeof(float);
-    static const bool no_stage = std::getenv("CPPFLOW_SEG_NO_STAGE") != nullptr;  // A/B switch (tools/probe_segsolve.py)
-    if (stage_bytes <= 200 * 1024 && !no_stage) {
+    if (stage_bytes <= 200 * 1024) {
         static SmemGrant granted3;  // per template instantiation and device
         if (int rc = ensure_dynamic_smem(lm_seg_substitute_staged_kernel<M>, 200 * 1024, granted3)) return rc;
         const float* fac_c = fac;
@@ -1441,45 +1244,16 @@ static int launch_solve(const cppflow_lm_params* p, const float* q, int64_t P, i
         lm_block_solve_resident_kernel<M><<<(unsigned)P, 32, sh, st>>>(q, P, T, sp, ws, x_out);
         return CPPFLOW_OK;
     }
-    // CPPFLOW_SOLVE = "tma" keeps the ring kernel for every path count (A/B of the two kernels, tools/probe_solve.py);
-    // the other variants measured in round 2 (8 or 1 warps per CTA, the register-resident kernel with 2 / 4 / 8 warps or
-    // without prefetch) are in profiles/r02_notes.md
-    static const char* which = std::getenv("CPPFLOW_SOLVE");
     // few paths: the chain latency is all there is, and the register-resident kernel's step is the shortest (no ring
     // bookkeeping): P = 512 alone 0.128 ms against 0.21; under overlap it only wins for chunks of <= 256 paths
     // (4 chunks of 256: 0.203 ms per iteration against 0.254, of 512: 0.337 against 0.286).  Bit-identical either way.
+    // The other variants measured in round 2 (8 or 1 warps per CTA, the register-resident kernel with 2 / 4 / 8 warps
+    // or without prefetch) are in profiles/r02_notes.md.
     const bool overlap = (flags & CPPFLOW_LM_OVERLAP) != 0;
-    if (!which && P <= (overlap ? SOLVE_V2_MAX_PATHS_OVERLAP : SOLVE_V2_MAX_PATHS_ALONE))
+    if (P <= (overlap ? SOLVE_V2_MAX_PATHS_OVERLAP : SOLVE_V2_MAX_PATHS_ALONE))
         return launch_solve_v2<M, 1, true>(sp, q, P, T, overlap, ws, x_out, st);
     if (overlap) return launch_solve_variant<M, SOLVE_RING_OVERLAP>(sp, q, P, T, true, ws, x_out, st);
     return launch_solve_variant<M, SOLVE_RING_ALONE>(sp, q, P, T, false, ws, x_out, st);
-}
-
-// CPPFLOW_LM_FUSED: assembly + elimination in one kernel (FuseParams above), then the back-substitution
-template <class M>
-static int launch_fused_step(const cppflow_lm_params* p, const float* q, const float* xv, const float* target, int64_t P,
-                             int64_t T, const Obstacles& ob, int flags, float* ws, float* x_out, cudaStream_t st) {
-    AssembleParams ap;
-    SolveParams sp;
-    make_params<M>(p, ob.n, flags & CPPFLOW_LM_CLAMP, ap, sp);
-    ap.prefetch = 0;  // rows are not taken in waypoint order
-    const size_t sh = sizeof(float) * ABLOCK * SmemLayout<M>::N_FULL;
-    static SmemGrant granted;  // per template instantiation and device
-    if (int rc = ensure_dynamic_smem(lm_assemble_kernel<M, true>, sh, granted)) return rc;
-    FuseParams fz;
-    int* tail = reinterpret_cast<int*>(reinterpret_cast<unsigned char*>(ws) + ws_block_bytes<M>(P, T));
-    fz.npb = (int)grid_for(P, ABLOCK);
-    fz.flags = tail + 64;
-    fz.ticket = tail;
-    fz.q = q;
-    fz.x_out = x_out;
-    fz.sp = sp;
-    cudaError_t e = cudaMemsetAsync(tail, 0, ws_tail_bytes(P), st);
-    if (e != cudaSuccess) return fail(CPPFLOW_E_CUDA, "lm_full fused: memset: %s", cudaGetErrorString(e));
-    lm_assemble_kernel<M, true><<<dim3((unsigned)(fz.npb * T)), ABLOCK, sh, st>>>(q, xv, target, (int)P, (int)T, ob, ap, ws, fz);
-    if (T < 2) return CPPFLOW_OK;  // a single waypoint is the middle block: nothing to back-substitute
-    if (flags & CPPFLOW_LM_OVERLAP) return launch_solve_variant<M, SOLVE_RING_OVERLAP, SOLVE_WARPS_DEFAULT, true>(sp, q, P, T, true, ws, x_out, st);
-    return launch_solve_variant<M, SOLVE_RING_ALONE, SOLVE_WARPS_DEFAULT, true>(sp, q, P, T, false, ws, x_out, st);
 }
 
 }  // namespace cppflow
@@ -1499,6 +1273,10 @@ extern "C" size_t cppflow_lm_full_workspace_bytes_ex(int robot, int64_t P, int64
 extern "C" size_t cppflow_lm_full_workspace_bytes(int robot, int64_t P, int64_t T) {
     return cppflow_lm_full_workspace_bytes_ex(robot, P, T, 0);
 }
+
+// the bits of `do_clamp` that cppflow_lm_full_step / cppflow_lm_full_solve know; any other bit is rejected, so that a
+// caller still passing a removed option gets an error instead of a step computed some other way
+constexpr int LM_KNOWN_FLAGS = CPPFLOW_LM_CLAMP | CPPFLOW_LM_OVERLAP | CPPFLOW_LM_SEGMENTS(0xff);
 
 static int check_common(int robot, const cppflow_lm_params* params, int64_t P, int64_t T, const void* d_workspace,
                         size_t workspace_bytes, int flags = 0) {
@@ -1536,6 +1314,7 @@ extern "C" int cppflow_lm_full_assemble(int robot, const cppflow_lm_params* para
 extern "C" int cppflow_lm_full_solve(int robot, const cppflow_lm_params* params, const float* d_q, int64_t P, int64_t T,
                                      int do_clamp, void* d_workspace, size_t workspace_bytes, float* d_x_out,
                                      void* stream) {
+    CPPFLOW_CHECK_ARG((do_clamp & ~LM_KNOWN_FLAGS) == 0, "unknown do_clamp bits");
     if (P == 0 || T == 0) return CPPFLOW_OK;
     if (int rc = check_common(robot, params, P, T, d_workspace, workspace_bytes, do_clamp)) return rc;
     CPPFLOW_CHECK_ARG(d_q && d_x_out, "null pointer");
@@ -1551,21 +1330,7 @@ extern "C" int cppflow_lm_full_step(int robot, const cppflow_lm_params* params, 
                                     const float* d_target, int64_t P, int64_t T, const float* h_cuboids,
                                     const float* h_Tcuboids, int n_obstacles, int do_clamp, void* d_workspace,
                                     size_t workspace_bytes, float* d_x_out, void* stream) {
-    if (do_clamp & CPPFLOW_LM_FUSED) {
-        if (P == 0 || T == 0) return CPPFLOW_OK;
-        if (int rc = check_common(robot, params, P, T, d_workspace, workspace_bytes)) return rc;
-        CPPFLOW_CHECK_ARG(d_q && d_x_out, "null pointer");
-        CPPFLOW_CHECK_ARG(!params->use_pose || d_target, "target path required when use_pose");
-        CPPFLOW_CHECK_ARG(P * T < ((int64_t)1 << 31) / 2, "P * T too large for the fused elimination's ticket counter");
-        Obstacles ob;
-        if (int rc = make_obstacles(h_cuboids, h_Tcuboids, n_obstacles, ob)) return rc;
-        int rc = CPPFLOW_OK;
-        CPPFLOW_DISPATCH_ROBOT(robot, rc = launch_fused_step<M>(params, d_q, d_xv, d_target, P, T, ob, do_clamp, (float*)d_workspace,
-                                                                d_x_out, (cudaStream_t)stream));
-        if (rc) return rc;
-        CPPFLOW_CHECK_LAUNCH();
-        return CPPFLOW_OK;
-    }
+    CPPFLOW_CHECK_ARG((do_clamp & ~LM_KNOWN_FLAGS) == 0, "unknown do_clamp bits");
     if (int rc = cppflow_lm_full_assemble(robot, params, d_q, d_xv, d_target, P, T, h_cuboids, h_Tcuboids, n_obstacles,
                                           d_workspace, workspace_bytes, stream))
         return rc;

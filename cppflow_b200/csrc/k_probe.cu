@@ -20,39 +20,9 @@ __global__ void __launch_bounds__(1024) fp32_probe_kernel(int iters, float* __re
     if (s == 12345.678f) out[0] = s;  // keep the chains alive
 }
 
-// Stand-in neighbour for co-residency experiments (tools/probe_coresident.py): 256-thread CTAs running FMA chains with
-// `smem_bytes` of dynamic shared memory that is either never touched (touch = 0: only the carve-out is taken from the
-// L1) or used like the assembly's column (touch = n: n scalar stores + loads per inner iteration).
-__global__ void __launch_bounds__(256, 2) neighbour_probe_kernel(int iters, int touch, int slots, float* __restrict__ out) {
-    extern __shared__ __align__(16) float nb_smem[];
-    float a0 = threadIdx.x * 1e-3f, a1 = a0 + 1.f, a2 = a0 + 2.f, a3 = a0 + 3.f;
-    const float m = 0.999f, c = 1e-3f;
-    float* col = nb_smem + threadIdx.x;
-    for (int i = 0; i < iters; ++i) {
-#pragma unroll
-        for (int u = 0; u < 8; ++u) { a0 = fmaf(a0, m, c); a1 = fmaf(a1, m, c); a2 = fmaf(a2, m, c); a3 = fmaf(a3, m, c); }
-        for (int k = 0; k < touch; ++k) {
-            const int s = (i + k) % slots;
-            col[s * 256] = a0;
-            a1 += col[((s + 7) % slots) * 256];
-        }
-    }
-    const float s = a0 + a1 + a2 + a3;
-    if (s == 12345.678f) out[0] = s;
-}
-
 }  // namespace cppflow
 
 using namespace cppflow;
-
-extern "C" int cppflow_neighbour_probe(int blocks, int iters, int smem_bytes, int touch, float* d_scratch, void* stream) {
-    CPPFLOW_CHECK_ARG(blocks > 0 && iters > 0 && d_scratch && smem_bytes >= 4096, "blocks, iters, scratch, smem");
-    static SmemGrant granted;
-    if (int rc = ensure_dynamic_smem(neighbour_probe_kernel, 110 * 1024, granted)) return rc;
-    neighbour_probe_kernel<<<blocks, 256, smem_bytes, (cudaStream_t)stream>>>(iters, touch, smem_bytes / 1024, d_scratch);
-    CPPFLOW_CHECK_LAUNCH();
-    return CPPFLOW_OK;
-}
 
 // Launches `blocks` CTAs of 1024 threads; returns the FLOP count of the launch in *flops_out.
 extern "C" int cppflow_fp32_probe(int blocks, int iters, float* d_scratch, double* flops_out, void* stream) {

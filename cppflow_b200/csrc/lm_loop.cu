@@ -11,7 +11,6 @@
 #include <atomic>
 #include <chrono>
 #include <cmath>
-#include <cstdlib>
 #include <vector>
 
 #include "common.cuh"
@@ -23,15 +22,9 @@ namespace {
 inline size_t align256(size_t n) { return (n + 255) / 256 * 256; }
 
 // The differencing step of ONE path is the block solve's dependent chain and nothing else: it takes the segmented
-// solve (csrc/lm_segsolve.cuh; 0.098 -> 0.046 ms for T = 300).  CPPFLOW_LOOP_SEGMENTS = 0 restores the twisted solve.
-inline int loop_step_flags() {
-    static const int segments = [] {
-        const char* e = std::getenv("CPPFLOW_LOOP_SEGMENTS");
-        const int n = e ? std::atoi(e) : 16;
-        return n < 0 ? 0 : n > 255 ? 255 : n;
-    }();
-    return CPPFLOW_LM_CLAMP | CPPFLOW_LM_SEGMENTS(segments);
-}
+// solve (csrc/lm_segsolve.cuh; 0.098 -> 0.046 ms for T = 300) with 16 segments.  ops.LOOP_SEGMENTS must be the same
+// number: the Python loop then takes the same solve and returns the same bits.
+constexpr int LOOP_STEP_FLAGS = CPPFLOW_LM_CLAMP | CPPFLOW_LM_SEGMENTS(16);
 
 struct LoopLayout {
     size_t x_bytes, off_xa, off_xb, off_valid, off_metrics, off_lm, total;
@@ -43,7 +36,7 @@ struct LoopLayout {
         off_valid = off_xb + x_bytes;
         off_metrics = off_valid + x_bytes;
         off_lm = off_metrics + 256;
-        total = off_lm + align256(cppflow_lm_full_workspace_bytes_ex(robot, 1, T, loop_step_flags()));
+        total = off_lm + align256(cppflow_lm_full_workspace_bytes_ex(robot, 1, T, LOOP_STEP_FLAGS));
     }
 };
 
@@ -82,7 +75,6 @@ struct LoopState {
     float tag = 0.f;               // completion tag of the iteration in flight: (per-call nonce << 8) + (i mod 255) + 1
     unsigned nonce = 0;            // distinguishes this call's tags from stale ones of an earlier (failed) call that
                                    // shared the pinned buffer; < 2^12, so every tag is an exact float below 2^20
-    bool fuse_pose = std::getenv("CPPFLOW_LM_NO_FUSE") == nullptr;  // pose step + metrics in one launch
     float* metrics_dst = nullptr;  // where the metrics kernel writes: the pinned host buffer itself when the device can
     bool zero_copy = false;        // address it (no copy engine round trip per iteration), the device scratch otherwise
 
@@ -129,10 +121,10 @@ struct LoopState {
         if (pose_pos_valid && pose_rot_valid) {
             // virtual configs = the current iterate (:253): their residual is identically zero -> d_xv = NULL
             if (int rc = cppflow_lm_full_step(j->robot, j->params_diff, x_cur, nullptr, j->d_target, 1, j->T, j->h_cuboids,
-                                              j->h_Tcuboids, j->n_obstacles, loop_step_flags(), lm_ws, lm_ws_bytes, x_new, j->stream))
+                                              j->h_Tcuboids, j->n_obstacles, LOOP_STEP_FLAGS, lm_ws, lm_ws_bytes, x_new, j->stream))
                 return rc;
             was_differencing = true;
-        } else if (fuse_pose && j->T <= 1024) {
+        } else if (j->T <= 1024) {
             // pose-only step and the metrics of its result in ONE launch (both kernels are launch-bound for one path)
             if (int rc = pose_step_metrics_tagged(j->robot, j->params_pose, x_cur, j->d_target, j->T, j->h_cuboids, j->h_Tcuboids,
                                                   j->n_obstacles, x_new, metrics_dst, tag, j->stream))

@@ -30,17 +30,12 @@ def _on_device(fn):
 
 
 ROBOT_IDS = {"fetch": 0, "fetch_arm": 1, "panda": 2}
-LM_CLAMP, LM_OVERLAP, LM_FUSED = 1, 2, 4  # CPPFLOW_LM_CLAMP / _OVERLAP / _FUSED (include/cppflow_b200.h)
+LM_CLAMP, LM_OVERLAP = 1, 2  # CPPFLOW_LM_CLAMP / _OVERLAP (include/cppflow_b200.h)
 
-
-def loop_segments() -> int:
-    """Segments of the single-path full step (the differencing step of run_lm_alternating_loss): the native loop
-    (csrc/lm_loop.cu: loop_step_flags) and the Python loop must take the same solve to return the same bits.
-    CPPFLOW_LOOP_SEGMENTS = 0 restores the twisted solve in both."""
-    import os
-
-    n = int(os.environ.get("CPPFLOW_LOOP_SEGMENTS", "16"))
-    return min(max(n, 0), 255)
+# Segments of the single-path full step (the differencing step of run_lm_alternating_loss).  Must equal the segment
+# count of LOOP_STEP_FLAGS in csrc/lm_loop.cu: the native loop and the Python loop then take the same solve and return
+# the same bits.
+LOOP_SEGMENTS = 16
 
 
 def lm_segments(n: int) -> int:
@@ -251,11 +246,10 @@ def _workspace(device, nbytes: int, key: str) -> torch.Tensor:
 def lm_full_step(rid: int, ndof: int, params: LmParamsC, q: torch.Tensor, xv: Optional[torch.Tensor],
                  target: Optional[torch.Tensor], P: int, T: int, ob: Optional[Obstacles], clamp: bool,
                  out: Optional[torch.Tensor] = None, overlap: bool = False,
-                 workspace: Optional[torch.Tensor] = None, fused: bool = False, segments: int = 0) -> torch.Tensor:
-    """levenberg_marquardt_full (+ clamp) for P paths of T waypoints on the current stream.  `fused`: CPPFLOW_LM_FUSED
-    (elimination inside the assembly kernel, same bits).  `segments`: CPPFLOW_LM_SEGMENTS (parallel-in-time solve for
-    few paths, csrc/lm_segsolve.cuh; rounding-level differences, larger workspace).  `overlap`: launch the
-    solve with CPPFLOW_LM_OVERLAP (footprint that fits next to an assembly CTA, high launch priority) - for callers that run several chunks
+                 workspace: Optional[torch.Tensor] = None, segments: int = 0) -> torch.Tensor:
+    """levenberg_marquardt_full (+ clamp) for P paths of T waypoints on the current stream.  `segments`:
+    CPPFLOW_LM_SEGMENTS (parallel-in-time solve for few paths, csrc/lm_segsolve.cuh; rounding-level differences, larger
+    workspace).  `overlap`: launch the solve with CPPFLOW_LM_OVERLAP (footprint that fits next to an assembly CTA, high launch priority) - for callers that run several chunks
     of paths on several streams (pipeline.ResidentPipeline), which must also pass one `workspace` per stream."""
     q = _check_q(q, ndof)
     assert q.shape[0] == P * T, f"x must have P*T = {P * T} rows, has {q.shape[0]}"
@@ -266,7 +260,7 @@ def lm_full_step(rid: int, ndof: int, params: LmParamsC, q: torch.Tensor, xv: Op
         target = require_cuda(target, "target_path")
         assert target.shape == (T, 7), f"target_path must be [{T}, 7], is {tuple(target.shape)}"
     lib = _lib.load()
-    flags = (LM_CLAMP if clamp else 0) | (LM_OVERLAP if overlap else 0) | (LM_FUSED if fused else 0) | lm_segments(segments)
+    flags = (LM_CLAMP if clamp else 0) | (LM_OVERLAP if overlap else 0) | lm_segments(segments)
     nbytes = lib.cppflow_lm_full_workspace_bytes_ex(rid, P, T, flags)
     if workspace is None:
         ws = _workspace(q.device, nbytes, "lm_full")

@@ -83,7 +83,7 @@ def levenberg_marquardt_full(opt_problem: OptimizationProblem, opt_state: Optimi
     x_new = ops.lm_full_step(robot.robot_id, robot.ndof, ops.make_params(opt_params), opt_state.x, xv,
                              problem.target_path, opt_problem.parallel_count, problem.n_timesteps,
                              problem.obstacle_tables, clamp,
-                             segments=ops.loop_segments() if opt_problem.parallel_count == 1 else 0)
+                             segments=ops.LOOP_SEGMENTS if opt_problem.parallel_count == 1 else 0)
     if return_residual:
         assert opt_problem.parallel_count == 1, "dense residuals are only built for a single path"
         jac, res = LmResidualFns.get_r_and_J(opt_params, robot, opt_state.x, problem.target_path,

@@ -202,26 +202,6 @@ def split_paths(n_paths: int, n_chunks: int):
     return chunks
 
 
-class SmPartition:
-    """Two CUDA green contexts splitting the SMs of a device (cppflow_sm_partition_create) and streams in each:
-    `first` has at least `min_sms_first` SMs, `second` the rest.  Partitions live until the process ends."""
-
-    def __init__(self, device, min_sms_first: int, n_streams_first: int, n_streams_second: int):
-        import ctypes as C
-
-        device = torch.device(device)
-        lib = ops._lib.load()
-        a1 = (C.c_void_p * max(1, n_streams_first))()
-        a2 = (C.c_void_p * max(1, n_streams_second))()
-        s1, s2 = C.c_int(0), C.c_int(0)
-        torch.cuda.current_stream(device)  # primary context initialised
-        ops.check(lib.cppflow_sm_partition_create(device.index or 0, int(min_sms_first), n_streams_first, n_streams_second,
-                                                  a1, a2, C.byref(s1), C.byref(s2)))
-        self.sms_first, self.sms_second = s1.value, s2.value
-        self.streams_first = [torch.cuda.ExternalStream(a1[i], device=device) for i in range(n_streams_first)]
-        self.streams_second = [torch.cuda.ExternalStream(a2[i], device=device) for i in range(n_streams_second)]
-
-
 class ResidentPipeline:
     """LM iterations over device-resident paths with the two kernels of the step overlapped across path chunks.
 
@@ -235,14 +215,11 @@ class ResidentPipeline:
     Chunks are multiples of 256 paths (the assembly CTA) where P allows."""
 
     def __init__(self, problem: Problem, n_paths: int, params: Optional[OptimizationParameters] = None,
-                 n_chunks: Optional[int] = None, device=None, overlap: bool = True, solve_sms: Optional[int] = None,
-                 segments=0):
+                 n_chunks: Optional[int] = None, device=None, overlap: bool = True, segments=0):
         """`segments`: time segments of the segmented solve (CPPFLOW_LM_SEGMENTS, csrc/lm_segsolve.cuh; 0 = the twisted
         solve).  For <= ~2000 paths per GPU the twisted solve's chain of T dependent steps is most of the iteration; the
         segmented solve's result differs by rounding and depends on `segments` only, not on the chunking.  "auto": 16
-        segments up to 2048 paths (where it is faster), the twisted solve above.
-        `solve_sms`: instead of sharing SMs, give the block solves `solve_sms` SMs of their own (a green-context
-        partition) and the assembly the rest: the solves then run at their stand-alone speed and displace nothing."""
+        segments up to 2048 paths (where it is faster), the twisted solve above."""
         self.problem = problem
         self.robot = problem.robot
         self.T = problem.n_timesteps
@@ -267,55 +244,25 @@ class ResidentPipeline:
         self.chunks = split_paths(n_paths, n_chunks)
         if len(self.chunks) == 1:
             self.overlap = False  # nothing to run under: the stand-alone solve variants are faster
-        self.partition = None
-        if solve_sms:
-            self.partition = SmPartition(self.device, solve_sms, len(self.chunks), len(self.chunks))
-            self.solve_streams = self.partition.streams_first   # the small partition
-            self.streams = self.partition.streams_second        # assembly: the rest of the SMs
-            self.ev_asm = [torch.cuda.Event() for _ in self.chunks]
-            self.ev_solve = [torch.cuda.Event() for _ in self.chunks]
-        else:
-            self.streams = [torch.cuda.Stream(self.device) for _ in self.chunks]
+        self.streams = [torch.cuda.Stream(self.device) for _ in self.chunks]
         lib = ops._lib.load()
         self.ws = [torch.empty((lib.cppflow_lm_full_workspace_bytes_ex(self.robot.robot_id, n, self.T, ops.lm_segments(segments)),),
                                device=self.device, dtype=torch.uint8) for _, n in self.chunks]
 
-    def _all_streams(self):
-        return self.streams + (self.solve_streams if self.partition is not None else [])
-
     def begin(self):
         cur = torch.cuda.current_stream(self.device)
-        for s in self._all_streams():
+        for s in self.streams:
             s.wait_stream(cur)
-        if self.partition is not None:
-            for ev, s in zip(self.ev_solve, self.solve_streams):
-                ev.record(s)
 
     def end(self):
         cur = torch.cuda.current_stream(self.device)
-        for s in self._all_streams():
+        for s in self.streams:
             cur.wait_stream(s)
 
     def enqueue_step(self, x: torch.Tensor, out: torch.Tensor, clamp: bool = True):
         """One LM iteration x -> out ([P*T, D] device tensors) for every chunk, each on its own stream; call between
         begin() and end().  Steps enqueued back to back pipeline across chunks."""
         T, D, rid = self.T, self.robot.ndof, self.robot.robot_id
-        if self.partition is not None:
-            lib = ops._lib.load()
-            cu, tc, no = ops._obs(self.problem.obstacle_tables)
-            flags = (ops.LM_CLAMP if clamp else 0) | (ops.LM_OVERLAP if self.overlap else 0) | ops.lm_segments(self.segments)  # overlap: the 4-slot ring
-            for c, ((p0, n), ws) in enumerate(zip(self.chunks, self.ws)):
-                sl = slice(p0 * T, (p0 + n) * T)
-                sa, ss = self.streams[c], self.solve_streams[c]
-                sa.wait_event(self.ev_solve[c])  # the chunk's previous solve has read the workspace and written x
-                ops.check(lib.cppflow_lm_full_assemble(rid, self.prm, ops.ptr(x[sl]), None, ops.ptr(self.problem.target_path), n, T,
-                                                       cu, tc, no, ops.ptr(ws), ws.numel(), sa.cuda_stream))
-                self.ev_asm[c].record(sa)
-                ss.wait_event(self.ev_asm[c])
-                ops.check(lib.cppflow_lm_full_solve(rid, self.prm, ops.ptr(x[sl]), n, T, flags, ops.ptr(ws), ws.numel(),
-                                                    ops.ptr(out[sl]), ss.cuda_stream))
-                self.ev_solve[c].record(ss)
-            return
         # straight through the C ABI on each chunk's stream (the ops wrapper costs ~20 us of host time per call: with six
         # chunks that is a quarter of the step)
         lib = ops._lib.load()
@@ -337,8 +284,7 @@ class ResidentPipeline:
         T, D, rid = self.T, self.robot.ndof, self.robot.robot_id
         lib = ops._lib.load()
         cu, tc, no = ops._obs(self.problem.obstacle_tables)
-        last = self.solve_streams if self.partition is not None else self.streams  # where a chunk's last solve ran
-        for (p0, n), s in zip(self.chunks, last):
+        for (p0, n), s in zip(self.chunks, self.streams):
             ops.check(lib.cppflow_path_metrics_ex(rid, ops.ptr(x[p0 * T:(p0 + n) * T]), ops.ptr(self.problem.target_path), n, T,
                                                   cu, tc, no, ops.METRICS_SIGN_ONLY if sign_only else 0,
                                                   ops.ptr(metrics[p0:p0 + n]), s.cuda_stream))

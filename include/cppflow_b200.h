@@ -83,7 +83,7 @@ const char* cppflow_last_error(void);
  * cppflow_robot_info, cppflow_constraints, cppflow_lm_loop_result, cppflow_lm_loop_job (as many as fit in n).
  * Returns the number of values the library knows (6).  A binding compares them with its own struct sizes after
  * dlopen and refuses a library built from another header. */
-#define CPPFLOW_ABI_VERSION 4
+#define CPPFLOW_ABI_VERSION 5
 int cppflow_abi_info(int64_t* out, int n);
 
 /* jrl.Robot properties (ndof, actuated_joints_limits, prismatic_joint_idxs, _collision_capsules_by_link). */
@@ -137,7 +137,9 @@ int cppflow_collision_flags(int robot, const float* d_q, int64_t n, const float*
  * waypoints (optimization.py:95-144, optimization_utils.py:486-731).  The normal equations are assembled
  * implicitly as a symmetric block-tridiagonal system (ndof x ndof blocks) and solved by block Cholesky.
  * d_xv = virtual configs [P,T,ndof] (NULL: equal to x, the run_lm_alternating_loss case, optimization.py:253).
- * Workspace: cppflow_lm_full_workspace_bytes(robot, P, T) bytes of device memory. */
+ * Workspace: cppflow_lm_full_workspace_bytes(robot, P, T) bytes of device memory, 16-byte aligned: the packed
+ * (A_tt, b_t) blocks of the paths in 16-path groups, rounded up to 256 bytes; with CPPFLOW_LM_SEGMENTS the segmented
+ * solve's factors, corner blocks and separator solutions follow (cppflow_lm_full_workspace_bytes_ex). */
 size_t cppflow_lm_full_workspace_bytes(int robot, int64_t P, int64_t T);
 int cppflow_lm_full_step(int robot, const cppflow_lm_params* params, const float* d_q, const float* d_xv,
                          const float* d_target, int64_t P, int64_t T, const float* h_cuboids, const float* h_Tcuboids,
@@ -160,18 +162,15 @@ int cppflow_lm_full_solve(int robot, const cppflow_lm_params* params, const floa
  * assembly of another chunk of paths enqueued on another stream (same results bit for bit). */
 #define CPPFLOW_LM_CLAMP 1
 #define CPPFLOW_LM_OVERLAP 2
-/* cppflow_lm_full_step only: the assembly CTA of a waypoint also takes the elimination step of that waypoint (the chain
- * runs from CTA to CTA through L2), so the (A, b) blocks never reach HBM; the solve then only back-substitutes.  Same
- * results bit for bit. */
-#define CPPFLOW_LM_FUSED 4
 /* cppflow_lm_full_step / cppflow_lm_full_solve: bits 8..15 of `do_clamp` ask for the SEGMENTED solve with that many
  * time segments per path (csrc/lm_segsolve.cuh): the segments between S - 1 separator waypoints are eliminated in
  * parallel, the separators' reduced block-tridiagonal system is solved, the segments are back-substituted in parallel.
  * For few paths (<= ~2000) the twisted solve's dependent chain of T steps is the whole solve time; this one's chain is
  * ~ T / S heavy + S + T / S light steps.  The result differs from the twisted solve's by rounding only and depends on
  * S, not on P or the chunking.  S is reduced to T / 4 for short paths (fewer than 2 segments: the twisted solve).
- * Needs the larger workspace of cppflow_lm_full_workspace_bytes_ex(robot, P, T, flags).  Ignored with
- * CPPFLOW_LM_FUSED. */
+ * Needs the larger workspace of cppflow_lm_full_workspace_bytes_ex(robot, P, T, flags).
+ * Bits of `do_clamp` other than CPPFLOW_LM_CLAMP, CPPFLOW_LM_OVERLAP and CPPFLOW_LM_SEGMENTS are rejected with
+ * CPPFLOW_E_INVALID. */
 #define CPPFLOW_LM_SEGMENTS_SHIFT 8
 #define CPPFLOW_LM_SEGMENTS(n) (((n) & 0xff) << CPPFLOW_LM_SEGMENTS_SHIFT)
 size_t cppflow_lm_full_workspace_bytes_ex(int robot, int64_t P, int64_t T, int flags);
@@ -272,13 +271,6 @@ int cppflow_path_metrics_ex(int robot, const float* d_q, const float* d_target, 
  * valid paths, first_index} - what each rank contributes to the all-gather. */
 int cppflow_path_key_argmin(const float* d_metrics, int64_t P, const cppflow_constraints* constraints,
                             int64_t first_index, int64_t* d_out, void* stream);
-
-/* Splits the SMs of `device` into two green contexts - the first with at least `min_sms_first` SMs (rounded up to the
- * architecture's granularity, 8 on sm_90+), the second with the rest - and creates streams in each.  Kernels launched
- * on a stream only run on its partition's SMs.  Used by the chunk-pipelined LM iteration to give the block solves a few
- * SMs of their own while the assembly owns the rest (no reference counterpart). */
-int cppflow_sm_partition_create(int device, int min_sms_first, int n_streams_first, int n_streams_second,
-                                void** streams_first, void** streams_second, int* sms_first, int* sms_second);
 
 /* IKFlow's conditional GLOW network (ikflow/model.py: glow_cNF_model; restated in oracle/ikflow.py), the candidate
  * generator of the reference (planners.py:116-189).  Forward (x -> z) or reverse (z -> x) pass over n rows; row i is
@@ -426,9 +418,6 @@ int cppflow_ik_select(int robot, const float* d_q, const uint8_t* d_status, cons
 /* Measurement aid (no reference counterpart): dependent-free FP32 FMA loop on `blocks` x 1024 threads, used by
  * bench.py to measure the FP32 roofline denominator on the box.  *flops_out = FLOPs of the launch. */
 int cppflow_fp32_probe(int blocks, int iters, float* d_scratch, double* flops_out, void* stream);
-/* Measurement aid (no reference counterpart): a stand-in neighbour kernel for co-residency experiments - 256-thread CTAs
- * of FMA chains holding `smem_bytes` of shared memory, untouched (touch = 0) or accessed `touch` times per iteration. */
-int cppflow_neighbour_probe(int blocks, int iters, int smem_bytes, int touch, float* d_scratch, void* stream);
 
 #ifdef __cplusplus
 }

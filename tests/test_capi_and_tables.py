@@ -37,26 +37,44 @@ def test_struct_layouts_match_header():
     assert ctypes.sizeof(_lib.RobotInfoC) == 4 * 4 + 8 * 4 * 3 + 10 * 7 * 4 + 10 * 4 + 28 * 2 * 4 + 16
 
 
-def test_error_codes_without_gpu():
+def test_error_codes_and_workspace_sizes_without_gpu():
     from cppflow_b200 import _lib
 
     lib = _lib.load()
     info = _lib.RobotInfoC()
     assert lib.cppflow_robot_info_get(7, info) == -1  # CPPFLOW_E_INVALID
     assert b"unknown robot id" in lib.cppflow_last_error()
-    # blocks (paths padded to 16-path groups, rounded to 256 bytes) + the flags / ticket of the fused elimination:
-    # (path blocks of 256) x 2 sides x 8 warps + 64 ints
-    assert lib.cppflow_lm_full_workspace_bytes(0, 8192, 300) == 8192 * 300 * 44 * 4 + (32 * 2 * 8 + 64) * 4
-    assert lib.cppflow_lm_full_workspace_bytes(2, 10, 20) == 16 * 20 * 36 * 4 + (1 * 2 * 8 + 64) * 4
+    # blocks (paths padded to 16-path groups, rounded to 256 bytes)
+    assert lib.cppflow_lm_full_workspace_bytes(0, 8192, 300) == 8192 * 300 * 44 * 4
+    assert lib.cppflow_lm_full_workspace_bytes(2, 10, 20) == 16 * 20 * 36 * 4
     # segmented solve (16 segments): + factor area (= blocks) + corners (2 sides x 27 float4 per segment) + 15 separators
-    base = 16 * 300 * 44 * 4 + (1 * 2 * 8 + 64) * 4
+    base = 16 * 300 * 44 * 4
     assert lib.cppflow_lm_full_workspace_bytes_ex(0, 16, 300, 16 << 8) == (
-        (base + 255) // 256 * 256 + 16 * 300 * 44 * 4 + 16 * 2 * 27 * 16 * 16 + 15 * 2 * 16 * 16)
+        base + 16 * 300 * 44 * 4 + 16 * 2 * 27 * 16 * 16 + 15 * 2 * 16 * 16)
     assert lib.cppflow_lm_full_workspace_bytes_ex(0, 16, 300, 0) == base
     assert lib.cppflow_lm_full_workspace_bytes_ex(0, 16, 6, 16 << 8) == lib.cppflow_lm_full_workspace_bytes(0, 16, 6)
     assert lib.cppflow_dp_search_workspace_bytes(175, 295) >= 4 * (295 * 175 + 294 * 175 * 175)
     with pytest.raises(_lib.CppflowError):
         _lib.check(-1)
+
+
+def test_lm_step_rejects_unknown_flags_without_gpu():
+    """A do_clamp bit outside CLAMP | OVERLAP | SEGMENTS (4 selected a removed variant) is an invalid argument, reported
+    before anything reaches the device - every other argument here would pass the checks."""
+    from cppflow_b200 import _lib
+    from cppflow_b200.lm_hyper_parameters import ALT_LOSS_V2_1_DIFF
+    from cppflow_b200.ops import make_params
+
+    lib = _lib.load()
+    P, T = 16, 20
+    nbytes = lib.cppflow_lm_full_workspace_bytes_ex(0, P, T, 4)
+    assert nbytes > 0
+    prm = make_params(ALT_LOSS_V2_1_DIFF)
+    dummy = ctypes.c_void_p(1 << 20)  # never dereferenced: non-null and 256-byte aligned
+    assert lib.cppflow_lm_full_step(0, prm, dummy, None, dummy, P, T, None, None, 0, 4, dummy, nbytes, dummy, None) == -1
+    assert b"do_clamp" in lib.cppflow_last_error()
+    assert lib.cppflow_lm_full_solve(0, prm, dummy, P, T, 4 | 1, dummy, nbytes, dummy, None) == -1
+    assert b"do_clamp" in lib.cppflow_last_error()
 
 
 @pytest.mark.parametrize("name", ["fetch", "fetch_arm", "panda"])

@@ -607,9 +607,9 @@ def _planted_paths(r, scene, P, T, seed):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("r", ROBOTS)
-def test_lm_step_vs_dense_oracle_on_crowded_scene(robots, r):
+def test_lm_step_and_overlap_launch_vs_dense_oracle_on_crowded_scene(robots, r):
     """lm_full_step (ALT_LOSS_V2_1_DIFF) on rotated8 with near-contact and second-group contacts planted against the dense
-    fp64 get_r_and_J + _lm_full_step: 1e-4 rad.  The fused and overlapped launches give the same bits; the segmented
+    fp64 get_r_and_J + _lm_full_step: 1e-4 rad.  The overlapped launch gives the same bits; the segmented
     solve stays within the tolerance of test_segmented_solve_long_paths."""
     from cppflow_b200 import ops
     from cppflow_b200.lm_hyper_parameters import ALT_LOSS_V2_1_DIFF
@@ -639,9 +639,8 @@ def test_lm_step_vs_dense_oracle_on_crowded_scene(robots, r):
         err = float((out[sl].cpu().double() - ref).abs().max())
         worst = max(worst, err)
         assert err < 1e-4, (p, err)
-    for fused, overlap in ((True, False), (True, True), (False, True)):
-        got = ops.lm_full_step(rob.robot_id, rob.ndof, prm, x, x, tg, P, T, ob, False, fused=fused, overlap=overlap)
-        assert torch.equal(got, out), (fused, overlap)
+    got = ops.lm_full_step(rob.robot_id, rob.ndof, prm, x, x, tg, P, T, ob, False, overlap=True)
+    assert torch.equal(got, out)
     seg = ops.lm_full_step(rob.robot_id, rob.ndof, prm, x, x, tg, P, T, ob, False, segments=4)
     step = float((out - x).abs().max())
     assert float((seg - out).abs().max()) < 1e-4 + 1e-3 * step

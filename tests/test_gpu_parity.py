@@ -410,29 +410,6 @@ def test_resident_solve_equals_streaming_solve(robots, r, T):
     assert torch.equal(step(x0[:3 * T].contiguous(), 3), streaming[:3 * T])
 
 
-def test_resident_pipeline_sm_partition(robots):
-    """ResidentPipeline(solve_sms=...): block solves on their own SM partition (CUDA green contexts), assembly on the
-    rest - same results as the single-stream step, for dependent iterations too."""
-    from cppflow_b200 import ops
-    from cppflow_b200.lm_hyper_parameters import all_terms_parameters
-    from cppflow_b200.pipeline import ResidentPipeline
-    from cppflow_b200.synthetic import synthetic_problem as gpu_problem, synthetic_seeds_host
-
-    rob = robots["fetch"]
-    P, T, D = 1024, 120, rob.ndof
-    problem = gpu_problem(rob, T, device=DEV)
-    _, xh = synthetic_seeds_host(rob, P, T)
-    x0 = xh.to(DEV)
-    prm = ops.make_params(all_terms_parameters())
-    seq = x0
-    for _ in range(3):
-        seq = ops.lm_full_step(rob.robot_id, D, prm, seq, None, problem.target_path, P, T, problem.obstacle_tables, True)
-    pipe = ResidentPipeline(problem, P, all_terms_parameters(), n_chunks=3, solve_sms=16)
-    assert pipe.partition.sms_first >= 16 and pipe.partition.sms_first + pipe.partition.sms_second <= 148
-    assert torch.equal(pipe.iterate(x0, 3), seq)
-    assert torch.equal(pipe.iterate(x0, 3), seq)
-
-
 @pytest.mark.parametrize("r", ROBOTS)
 def test_empty_inputs(robots, r):
     """Zero configurations / zero paths: every entry point returns an empty result of the right shape, no launch."""

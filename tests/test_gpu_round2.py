@@ -520,10 +520,11 @@ def test_resident_pipeline_graph_replay_equals_eager(robots):
 
 
 @pytest.mark.parametrize("r", ROBOTS)
-def test_fused_elimination_equals_two_kernel_step(robots, r):
-    """CPPFLOW_LM_FUSED: the assembly CTAs take the elimination steps (chain handed from CTA to CTA through L2), the solve
-    only back-substitutes.  Same bits as assembly + solve, for every path / waypoint count (one waypoint = only the middle
-    block, even / odd T, ragged path counts, more CTAs than can be resident at once) and parameter set."""
+def test_overlap_launch_equals_stand_alone_step(robots, r):
+    """CPPFLOW_LM_OVERLAP: the solve launched to run under another chunk's assembly (the 4-slot ring, the smaller
+    register-resident threshold, high priority).  Same bits as the stand-alone step, with and without clamp, for every
+    path / waypoint count (one waypoint = only the middle block, even / odd T, ragged path counts, path counts on both
+    sides of the solve kernels' thresholds) and parameter set."""
     from cppflow_b200 import ops
     from cppflow_b200.lm_hyper_parameters import all_terms_parameters, ALT_LOSS_V2_1_DIFF
 
@@ -538,12 +539,10 @@ def test_fused_elimination_equals_two_kernel_step(robots, r):
                 continue
             prm = ops.make_params(pm)
             xv = x.clone() if pm.use_virtual_configs else None
-            ref = ops.lm_full_step(rob.robot_id, rob.ndof, prm, x, xv, tg, P, T, ob, True)
-            got = ops.lm_full_step(rob.robot_id, rob.ndof, prm, x, xv, tg, P, T, ob, True, fused=True)
-            assert torch.equal(got, ref), (r, P, T, name, float((got - ref).abs().max()))
-            got2 = ops.lm_full_step(rob.robot_id, rob.ndof, prm, x, xv, tg, P, T, ob, False, fused=True, overlap=True)
-            ref2 = ops.lm_full_step(rob.robot_id, rob.ndof, prm, x, xv, tg, P, T, ob, False)
-            assert torch.equal(got2, ref2), (r, P, T, name, "no clamp / overlap variant")
+            for clamp in (True, False):
+                ref = ops.lm_full_step(rob.robot_id, rob.ndof, prm, x, xv, tg, P, T, ob, clamp)
+                got = ops.lm_full_step(rob.robot_id, rob.ndof, prm, x, xv, tg, P, T, ob, clamp, overlap=True)
+                assert torch.equal(got, ref), (r, P, T, name, clamp, float((got - ref).abs().max()))
 
 
 def _dense_step_fp64(lib, rob, prm, pm, x, tg, ob_args, P, T, paths):

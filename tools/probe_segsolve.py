@@ -1,5 +1,5 @@
 """Segmented (parallel-in-time) solve against the twisted solve: stand-alone solve time per path count and segment
-count, the difference of the results, and a per-kernel split of the three passes.  One JSON line per path count."""
+count and the difference of the results.  One JSON line per path count."""
 import json, os, sys
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))

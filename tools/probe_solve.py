@@ -1,5 +1,5 @@
-"""A/B of the block-solve variants (CPPFLOW_SOLVE read once per process): stand-alone solve time at several path counts,
-the chunk-pipelined step, and a checksum of the result (variants must be bit-identical).  One JSON line."""
+"""Block-solve timings: stand-alone solve time at several path counts (the library picks the solve kernel by path
+count), the chunk-pipelined step, and a checksum of the result (every solve kernel gives the same bits).  One JSON line."""
 import hashlib, json, os, sys, time
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -28,7 +28,7 @@ def timeit(fn, n=30):
     e1.record(); torch.cuda.synchronize()
     return e0.elapsed_time(e1) / n
 
-out = {"variant": os.environ.get("CPPFLOW_SOLVE", "tma")}
+out = {}
 ws = torch.empty((lib.cppflow_lm_full_workspace_bytes(rid, P, T),), device=dev, dtype=torch.uint8)
 for n_paths in (8192, 2048, 512, 16):
     fa = lambda: _lib.check(lib.cppflow_lm_full_assemble(rid, prm, _lib.ptr(x0), None, _lib.ptr(problem.target_path), n_paths, T, cu, tc, no, _lib.ptr(ws), ws.numel(), st))
