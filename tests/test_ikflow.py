@@ -3,11 +3,13 @@
 CPU: the oracle is invertible, the packed tables are laid out as include/cppflow_b200.h documents, the C ABI reports
 its workspace and rejects every unsupported shape.  GPU: parity with the BF16-emulating fp64 oracle and the plain
 fp32 oracle, round trip, row independence, condition broadcasting, clamp, the planner with the mock flow, and no host
-synchronisation."""
+synchronisation.  The parity, round-trip, row-independence and clamp checks also run over FLOW_SHAPES, the network
+shapes below, which tests/test_ikflow_training.py shares."""
 import ctypes
 import os
 import shutil
 import subprocess
+from dataclasses import dataclass
 
 import numpy as np
 import pytest
@@ -17,6 +19,7 @@ from oracle import ikflow as OF
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DEV = "cuda:0"
+ROBOTS = ["fetch", "fetch_arm", "panda"]
 
 
 def _limits(name):
@@ -25,17 +28,78 @@ def _limits(name):
     return R.get_model(name).actuated_joints_limits
 
 
-def _params(width=9, nb=2, H=128, L=2):
+def _params(width=9, nb=2, H=128, L=2, softflow=True):
     from cppflow_b200.ikflow import IkflowModelParameters
 
-    return IkflowModelParameters(nb_nodes=nb, dim_latent_space=width, coeff_fn_config=L, coeff_fn_internal_size=H)
+    return IkflowModelParameters(nb_nodes=nb, dim_latent_space=width, coeff_fn_config=L, coeff_fn_internal_size=H,
+                                 softflow_enabled=softflow)
+
+
+@dataclass(frozen=True)
+class FlowShape:
+    robot: str
+    width: int
+    dim_cond: int
+    nb: int
+    H: int
+    L: int
+
+    def params(self):
+        return _params(width=self.width, nb=self.nb, H=self.H, L=self.L, softflow=self.dim_cond == 8)
+
+    @property
+    def ndof(self):
+        return len(_limits(self.robot))
+
+
+# Network shapes that cppflow_flow_run accepts beyond the width-9, dim_cond-8 networks of the small / full cases.  Each
+# row reaches code no other row does.  The GEMMs use BN = 256 column tiles when H % 256 == 0, else BN = 128.
+FLOW_SHAPES = {
+    # width = ndof without softflow; BN 128 x 3 column tiles; L 1: no hidden Linear, the head reads the first layer
+    "A": FlowShape("panda", 7, 7, 3, 384, 1),
+    # even split equal to ndof without softflow; BN 128 x 5 tiles; L 4: the head reads the second hidden buffer
+    "B": FlowShape("fetch", 8, 7, 2, 640, 4),
+    # the widest state (MAXW) and all 16 rows of the last Linear; nb 1: the first block is the last; BN 128 x 7 tiles
+    "C": FlowShape("fetch_arm", 16, 8, 1, 896, 2),
+    # BN 256 x 2 tiles
+    "D": FlowShape("panda", 10, 8, 2, 512, 3),
+    # odd width (6 / 7 split); BN 256 x 3 tiles; L 1
+    "E": FlowShape("fetch", 13, 8, 3, 768, 1),
+    # width = ndof with softflow: the training noise lands on joint columns only; L 4
+    "F": FlowShape("fetch_arm", 7, 8, 4, 256, 4),
+    # IKFlow's full size with L 4
+    "G": FlowShape("panda", 9, 8, 12, 1024, 4),
+    # width > ndof without softflow: cppflow_flow_run accepts it, cppflow_flow_train_step rejects it
+    "H": FlowShape("fetch", 12, 7, 2, 128, 2),
+}
+TRAIN_SHAPES = [k for k, s in FLOW_SHAPES.items() if s.dim_cond == 8 or s.width == s.ndof]
+HEAD_ROWS, HEAD_WARPS = 4, 8  # flow_head_kernel (csrc/flow.cuh): rows per warp and pass, warps per block
+
+
+def head_rows_per_pass(n):
+    """Rows one pass of flow_head_kernel's grid-stride loop covers for n rows on cuda:0: the launch (csrc/k_flow.cu)
+    has min(ceil(n / 32), 2 * SMs) blocks of HEAD_WARPS warps with HEAD_ROWS rows each."""
+    sms = torch.cuda.get_device_properties(0).multi_processor_count
+    per_block = HEAD_WARPS * HEAD_ROWS
+    return min(-(-n // per_block), 2 * sms) * per_block
+
+
+def head_passes(n):
+    return -(-n // head_rows_per_pass(n))
+
+
+def size_cases(robots, sizes=("small", "full"), shapes=FLOW_SHAPES):
+    """(robot, size) parameter sets: every robot at the small and full width-9 networks (ids "small-fetch", ...), then
+    each table row on its own robot (ids "A-panda", ...)."""
+    cases = [pytest.param(r, s, id=f"{s}-{r}") for s in sizes for r in robots]
+    return cases + [pytest.param(FLOW_SHAPES[k].robot, k, id=f"{k}-{FLOW_SHAPES[k].robot}") for k in shapes]
 
 
 # ----------------------------------------------------------------------------------------------------------- CPU
 
 
-@pytest.mark.parametrize("width", [7, 8, 9])
-@pytest.mark.parametrize("n_layers", [1, 3])
+@pytest.mark.parametrize("width", [7, 8, 9, 16])
+@pytest.mark.parametrize("n_layers", [1, 3, 4])
 def test_oracle_reverse_inverts_forward_fp64(width, n_layers):
     net = OF.random_glow(_limits("panda"), width, nb_nodes=4, internal=32, n_layers=n_layers, seed=width).double()
     g = torch.Generator().manual_seed(1)
@@ -106,6 +170,15 @@ def test_workspace_bytes():
     assert lib.cppflow_flow_workspace_bytes(_desc(), n) == a256(n * 64) + a256(n * 128) + 2 * a256(n * 2048)
     assert lib.cppflow_flow_workspace_bytes(_desc(coeff_fn_config=1, coeff_fn_internal_size=256), 5) == (
         a256(5 * 64) + a256(5 * 128) + a256(5 * 512))
+    # every shape of the table: the state, the subnet input and min(L, 2) hidden buffers
+    from cppflow_b200.robot import get_robot
+
+    n = 20011
+    for s in FLOW_SHAPES.values():
+        d = _desc(robot=get_robot(s.robot).robot_id, width=s.width, ndof=s.ndof, dim_cond=s.dim_cond, nb_nodes=s.nb,
+                  coeff_fn_config=s.L, coeff_fn_internal_size=s.H)
+        want = a256(n * 64) + a256(n * 128) + min(s.L, 2) * a256(n * s.H * 2)
+        assert lib.cppflow_flow_workspace_bytes(d, n) == want, s
 
 
 @pytest.mark.parametrize("change,message", [
@@ -173,12 +246,14 @@ def test_flow_desc_layout_matches_the_c_header(tmp_path):
 # full network stores ~7 * 10^4 activations per row, i.e. tens of such flips per row, each moving the outputs by
 # ~10^-4.  Against the plain fp32 oracle every stored activation carries its BF16 rounding error (2^-9 relative), the
 # error of a BF16 network.  The bounds are 3-4x the worst row and 6x the mean measured on a B200 over the 6 parity
-# cases (BF16 oracle: max 2.9e-3, mean 8.0e-5; fp32 oracle: max 5.0e-3, mean 4.9e-4).
+# cases (BF16 oracle: max 2.9e-3, mean 8.0e-5; fp32 oracle: max 5.0e-3, mean 4.9e-4).  The 8 rows of FLOW_SHAPES at
+# n = 20011 stay inside the same bounds (NVIDIA B200, 1000 W power limit; worst over rows and both directions: BF16
+# oracle max 2.1e-3, mean 5.7e-5; fp32 oracle max 9.8e-3, mean 1.2e-3, both of the latter in row A's reverse pass).
 PARITY_BF16 = dict(max=1e-2, mean=5e-4)
 PARITY_FP32 = dict(max=2e-2, mean=3e-3)
 # The reverse pass re-evaluates each subnet on an input rebuilt in FP32, not on the forward pass's bits: where the
 # rebuilt value rounds to another BF16 number the subnet's s and t move by ~2^-8 relative.  Measured worst row of
-# 6475: 1.4e-3 (joint units, after the 1 / M scale).
+# 6475: 1.4e-3 (joint units, after the 1 / M scale); of 20011 over the rows of FLOW_SHAPES: 2.2e-3 (row E).
 ROUND_TRIP = 5e-3
 
 
@@ -204,20 +279,28 @@ def _oracle(solver):
     return net.to(DEV)
 
 
+# The table's rows run n = 20011 rows (not a multiple of 32 or 128) conditioned on a 37-waypoint path (37 does not
+# divide n): at least 3 passes of the head's grid-stride loop on a 148-SM B200.
+TABLE_ROWS, TABLE_T = 20011, 37
+
+
 @pytest.mark.gpu
-@pytest.mark.parametrize("robot", ["fetch", "fetch_arm", "panda"])
-@pytest.mark.parametrize("size", ["small", "full"])
+@pytest.mark.parametrize("robot,size", size_cases(ROBOTS))
 def test_parity_with_the_oracle(robot, size):
     from cppflow_b200.ikflow import IkflowSolver
     from cppflow_b200.robot import get_robot
 
     rob = get_robot(robot)
-    p = _params(width=9, nb=2, H=128, L=2) if size == "small" else _params(width=9, nb=12, H=1024, L=3)
+    if size in FLOW_SHAPES:
+        p, n, T = FLOW_SHAPES[size].params(), TABLE_ROWS, TABLE_T
+        assert head_passes(n) >= 3, head_passes(n)
+    else:
+        p = _params(width=9, nb=2, H=128, L=2) if size == "small" else _params(width=9, nb=12, H=1024, L=3)
+        n, T = 175 * 37, 37  # n = 6475: not a multiple of any tile
     solver = IkflowSolver(rob, p, seed=11, device=DEV)
     net = _oracle(solver).double()
-    k, T = 175, 37  # n = 6475: not a multiple of any tile
-    z, path = _inputs(solver, k * T, T, 0)
-    cond = path.repeat(k, 1).double()
+    z, path = _inputs(solver, n, T, 0)
+    cond = path.repeat(-(-n // T), 1)[:n].double()
     with torch.no_grad():
         for reverse in (True, False):
             x_in = z if reverse else solver.run(z, path, True)
@@ -226,8 +309,8 @@ def test_parity_with_the_oracle(robot, size):
             ref32 = net.float()(x_in, cond.float(), rev=reverse).double()
             net.double()
             e16, e32 = _rel_err(got, ref16), _rel_err(got, ref32)
-            print(f"{robot} {size} reverse={reverse}: bf16 oracle max {e16.max():.2e} mean {e16.mean():.2e}; "
-                  f"fp32 oracle max {e32.max():.2e} mean {e32.mean():.2e}")
+            print(f"{robot} {size} reverse={reverse} n={n} head passes {head_passes(n)}: bf16 oracle max "
+                  f"{e16.max():.2e} mean {e16.mean():.2e}; fp32 oracle max {e32.max():.2e} mean {e32.mean():.2e}")
             assert torch.isfinite(got).all()
             assert e16.max() < PARITY_BF16["max"] and e16.mean() < PARITY_BF16["mean"]
             assert e32.max() < PARITY_FP32["max"] and e32.mean() < PARITY_FP32["mean"]
@@ -269,6 +352,45 @@ def test_round_trip_row_independence_conditions_clamp():
     assert gen.shape == (n, 8) and torch.equal(gen, clamped[:, :8])
     assert torch.equal(solver.solve_paths(path, z.reshape(k, T, 9)[:, 0]).reshape(n, 8),
                        solver.generate_ik_solutions(cond, z.reshape(k, T, 9)[:, :1].expand(k, T, 9).reshape(n, 9)))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("shape", list(FLOW_SHAPES))
+def test_round_trip_rows_across_head_passes_and_clamp_per_shape(shape):
+    from cppflow_b200.ikflow import IkflowSolver
+    from cppflow_b200.robot import get_robot
+
+    s = FLOW_SHAPES[shape]
+    rob = get_robot(s.robot)
+    D, W, n, T = rob.ndof, s.width, TABLE_ROWS, TABLE_T
+    per_pass = head_rows_per_pass(n)
+    assert head_passes(n) >= 3, head_passes(n)
+    solver = IkflowSolver(rob, s.params(), seed=3, device=DEV)
+    z, path = _inputs(solver, n, T, 1)
+    cond = path.repeat(-(-n // T), 1)[:n].contiguous()
+    # round trip of configurations inside the limits, padding 0
+    lim = torch.tensor(rob.actuated_joints_limits, device=DEV)
+    q = lim[:, 0] + (lim[:, 1] - lim[:, 0]) * torch.rand((n, D), device=DEV)
+    x = torch.cat([q, torch.zeros((n, W - D), device=DEV)], dim=1)
+    back = solver.run(solver.run(x, path, False), path, True)
+    err = (back - x).abs().max().item()
+    print(f"{shape} {s}: round trip max |dx| = {err:.2e}, head passes {head_passes(n)} of {per_pass} rows")
+    assert err < ROUND_TRIP
+    # a row of the third pass, a slice inside the second pass and the last 300 rows, run alone, give the bits of the
+    # full run, in both directions
+    slices = ((2 * per_pass + 7, 2 * per_pass + 8), (per_pass + 100, 2 * per_pass - 100), (n - 300, n))
+    assert all(hi <= n for _, hi in slices)
+    for reverse in (True, False):
+        full = solver.run(z, path, reverse)
+        for lo, hi in slices:
+            part = solver.run(z[lo:hi].contiguous(), cond[lo:hi].contiguous(), reverse)
+            assert torch.equal(part, full[lo:hi]), (reverse, lo, hi)
+    # the clamp clamps the first ndof columns (all of them at width = ndof) and leaves the padding alone
+    full = solver.run(z, path, True)
+    clamped = solver.run(z, path, True, clamp=True)
+    assert torch.equal(clamped[:, :D], torch.maximum(torch.minimum(full[:, :D], lim[:, 1]), lim[:, 0]))
+    assert torch.equal(clamped[:, D:], full[:, D:])
+    assert (clamped[:, :D] != full[:, :D]).any()
 
 
 @pytest.mark.gpu

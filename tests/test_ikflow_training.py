@@ -4,7 +4,9 @@ definition of oracle/ikflow_train.py.
 CPU: the log-determinant identity of the oracle, the round trip of packed tables and GraphINN state dicts, workspace
 sizes, rejected shapes and the struct layout.  GPU: forward parity (z bit-identical to cppflow_flow_run), gradient
 parity with torch autograd, Adam against torch.optim.Adam, determinism, graph replay, resume, no host
-synchronisation, skipped non-finite steps, a short training run that learns, and the planner on trained weights."""
+synchronisation, skipped non-finite steps, a short training run that learns, and the planner on trained weights.
+Forward and gradient parity, Adam and the batch draw also run over the trainable rows of tests/test_ikflow.py's
+FLOW_SHAPES, as does the packing round trip."""
 import ctypes
 import os
 import shutil
@@ -15,6 +17,7 @@ import torch
 
 from oracle import ikflow as OF
 from oracle import ikflow_train as OT
+from tests.test_ikflow import FLOW_SHAPES, TRAIN_SHAPES, head_passes, size_cases
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DEV = "cuda:0"
@@ -76,14 +79,18 @@ def test_training_batch_definition():
     assert torch.equal(x7, q[idx]) and cond7.shape == (n, 7)
 
 
-@pytest.mark.parametrize("L", [1, 3])
-def test_packed_tables_round_trip(L):
+@pytest.mark.parametrize("case", [1, 3, *FLOW_SHAPES])
+def test_packed_tables_round_trip(case):
+    """case: L of a width-9 Fetch network, or a row of FLOW_SHAPES"""
     from cppflow_b200.ikflow import pack_fp32, random_state_dict
     from cppflow_b200.ikflow_training import _TABLES, split_tables, unpack
     from cppflow_b200.robot import get_robot
 
-    p = _params(width=9, nb=3, H=128, L=L)
-    sd = random_state_dict(get_robot("fetch"), p, seed=4)
+    if case in FLOW_SHAPES:
+        robot, p = FLOW_SHAPES[case].robot, FLOW_SHAPES[case].params()
+    else:
+        robot, p = "fetch", _params(width=9, nb=3, H=128, L=case)
+    sd = random_state_dict(get_robot(robot), p, seed=4)
     packed = pack_fp32(p, sd)
     flat = torch.cat([packed[k].reshape(-1) for k in _TABLES])
     back = unpack(split_tables(flat, p), p)
@@ -113,18 +120,32 @@ def _train_desc(**kw):
 
 def test_train_workspace_bytes():
     from cppflow_b200 import _lib
+    from cppflow_b200.robot import get_robot
 
     lib = _lib.load()
     a256 = lambda b: (b + 255) // 256 * 256  # noqa: E731
-    for nb, H, L, W, n in ((12, 1024, 3, 9, 512), (2, 128, 1, 7, 4096)):
+
+    def want(nb, H, L, W, n):
         S = 2 * nb
         P = 2 * nb * (H * 64 + (L - 1) * H * H + L * H + 16 * H + 16)
-        want = (2 * a256(S * n * 64) + 2 * a256(S * n * 128) + 2 * a256(S * L * n * H * 2) + 2 * a256(n * 4)
+        return (2 * a256(S * n * 64) + 2 * a256(S * n * 128) + 2 * a256(S * L * n * H * 2) + 2 * a256(n * 4)
                 + a256(n * W * 4) + 2 * a256(n * 64) + a256(n * 128) + a256(16 * n * 2) + a256(16 * n * 4)
                 + 4 * a256(n * H * 2)
                 + a256(n * 256) + a256(P * 4) + a256(1024) + a256(4))
+
+    for nb, H, L, W, n in ((12, 1024, 3, 9, 512), (2, 128, 1, 7, 4096)):
         d = _train_desc(nb_nodes=nb, coeff_fn_internal_size=H, coeff_fn_config=L, width=W)
-        assert lib.cppflow_flow_train_workspace_bytes(d, n) == want
+        assert lib.cppflow_flow_train_workspace_bytes(d, n) == want(nb, H, L, W, n)
+    n = 128 * 149
+    for k, s in FLOW_SHAPES.items():
+        d = _train_desc(robot=get_robot(s.robot).robot_id, ndof=s.ndof, width=s.width, dim_cond=s.dim_cond,
+                        nb_nodes=s.nb, coeff_fn_internal_size=s.H, coeff_fn_config=s.L)
+        got = lib.cppflow_flow_train_workspace_bytes(d, n)
+        if k in TRAIN_SHAPES:
+            assert got == want(s.nb, s.H, s.L, s.width, n), k
+        else:  # width > ndof without softflow
+            assert got == 0 and b"needs softflow" in lib.cppflow_last_error(), k
+    assert TRAIN_SHAPES == [k for k in FLOW_SHAPES if k != "H"]
 
 
 @pytest.mark.parametrize("change,batch,message", [
@@ -184,10 +205,14 @@ def test_flow_train_desc_layout_matches_the_c_header(tmp_path):
 # ----------------------------------------------------------------------------------------------------------- GPU
 
 def _trainer(robot, size="small", **kw):
+    """size: "small" or "full" (width 9, dim_cond 8), or a row of FLOW_SHAPES"""
     from cppflow_b200.ikflow_training import IkflowTrainer
     from cppflow_b200.robot import get_robot
 
-    p = _params(width=9, nb=2, H=128, L=2) if size == "small" else _params(width=9, nb=12, H=1024, L=3)
+    if size in FLOW_SHAPES:
+        p = FLOW_SHAPES[size].params()
+    else:
+        p = _params(width=9, nb=2, H=128, L=2) if size == "small" else _params(width=9, nb=12, H=1024, L=3)
     kw.setdefault("n_data", 20000)
     return IkflowTrainer(get_robot(robot), p, seed=kw.pop("seed", 3), device=DEV, **kw)
 
@@ -214,16 +239,19 @@ def _ws_z_logdet(tr, n):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("robot", ROBOTS)
-@pytest.mark.parametrize("size", ["small", "full"])
+@pytest.mark.parametrize("robot,size", size_cases(ROBOTS, shapes=TRAIN_SHAPES))
 def test_training_forward_parity(robot, size):
     from cppflow_b200 import ops
 
     n = 128 * 41  # 5248 rows: a multiple of the 128-row tile, not of 256 or of the head's 32-row groups
+    if size in FLOW_SHAPES:
+        n = 128 * 149  # 19072 rows: at least 3 passes of the head's grid-stride loop on a 148-SM B200
+        assert head_passes(n) >= 3, head_passes(n)
     tr = _trainer(robot, size, batch_size=n)
     tr.draw_batch()
     x, cond = tr.x.clone(), tr.cond.clone()
-    cond[:, 7] = 0  # cppflow_flow_run conditions with a softflow scale of 0
+    if tr.dim_cond == 8:
+        cond[:, 7] = 0  # cppflow_flow_run conditions with a softflow scale of 0
     loss, _ = tr.loss_and_grad(x, cond)
     z, ld = _ws_z_logdet(tr, n)
     # the inference forward pass on the same rows gives the same bits
@@ -242,20 +270,21 @@ def test_training_forward_parity(robot, size):
     e16 = (got_ld - ld64).abs().max().item()
     e32 = (got_ld - ld32.double()).abs().max().item()
     l64 = OT.nll(z64, ld64).item()
-    print(f"{robot} {size}: log_det max err vs bf16 oracle {e16:.2e}, vs fp32 oracle {e32:.2e}; loss {loss.item():.6f} "
-          f"vs {l64:.6f}")
+    print(f"{robot} {size} n={n} head passes {head_passes(n)}: log_det max err vs bf16 oracle {e16:.2e}, vs fp32 "
+          f"oracle {e32:.2e}; loss {loss.item():.6f} vs {l64:.6f}")
     assert torch.isfinite(z).all()
     assert e16 < 2e-2 and e32 < 5e-2
     assert abs(loss.item() - l64) < 1e-3 * max(1.0, abs(l64))
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("size", ["small", "full"])
+@pytest.mark.parametrize("size", ["small", "full", *TRAIN_SHAPES])
 def test_gradient_parity_with_autograd(size):
+    """size: a width-9 Panda network ("small", "full") or a trainable row of FLOW_SHAPES, on its own robot"""
     from cppflow_b200.ikflow_training import split_tables, unpack
 
     n = 1024
-    tr = _trainer("panda", size, batch_size=n, seed=5)
+    tr = _trainer(FLOW_SHAPES[size].robot if size in FLOW_SHAPES else "panda", size, batch_size=n, seed=5)
     tr.draw_batch()
     x, cond = tr.x.clone(), tr.cond.clone()
     _, grad = tr.loss_and_grad(x, cond)
@@ -276,18 +305,18 @@ def test_gradient_parity_with_autograd(size):
         rel_t = ((torch_bf16[k] - r).norm() / r.norm()).item()
         cos = torch.nn.functional.cosine_similarity(g.reshape(1, -1), r.reshape(1, -1)).item()
         worst = max(worst, rel / rel_t)
-        print(f"{k}: rel L2 {rel:.2e} (torch bf16 autocast {rel_t:.2e}), cos {cos:.6f}")
+        print(f"{size} {k}: rel L2 {rel:.2e} (torch bf16 autocast {rel_t:.2e}), cos {cos:.6f}")
         assert rel <= 2 * rel_t, k
         assert cos >= 0.999, k
-    print(f"worst ratio to torch bf16: {worst:.2f}")
+    print(f"{size}: worst ratio to torch bf16: {worst:.2f}")
 
 
-@pytest.mark.gpu
-def test_adam_step_matches_torch_and_refreshes_the_tables():
+def _check_adam_steps(tr):
+    """Two steps of tr against torch.optim.Adam given the returned gradient, then the BF16 tables against a fresh
+    packing of state_dict()"""
     from cppflow_b200 import ops
     from cppflow_b200.ikflow import IkflowSolver
 
-    tr = _trainer("fetch", "small", batch_size=512)
     for _ in range(2):  # second step: nonzero moments and bias corrections of t = 2
         tr.draw_batch()
         before = [t.clone() for t in (tr.params_flat, tr.adam_m, tr.adam_v)]
@@ -307,14 +336,28 @@ def test_adam_step_matches_torch_and_refreshes_the_tables():
             torch.testing.assert_close(mine, ref, rtol=2e-6, atol=2e-6 * ref.abs().max().item())
     assert tr.counters.tolist() == [2, 0, 2]
     sol = IkflowSolver(tr.robot, tr.params, state_dict=tr.state_dict(), device=DEV)
-    for k in ("w_in", "w_hidden"):
+    hidden = tr.params.coeff_fn_config > 1
+    assert (sol._tables["w_hidden"] is not None) == hidden and (tr.bf16["w_hidden"] is not None) == hidden
+    for k in ("w_in", "w_hidden") if hidden else ("w_in",):
         assert torch.equal(tr.bf16[k], sol._tables[k]), k
     for k in ("b_hidden", "w_out", "b_out"):
         assert torch.equal(tr.tables[k], sol._tables[k]), k
     assert torch.equal(tr.bf16["w_in_t"], sol._tables["w_in"].transpose(-1, -2))
-    assert torch.equal(tr.bf16["w_hidden_t"], sol._tables["w_hidden"].transpose(-1, -2))
+    if hidden:
+        assert torch.equal(tr.bf16["w_hidden_t"], sol._tables["w_hidden"].transpose(-1, -2))
     assert torch.equal(tr.bf16["w_out_t"][..., :16], sol._tables["w_out"].to(torch.bfloat16).transpose(-1, -2))
     assert tr.bf16["w_out_t"][..., 16:].abs().max() == 0
+
+
+@pytest.mark.gpu
+def test_adam_step_matches_torch_and_refreshes_the_tables():
+    _check_adam_steps(_trainer("fetch", "small", batch_size=512))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("shape", TRAIN_SHAPES)
+def test_adam_step_matches_torch_and_refreshes_the_tables_per_shape(shape):
+    _check_adam_steps(_trainer(FLOW_SHAPES[shape].robot, shape, batch_size=512))
 
 
 @pytest.mark.gpu
@@ -328,6 +371,26 @@ def test_batch_draw_matches_the_oracle_definition():
     assert torch.equal(tr.x, x) and torch.equal(tr.cond, cond)
     assert 0.3 < noise[:, 10].mean().item() < 0.7 and 0.3 < noise[:, 9].mean().item() < 0.7
     assert abs(noise[:, :9].std().item() - 1) < 0.1 and idx.max().item() < tr.data_q.shape[0]
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("shape", TRAIN_SHAPES)
+def test_batch_draw_matches_the_oracle_definition_per_shape(shape):
+    s = FLOW_SHAPES[shape]
+    W, n = s.width, 1024
+    tr = _trainer(s.robot, shape, batch_size=n)
+    idx = torch.empty(n, dtype=torch.int64, device=DEV)
+    noise = torch.empty((n, W + 2), device=DEV)
+    tr.draw_batch(idx, noise)
+    x, cond = OT.training_batch(tr.data_q, tr.data_poses, idx, noise[:, W], noise[:, :W], noise[:, W + 1], W,
+                                s.dim_cond, tr.softflow_noise_scale)
+    assert torch.equal(tr.x, x) and torch.equal(tr.cond, cond)
+    assert 0.3 < noise[:, W + 1].mean().item() < 0.7 and idx.max().item() < tr.data_q.shape[0]
+    if s.dim_cond == 8:  # every column, the Box-Muller tail of an odd width included, draws a standard normal
+        assert 0.3 < noise[:, W].mean().item() < 0.7
+        assert (noise[:, :W].std(dim=0) - 1).abs().max().item() < 0.15 and noise[:, :W].mean(dim=0).abs().max() < 0.15
+    else:  # no noise: x is the configuration
+        assert torch.equal(tr.x, tr.data_q[idx])
 
 
 @pytest.mark.gpu
