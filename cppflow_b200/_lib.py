@@ -205,6 +205,10 @@ _PROTOTYPES = {
     "cppflow_flow_train_step": (_I, [C.POINTER(FlowTrainDescC), _VP, _VP, _I64, _I, _VP, _SZ, _VP, _VP, _VP]),
     "cppflow_flow_train_batch": (_I, [C.POINTER(FlowTrainDescC), _VP, _VP, _I64, _I64, C.c_uint64, _F, _VP, _VP, _VP, _VP,
                                       _VP]),
+    "cppflow_flow_train_batch_rows": (_I, [C.POINTER(FlowTrainDescC), _VP, _VP, _I64, _I64, _I64, C.c_uint64, _F, _VP, _VP,
+                                           _VP, _VP, _VP]),
+    "cppflow_flow_train_apply": (_I, [C.POINTER(FlowTrainDescC), _VP, _I64, _VP, _SZ, _VP]),
+    "cppflow_flow_grad_tree_reduce": (_I, [_VP, _I, _I64, _I64, _F, _VP, _VP]),
     "cppflow_ik_refine": (_I, [_I, C.POINTER(IkRefineDescC), _VP, _VP, _I64, _I64, _VP, _VP, _VP, _VP, _VP]),
     "cppflow_ik_round_inputs": (_I, [_VP, _I64, _I, _VP, C.c_uint64, _I, _I, _F, _VP, _VP, _VP]),
     "cppflow_ik_select_workspace_bytes": (_SZ, [_I64]),

@@ -15,6 +15,9 @@
 // skipped and advances the counters, and flow_adam_kernel updates the FP32 master weights and moments and rewrites the
 // BF16 tables and their transposed copies.  No kernel uses atomics and every sum has a fixed order: two runs are
 // bit-identical.
+// Data-parallel training splits a step into its parts: sharded batch draws (cppflow_flow_train_batch_rows), shard
+// gradients (NO_UPDATE), their balanced-tree sum (flow_tree_reduce_kernel, on one GPU and on each rank's slice after
+// the exchange) and the optimizer tail on the reduced gradient (cppflow_flow_train_apply).
 #include "flow.cuh"
 #include "rng.cuh"
 
@@ -314,18 +317,47 @@ __global__ void __launch_bounds__(256) flow_adam_kernel(AdamArgs a) {
     }
 }
 
+// ------------------------------------------------------------------------------------------ gradient reduction
+
+// out[k] = scale * T(in[0 * stride + k], ..., in[(N - 1) * stride + k]) for k < len, T the balanced pairwise tree in
+// slice order ((s0 + s1) + (s2 + s3)) + ...; four floats per thread.  out may be slice 0 (each thread reads its
+// elements of every slice before it writes them).
+template <int N>
+__global__ void __launch_bounds__(256) flow_tree_reduce_kernel(const float* in, int64_t len4, int64_t stride4, float scale,
+                                                               float* out) {
+    const float4* src = reinterpret_cast<const float4*>(in);
+    float4* dst = reinterpret_cast<float4*>(out);
+    for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < len4; k += (int64_t)gridDim.x * blockDim.x) {
+        float4 v[N];
+#pragma unroll
+        for (int i = 0; i < N; ++i) v[i] = src[i * stride4 + k];
+#pragma unroll
+        for (int w = 1; w < N; w *= 2)
+#pragma unroll
+            for (int i = 0; i < N; i += 2 * w) {
+                v[i].x = __fadd_rn(v[i].x, v[i + w].x);
+                v[i].y = __fadd_rn(v[i].y, v[i + w].y);
+                v[i].z = __fadd_rn(v[i].z, v[i + w].z);
+                v[i].w = __fadd_rn(v[i].w, v[i + w].w);
+            }
+        dst[k] = make_float4(__fmul_rn(v[0].x, scale), __fmul_rn(v[0].y, scale), __fmul_rn(v[0].z, scale),
+                             __fmul_rn(v[0].w, scale));
+    }
+}
+
 // --------------------------------------------------------------------------------------------- batch sampling
 
-// One thread per batch row; the random numbers of (seed, step, row) do not depend on the batch size.
+// One thread per batch row; the random numbers of (seed, step, first_row + row) do not depend on the batch size, so a
+// batch drawn in shards from first_row = 0, B, 2B, ... is the batch drawn at once.
 __global__ void __launch_bounds__(256) flow_train_batch_kernel(const float* __restrict__ q, const float* __restrict__ poses,
-                                                               int64_t n_data, int64_t batch, int ndof, int width,
-                                                               int dim_cond, uint64_t seed, const int64_t* __restrict__ step,
-                                                               float noise_scale, float* __restrict__ x,
-                                                               float* __restrict__ cond, int64_t* __restrict__ idx_out,
-                                                               float* __restrict__ noise_out) {
+                                                               int64_t n_data, int64_t batch, int64_t first_row, int ndof,
+                                                               int width, int dim_cond, uint64_t seed,
+                                                               const int64_t* __restrict__ step, float noise_scale,
+                                                               float* __restrict__ x, float* __restrict__ cond,
+                                                               int64_t* __restrict__ idx_out, float* __restrict__ noise_out) {
     const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (row >= batch) return;
-    const uint64_t key = mix64(seed ^ mix64((uint64_t)*step)) ^ mix64((uint64_t)row * 0x2545F4914F6CDD1Dull);
+    const uint64_t key = mix64(seed ^ mix64((uint64_t)*step)) ^ mix64((uint64_t)(first_row + row) * 0x2545F4914F6CDD1Dull);
     auto draw = [&](int k) { return mix64(key + (uint64_t)k * 0x9E3779B97F4A7C15ull); };
     const int64_t idx = (int64_t)__umul64hi(draw(0), (uint64_t)n_data);
     const bool soft = dim_cond == 8;
@@ -370,6 +402,50 @@ static int gemm_bf16(EncodeFn enc, const void* a, int64_t m_rows, const void* w,
                      cudaStream_t st) {
     return n_cols % 256 == 0 ? launch_gemm_epi<256, EPI>(enc, a, m_rows, w, n_cols, K, ep, st)
                              : launch_gemm_epi<128, EPI>(enc, a, m_rows, w, n_cols, K, ep, st);
+}
+
+// The optimizer tail of a step on the gradient grad [P]: finite check into flags, the skip decision and counters,
+// Adam and the BF16 table rewrites.
+static int apply_update(const cppflow_flow_train_desc* t, const float* grad, int* flags, int* skip, int sms,
+                        cudaStream_t st) {
+    const cppflow_flow_desc* d = &t->flow;
+    const ParamLayout pl = param_layout(d);
+    flow_finite_kernel<<<FLAG_BLOCKS, 256, 0, st>>>(grad, pl.total, flags);
+    CPPFLOW_CHECK_LAUNCH();
+    flow_step_decide_kernel<<<1, 32, 0, st>>>(flags, skip, t->d_counters);
+    CPPFLOW_CHECK_LAUNCH();
+    AdamArgs a;
+    std::memset(&a, 0, sizeof(a));
+    a.p = pl;
+    a.H = d->coeff_fn_internal_size;
+    a.L = d->coeff_fn_config;
+    a.grad = grad;
+    a.w = t->d_params;
+    a.m = t->d_adam_m;
+    a.v = t->d_adam_v;
+    a.w_in = static_cast<__nv_bfloat16*>(const_cast<void*>(d->d_w_in));
+    a.w_hidden = static_cast<__nv_bfloat16*>(const_cast<void*>(d->d_w_hidden));
+    a.w_in_t = static_cast<__nv_bfloat16*>(t->d_w_in_t);
+    a.w_hidden_t = static_cast<__nv_bfloat16*>(t->d_w_hidden_t);
+    a.w_out_t = static_cast<__nv_bfloat16*>(t->d_w_out_t);
+    a.skip = skip;
+    a.counters = t->d_counters;
+    a.lr = t->lr;
+    a.beta1 = t->beta1;
+    a.beta2 = t->beta2;
+    a.eps = t->eps;
+    a.weight_decay = t->weight_decay;
+    a.lr_decay = t->lr_decay;
+    a.lr_decay_steps = t->lr_decay_steps;
+    flow_adam_kernel<<<(unsigned)std::min<size_t>(grid_for((int64_t)pl.total, 256), (size_t)sms * 8), 256, 0, st>>>(a);
+    CPPFLOW_CHECK_LAUNCH();
+    return CPPFLOW_OK;
+}
+
+static int sm_count() {
+    int dev = 0, sms = 148;
+    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    return sms;
 }
 
 }  // namespace flow
@@ -429,8 +505,7 @@ extern "C" int cppflow_flow_train_step(const cppflow_flow_train_desc* t, const f
     auto step_subnet = [&](int i) { return 1 - i % 2; };  // forward order, as cppflow_flow_run
 
     cudaStream_t st = (cudaStream_t)stream;
-    int dev = 0, sms = 148;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int sms = sm_count();
     const unsigned row_warps = (unsigned)((n + 7) / 8);
 
     // ---- forward
@@ -575,36 +650,63 @@ extern "C" int cppflow_flow_train_step(const cppflow_flow_train_desc* t, const f
         }
     }
     if (flags & CPPFLOW_FLOW_TRAIN_NO_UPDATE) return CPPFLOW_OK;
+    return apply_update(t, grad, ws.flags, ws.skip, sms, st);
+}
 
-    // ---- optimizer
-    flow_finite_kernel<<<FLAG_BLOCKS, 256, 0, st>>>(grad, pl.total, ws.flags);
+extern "C" int cppflow_flow_train_apply(const cppflow_flow_train_desc* t, const float* d_grad, int64_t batch,
+                                       void* d_workspace, size_t ws_bytes, void* stream) {
+    int rc = validate_train(t, batch);
+    if (rc) return rc;
+    const cppflow_flow_desc* d = &t->flow;
+    CPPFLOW_CHECK_ARG(d_grad, "d_grad");
+    CPPFLOW_CHECK_ARG(d->d_w_in && (d->coeff_fn_config == 1 || (d->d_w_hidden && t->d_w_hidden_t)), "null BF16 table");
+    CPPFLOW_CHECK_ARG(t->d_params && t->d_adam_m && t->d_adam_v && t->d_w_in_t && t->d_w_out_t && t->d_counters,
+                      "null training table");
+    const size_t need = train_ws(d, batch, nullptr, nullptr);
+    if (!d_workspace || ws_bytes < need)
+        return fail(CPPFLOW_E_WORKSPACE, "cppflow_flow_train_apply: workspace %zu bytes < %zu", ws_bytes, need);
+    TrainWs ws;
+    train_ws(d, batch, static_cast<uint8_t*>(d_workspace), &ws);
+    return apply_update(t, d_grad, ws.flags, ws.skip, sm_count(), (cudaStream_t)stream);
+}
+
+extern "C" int cppflow_flow_grad_tree_reduce(const float* d_in, int n, int64_t len, int64_t stride, float scale,
+                                            float* d_out, void* stream) {
+    CPPFLOW_CHECK_ARG(d_in && d_out, "d_in / d_out");
+    CPPFLOW_CHECK_ARG(n >= 1 && n <= CPPFLOW_TREE_REDUCE_MAX && (n & (n - 1)) == 0, "n is not a power of two in [1, 32]");
+    CPPFLOW_CHECK_ARG(len >= 0 && len % 4 == 0 && stride % 4 == 0 && (n == 1 || stride >= len),
+                      "len and stride must be multiples of 4, stride >= len");
+    CPPFLOW_CHECK_ARG(reinterpret_cast<uintptr_t>(d_in) % 16 == 0 && reinterpret_cast<uintptr_t>(d_out) % 16 == 0,
+                      "d_in / d_out not 16-byte aligned");
+    if (len == 0) return CPPFLOW_OK;
+    const int64_t len4 = len / 4, stride4 = stride / 4;
+    const unsigned grid = (unsigned)std::min<int64_t>(grid_for(len4, 256), (int64_t)sm_count() * 8);
+    cudaStream_t st = (cudaStream_t)stream;
+    switch (n) {
+        case 1: flow_tree_reduce_kernel<1><<<grid, 256, 0, st>>>(d_in, len4, stride4, scale, d_out); break;
+        case 2: flow_tree_reduce_kernel<2><<<grid, 256, 0, st>>>(d_in, len4, stride4, scale, d_out); break;
+        case 4: flow_tree_reduce_kernel<4><<<grid, 256, 0, st>>>(d_in, len4, stride4, scale, d_out); break;
+        case 8: flow_tree_reduce_kernel<8><<<grid, 256, 0, st>>>(d_in, len4, stride4, scale, d_out); break;
+        case 16: flow_tree_reduce_kernel<16><<<grid, 256, 0, st>>>(d_in, len4, stride4, scale, d_out); break;
+        default: flow_tree_reduce_kernel<32><<<grid, 256, 0, st>>>(d_in, len4, stride4, scale, d_out); break;
+    }
     CPPFLOW_CHECK_LAUNCH();
-    flow_step_decide_kernel<<<1, 32, 0, st>>>(ws.flags, ws.skip, t->d_counters);
-    CPPFLOW_CHECK_LAUNCH();
-    AdamArgs a;
-    std::memset(&a, 0, sizeof(a));
-    a.p = pl;
-    a.H = H;
-    a.L = L;
-    a.grad = grad;
-    a.w = t->d_params;
-    a.m = t->d_adam_m;
-    a.v = t->d_adam_v;
-    a.w_in = const_cast<__nv_bfloat16*>(w_in);
-    a.w_hidden = const_cast<__nv_bfloat16*>(w_hid);
-    a.w_in_t = static_cast<__nv_bfloat16*>(t->d_w_in_t);
-    a.w_hidden_t = static_cast<__nv_bfloat16*>(t->d_w_hidden_t);
-    a.w_out_t = static_cast<__nv_bfloat16*>(t->d_w_out_t);
-    a.skip = ws.skip;
-    a.counters = t->d_counters;
-    a.lr = t->lr;
-    a.beta1 = t->beta1;
-    a.beta2 = t->beta2;
-    a.eps = t->eps;
-    a.weight_decay = t->weight_decay;
-    a.lr_decay = t->lr_decay;
-    a.lr_decay_steps = t->lr_decay_steps;
-    flow_adam_kernel<<<(unsigned)std::min<size_t>(grid_for((int64_t)pl.total, 256), (size_t)sms * 8), 256, 0, st>>>(a);
+    return CPPFLOW_OK;
+}
+
+extern "C" int cppflow_flow_train_batch_rows(const cppflow_flow_train_desc* t, const float* d_q, const float* d_poses,
+                                            int64_t n_data, int64_t batch, int64_t first_row, uint64_t seed,
+                                            float softflow_noise_scale, float* d_x, float* d_cond, int64_t* d_idx,
+                                            float* d_noise, void* stream) {
+    int rc = validate_train(t, batch);
+    if (rc) return rc;
+    CPPFLOW_CHECK_ARG(d_q && d_poses && d_x && d_cond && t->d_counters, "d_q / d_poses / d_x / d_cond / d_counters");
+    CPPFLOW_CHECK_ARG(n_data >= 1, "n_data < 1");
+    CPPFLOW_CHECK_ARG(first_row >= 0, "first_row < 0");
+    const cppflow_flow_desc* d = &t->flow;
+    flow_train_batch_kernel<<<grid_for(batch, 256), 256, 0, (cudaStream_t)stream>>>(
+        d_q, d_poses, n_data, batch, first_row, d->ndof, d->width, d->dim_cond, seed, t->d_counters + 2,
+        softflow_noise_scale, d_x, d_cond, d_idx, d_noise);
     CPPFLOW_CHECK_LAUNCH();
     return CPPFLOW_OK;
 }
@@ -612,14 +714,6 @@ extern "C" int cppflow_flow_train_step(const cppflow_flow_train_desc* t, const f
 extern "C" int cppflow_flow_train_batch(const cppflow_flow_train_desc* t, const float* d_q, const float* d_poses,
                                        int64_t n_data, int64_t batch, uint64_t seed, float softflow_noise_scale,
                                        float* d_x, float* d_cond, int64_t* d_idx, float* d_noise, void* stream) {
-    int rc = validate_train(t, batch);
-    if (rc) return rc;
-    CPPFLOW_CHECK_ARG(d_q && d_poses && d_x && d_cond && t->d_counters, "d_q / d_poses / d_x / d_cond / d_counters");
-    CPPFLOW_CHECK_ARG(n_data >= 1, "n_data < 1");
-    const cppflow_flow_desc* d = &t->flow;
-    flow_train_batch_kernel<<<grid_for(batch, 256), 256, 0, (cudaStream_t)stream>>>(
-        d_q, d_poses, n_data, batch, d->ndof, d->width, d->dim_cond, seed, t->d_counters + 2, softflow_noise_scale, d_x,
-        d_cond, d_idx, d_noise);
-    CPPFLOW_CHECK_LAUNCH();
-    return CPPFLOW_OK;
+    return cppflow_flow_train_batch_rows(t, d_q, d_poses, n_data, batch, 0, seed, softflow_noise_scale, d_x, d_cond,
+                                         d_idx, d_noise, stream);
 }

@@ -10,9 +10,18 @@ graph.  `state_dict()` is in FrEIA's GraphINN format: it loads into `oracle.ikfl
 The defaults are ikflow's `train.py` defaults as far as they are known without its source at hand, and are UNVERIFIED:
 batch 512, lr 5e-4, Adam betas (0.9, 0.999), weight decay 1.8e-5 (L2, added to the gradient as torch.optim.Adam
 does), ExponentialLR gamma 0.9794 stepped once per 2.5 M samples, softflow noise scale 1e-3.  Adam's eps is torch's
-default 1e-8.  The training definition (loss, softflow, padding, quaternion signs) is oracle/ikflow_train.py's."""
+default 1e-8.  The training definition (loss, softflow, padding, quaternion signs) is oracle/ikflow_train.py's.
+
+Data-parallel training (IkflowTrainer's process_group and micro_batches): one global step uses S = W x M shards of B
+rows, W ranks (one GPU each) of M micro-batches each.  Shard j holds rows j B ... (j + 1) B - 1 of the global batch,
+whose row g is drawn from (seed, step, g).  The reduced gradient is G = (1 / S) T(g_0, ..., g_{S-1}), g_j the gradient
+of shard j's mean NLL and T the balanced pairwise tree in shard order (tree_levels).  With W and M powers of two a
+rank owns an aligned subtree: it sums its M gradients with the same tree (local_schedule), and the W partials are
+combined by the top of the tree in rank order, on the slice of the vector each rank owns, by the library's
+fixed-order reduction.  NCCL only moves bytes (all_to_all, all_gather), so G, the shard losses' mean carried in the
+same vector, and every update depend on (S, B) alone: (W, M) = (8, 1), (2, 4) and (1, 8) give the same bits."""
 from dataclasses import asdict
-from typing import Dict, Optional
+from typing import Dict, List, Optional, Tuple
 
 import numpy as np
 import torch
@@ -94,21 +103,68 @@ def sample_accuracy(solver, poses: torch.Tensor, k: int = 16, seed: int = 0) -> 
             "rot_median_rad": rot.median().item()}
 
 
+def _is_pow2(v: int) -> bool:
+    return v >= 1 and v & (v - 1) == 0
+
+
+def tree_levels(S: int) -> List[List[Tuple[Tuple[int, int], Tuple[int, int]]]]:
+    """The balanced pairwise tree over S (a power of two) shards in shard order, level by level: each entry is a pair
+    (left, right) of half-open shard ranges whose sums are added, left + right; T(g_0, ..., g_{S-1}) is the root."""
+    if not _is_pow2(S):
+        raise ValueError(f"{S} shards: the tree needs a power of two")
+    levels, w = [], 1
+    while w < S:
+        levels.append([((a, a + w), (a + w, a + 2 * w)) for a in range(0, S, 2 * w)])
+        w *= 2
+    return levels
+
+
+def local_schedule(M: int) -> List[Tuple]:
+    """A rank's M micro-batch gradients summed with the tree of tree_levels(M) while they arrive, in log2(M) + 1
+    buffers used as a stack: ("grad", j, slot) computes the gradient of micro-batch j into `slot`, ("add", slot)
+    replaces slot by slot + (slot + 1) (the left and right subtrees of equal size on top of the stack).  The sum ends
+    in slot 0."""
+    if not _is_pow2(M):
+        raise ValueError(f"micro_batches {M} is not a power of two")
+    ops, sizes = [], []
+    for j in range(M):
+        ops.append(("grad", j, len(sizes)))
+        sizes.append(1)
+        while len(sizes) >= 2 and sizes[-1] == sizes[-2]:
+            ops.append(("add", len(sizes) - 2))
+            sizes[-2:] = [2 * sizes[-1]]
+    return ops
+
+
+def tree_sum(values, add=lambda a, b: a + b):
+    """T(values) in the order of tree_levels: the reference the library's reduction and local_schedule implement."""
+    v = list(values)
+    if not _is_pow2(len(v)):
+        raise ValueError(f"{len(v)} values: the tree needs a power of two")
+    while len(v) > 1:
+        v = [add(v[i], v[i + 1]) for i in range(0, len(v), 2)]
+    return v[0]
+
+
 class IkflowTrainer:
-    """Trains IKFlow's network for `robot` on one GPU.
+    """Trains IKFlow's network for `robot` on one GPU, or data-parallel on the ranks of a process group.
 
     robot, params (the network's shape), seed (initial weights, dataset and batch draws), batch_size (a multiple of
-    128), lr, betas, eps, weight_decay, lr_decay (gamma of the exponential decay), lr_decay_samples (samples between
-    two decays), softflow_noise_scale, n_data (configurations drawn for the dataset before self-colliding ones are
-    dropped), state_dict (initial weights in GraphINN format; seeded nn.Linear initialisation otherwise), use_graph
-    (replay steps after the first as one CUDA graph), history (capacity of the loss ring buffer).  See the module
-    docstring for which defaults are unverified."""
+    128; per shard), lr, betas, eps, weight_decay, lr_decay (gamma of the exponential decay), lr_decay_samples
+    (samples between two decays; counted in global steps of S x batch_size samples), softflow_noise_scale, n_data
+    (configurations drawn for the dataset before self-colliding ones are dropped; every rank draws the same),
+    state_dict (initial weights in GraphINN format; seeded nn.Linear initialisation otherwise), use_graph (replay
+    steps after the first as one CUDA graph, collectives included), history (capacity of the loss ring buffer),
+    process_group (a torch.distributed NCCL group of W ranks, W a power of two, one GPU each; None: one GPU, W = 1),
+    micro_batches (M, a power of two: shards per rank and step).  With process_group None and micro_batches 1 a step
+    is the one-call step of csrc/k_flow_train.cu; otherwise it is the data-parallel step of the module docstring, and
+    every rank holds bit-identical weights after it.  See the module docstring for which defaults are unverified."""
 
     def __init__(self, robot, params: Optional[IkflowModelParameters] = None, seed: int = 0, batch_size: int = 512,
                  lr: float = 5e-4, betas=(0.9, 0.999), eps: float = 1e-8, weight_decay: float = 1.8e-5,
                  lr_decay: float = 0.9794, lr_decay_samples: int = 2_500_000, softflow_noise_scale: float = 1e-3,
                  n_data: int = 1_000_000, state_dict: Optional[Dict] = None, use_graph: bool = False,
-                 history: int = 1 << 16, device=DEVICE):
+                 history: int = 1 << 16, device=DEVICE, process_group=None, micro_batches: int = 1):
         params = params if params is not None else IkflowModelParameters()
         if params.coupling_layer != "glow":
             raise ValueError(f"coupling_layer '{params.coupling_layer}' is not supported (only 'glow')")
@@ -116,11 +172,24 @@ class IkflowTrainer:
             raise ValueError(f"batch_size {batch_size} is not a positive multiple of 128")
         if params.dim_latent_space > robot.ndof and not params.softflow_enabled:
             raise ValueError("dim_latent_space > ndof needs softflow_enabled: the padding has no density without it")
+        self.group = process_group
+        if process_group is not None:
+            import torch.distributed as dist
+
+            self.world, self.rank = dist.get_world_size(process_group), dist.get_rank(process_group)
+        else:
+            self.world, self.rank = 1, 0
+        if not _is_pow2(self.world):
+            raise ValueError(f"{self.world} ranks: data-parallel training needs a power of two")
+        if not isinstance(micro_batches, int) or not _is_pow2(micro_batches):
+            raise ValueError(f"micro_batches {micro_batches} is not a power of two")
+        self.micro_batches = micro_batches
+        self.shards = self.world * micro_batches
         self.robot, self.params, self.seed, self.batch_size = robot, params, seed, batch_size
         self.softflow_noise_scale = float(softflow_noise_scale)
         self.n_data, self.use_graph = n_data, use_graph
         self.hyper = dict(lr=lr, beta1=betas[0], beta2=betas[1], eps=eps, weight_decay=weight_decay, lr_decay=lr_decay,
-                          lr_decay_steps=max(1, round(lr_decay_samples / batch_size)))
+                          lr_decay_steps=max(1, round(lr_decay_samples / (self.shards * batch_size))))
         self.device = torch.device(device)
         self.dim_cond = 8 if params.softflow_enabled else 7
         dev, W, B = self.device, params.dim_latent_space, batch_size
@@ -144,6 +213,20 @@ class IkflowTrainer:
         self.workspace = torch.empty(ops.flow_train_workspace_bytes(self.desc, B), dtype=torch.uint8, device=dev)
         self.steps_issued = 0
         self._graph = None
+        self._sharded = process_group is not None or micro_batches > 1
+        if self._sharded:
+            self._init_shards()
+
+    def _init_shards(self):
+        """Buffers of the data-parallel step: the local tree's stack of log2(M) + 1 gradients and the reduced G, each
+        padded to a multiple of W x 64 floats with the shard's mean loss at index P, and the all_to_all output."""
+        P, W = self.params_flat.numel(), self.world
+        self._P = P
+        self._Ppad = -(-(P + 1) // (64 * W)) * 64 * W
+        depth = self.micro_batches.bit_length()
+        self._stack = torch.zeros((depth, self._Ppad), device=self.device)
+        self._G = torch.zeros(self._Ppad, device=self.device)
+        self._recv = torch.empty((W, self._Ppad // W), device=self.device) if W > 1 else None
 
     # ---------------------------------------------------------------------------------------------- tables
     def _refresh_bf16(self):
@@ -183,10 +266,52 @@ class IkflowTrainer:
                              self.cond, idx, noise)
 
     def _issue(self):
-        self.draw_batch()
-        ops.flow_train_step(self.desc, self.x, self.cond, self.workspace, self.loss)
+        if self._sharded:
+            self._issue_sharded()
+        else:
+            self.draw_batch()
+            ops.flow_train_step(self.desc, self.x, self.cond, self.workspace, self.loss)
         slot = torch.remainder(self.counters[2:3] - 1, self._hist.numel())
         self._hist.index_copy_(0, slot, self.loss)
+
+    def _draw_shard(self, j: int):
+        """Shard j of this rank's M: rows (rank M + j) B ... of the global batch, into self.x / self.cond."""
+        B = self.batch_size
+        ops.flow_train_batch(self.desc, self.data_q, self.data_poses, self.seed, self.softflow_noise_scale, self.x,
+                             self.cond, first_row=(self.rank * self.micro_batches + j) * B)
+
+    def _local_partial(self) -> torch.Tensor:
+        """T over this rank's M shard gradients (and shard losses at index P), in self._stack[0]."""
+        P = self._P
+        for op in local_schedule(self.micro_batches):
+            if op[0] == "grad":
+                _, j, slot = op
+                self._draw_shard(j)
+                buf = self._stack[slot]
+                ops.flow_train_step(self.desc, self.x, self.cond, self.workspace, buf[P:P + 1], buf[:P], update=False)
+            else:
+                ops.flow_grad_tree_reduce(self._stack[op[1]:op[1] + 2], self._stack[op[1]])
+        return self._stack[0]
+
+    def _exchange(self, partial: torch.Tensor):
+        """G = (1 / S) T(partials of the W ranks in rank order) into self._G: all_to_all gives this rank slice `rank`
+        of every partial, the library's tree reduces it, all_gather assembles G on every rank."""
+        W, scale = self.world, 1.0 / self.shards
+        if W == 1:
+            ops.flow_grad_tree_reduce(partial.view(1, -1), self._G, scale)
+            return
+        import torch.distributed as dist
+
+        chunk = self._Ppad // W
+        dist.all_to_all_single(self._recv.view(-1), partial, group=self.group)
+        mine = self._G[self.rank * chunk:(self.rank + 1) * chunk]
+        ops.flow_grad_tree_reduce(self._recv, mine, scale)
+        dist.all_gather_into_tensor(self._G, mine, group=self.group)
+
+    def _issue_sharded(self):
+        self._exchange(self._local_partial())
+        ops.flow_train_apply(self.desc, self._G, self.batch_size, self.workspace)
+        self.loss.copy_(self._G[self._P:self._P + 1])
 
     def step(self, n: int = 1):
         """n training steps on the current stream, without a host synchronisation (graph mode: the capture after
@@ -252,27 +377,47 @@ class IkflowTrainer:
     # ------------------------------------------------------------------------------------- checkpointing
     def save(self, path: str):
         """Weights, Adam moments, counters (step count and the generator's position: batches are drawn from
-        (seed, step)), the loss ring buffer and the configuration."""
+        (seed, step)), the loss ring buffer and the configuration, with the shard count S and the per-shard batch B.
+        Data-parallel: every rank holds the same state, and rank 0 writes it (the other ranks return)."""
+        if self.rank != 0:
+            return
         torch.save({"robot": self.robot.name, "model": asdict(self.params), "seed": self.seed,
-                    "batch_size": self.batch_size, "hyper": dict(self.hyper), "n_data": self.n_data,
+                    "batch_size": self.batch_size, "shards": self.shards, "hyper": dict(self.hyper), "n_data": self.n_data,
                     "softflow_noise_scale": self.softflow_noise_scale, "history": self._hist.numel(),
                     "params": self.params_flat.cpu(), "adam_m": self.adam_m.cpu(), "adam_v": self.adam_v.cpu(),
                     "counters": self.counters.cpu(), "loss_ring": self._hist.cpu(), "steps_issued": self.steps_issued},
                    path)
 
     @classmethod
-    def load(cls, path: str, use_graph: bool = False, device=DEVICE) -> "IkflowTrainer":
-        """A trainer that continues the saved run exactly where it stopped."""
+    def load(cls, path: str, use_graph: bool = False, device=DEVICE, process_group=None,
+             micro_batches: Optional[int] = None, batch_size: Optional[int] = None) -> "IkflowTrainer":
+        """A trainer that continues the saved run exactly where it stopped, bit for bit, on any W ranks of
+        process_group (None: one GPU) with M = micro_batches such that W x M is the saved shard count S (None: S / W).
+        batch_size, when given, must be the saved per-shard batch.  A different S or B would be another run: rejected."""
         from .robot import get_robot
 
         ck = torch.load(path, map_location="cpu", weights_only=False)
         h = ck["hyper"]
+        S, B = ck.get("shards", 1), ck["batch_size"]
+        if process_group is not None:
+            import torch.distributed as dist
+
+            W = dist.get_world_size(process_group)
+        else:
+            W = 1
+        if micro_batches is None:
+            micro_batches = S // W if S % W == 0 else 0
+        if W * micro_batches != S:
+            raise ValueError(f"{path} was trained with {S} shards per step; {W} ranks x {micro_batches} micro-batches "
+                             "is another run")
+        if batch_size is not None and batch_size != B:
+            raise ValueError(f"{path} was trained with {B} rows per shard, not {batch_size}")
         params = IkflowModelParameters(**ck["model"])
-        tr = cls(get_robot(ck["robot"]), params, seed=ck["seed"], batch_size=ck["batch_size"], lr=h["lr"],
+        tr = cls(get_robot(ck["robot"]), params, seed=ck["seed"], batch_size=B, lr=h["lr"],
                  betas=(h["beta1"], h["beta2"]), eps=h["eps"], weight_decay=h["weight_decay"], lr_decay=h["lr_decay"],
-                 lr_decay_samples=h["lr_decay_steps"] * ck["batch_size"],
+                 lr_decay_samples=h["lr_decay_steps"] * S * B,
                  softflow_noise_scale=ck["softflow_noise_scale"], n_data=ck["n_data"], use_graph=use_graph,
-                 history=ck["history"], device=device)
+                 history=ck["history"], device=device, process_group=process_group, micro_batches=micro_batches)
         tr.params_flat.copy_(ck["params"])
         tr.adam_m.copy_(ck["adam_m"])
         tr.adam_v.copy_(ck["adam_v"])

@@ -500,9 +500,10 @@ def flow_train_step(desc: _lib.FlowTrainDescC, x: torch.Tensor, cond: torch.Tens
 
 def flow_train_batch(desc: _lib.FlowTrainDescC, q: torch.Tensor, poses: torch.Tensor, seed: int, noise_scale: float,
                      x: torch.Tensor, cond: torch.Tensor, idx: Optional[torch.Tensor] = None,
-                     noise: Optional[torch.Tensor] = None) -> None:
-    """Draws the training batch of the desc's current step counter into x [n, width] and cond [n, dim_cond] from the
-    dataset q [N, ndof], poses [N, 7] (include/cppflow_b200.h: cppflow_flow_train_batch).  No host synchronisation."""
+                     noise: Optional[torch.Tensor] = None, first_row: int = 0) -> None:
+    """Draws rows first_row ... first_row + n - 1 of the training batch of the desc's current step counter into
+    x [n, width] and cond [n, dim_cond] from the dataset q [N, ndof], poses [N, 7] (include/cppflow_b200.h:
+    cppflow_flow_train_batch_rows).  No host synchronisation."""
     import ctypes as C
 
     n = x.shape[0]
@@ -510,9 +511,32 @@ def flow_train_batch(desc: _lib.FlowTrainDescC, q: torch.Tensor, poses: torch.Te
     assert poses.is_cuda and poses.dtype == torch.float32 and poses.is_contiguous() and poses.shape == (q.shape[0], 7)
     assert x.is_contiguous() and x.shape == (n, desc.flow.width) and cond.is_contiguous()
     assert cond.shape == (n, desc.flow.dim_cond)
-    check(_lib.load().cppflow_flow_train_batch(C.byref(desc), ptr(q), ptr(poses), q.shape[0], n, seed & (2**64 - 1),
-                                               float(noise_scale), ptr(x), ptr(cond), ptr(idx), ptr(noise),
-                                               stream_ptr(x.device)))
+    check(_lib.load().cppflow_flow_train_batch_rows(C.byref(desc), ptr(q), ptr(poses), q.shape[0], n, first_row,
+                                                    seed & (2**64 - 1), float(noise_scale), ptr(x), ptr(cond), ptr(idx),
+                                                    ptr(noise), stream_ptr(x.device)))
+
+
+def flow_train_apply(desc: _lib.FlowTrainDescC, grad: torch.Tensor, batch: int, workspace: torch.Tensor) -> None:
+    """The optimizer tail of flow_train_step (finite check, skip decision, Adam, BF16 tables) on grad [>= P], a
+    gradient in the packed layout; workspace is flow_train_step's for `batch` rows (only its flag words are used)."""
+    import ctypes as C
+
+    assert grad.is_cuda and grad.dtype == torch.float32 and grad.is_contiguous()
+    check(_lib.load().cppflow_flow_train_apply(C.byref(desc), ptr(grad), batch, ptr(workspace),
+                                               workspace.numel() * workspace.element_size(), stream_ptr(grad.device)))
+
+
+def flow_grad_tree_reduce(slices: torch.Tensor, out: torch.Tensor, scale: float = 1.0) -> torch.Tensor:
+    """out = scale * (balanced pairwise tree sum of the rows of slices [n, len] in row order), n a power of two
+    (include/cppflow_b200.h: cppflow_flow_grad_tree_reduce).  slices may be a view with any row stride; out may be
+    slices[0].  No host synchronisation."""
+    import ctypes as C
+
+    assert slices.is_cuda and slices.dtype == torch.float32 and slices.dim() == 2 and slices.stride(1) == 1
+    assert out.is_cuda and out.dtype == torch.float32 and out.is_contiguous() and out.numel() == slices.shape[1]
+    check(_lib.load().cppflow_flow_grad_tree_reduce(ptr(slices), slices.shape[0], slices.shape[1], slices.stride(0),
+                                                    float(scale), ptr(out), stream_ptr(out.device)))
+    return out
 
 
 IK_CLAMP, IK_CHECK_SELF_COLLISION, IK_NO_EARLY_EXIT = 1, 2, 4  # CPPFLOW_IK_* (include/cppflow_b200.h)

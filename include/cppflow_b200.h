@@ -361,6 +361,28 @@ int cppflow_flow_train_step(const cppflow_flow_train_desc* desc, const float* d_
 int cppflow_flow_train_batch(const cppflow_flow_train_desc* desc, const float* d_q, const float* d_poses, int64_t n_data,
                              int64_t batch, uint64_t seed, float softflow_noise_scale, float* d_x, float* d_cond,
                              int64_t* d_idx, float* d_noise, void* stream);
+/* Rows first_row ... first_row + batch - 1 of a larger batch: row r of the outputs is keyed on (seed, d_counters[2],
+ * first_row + r), so shards drawn at first_row = 0, B, 2B, ... are, bit for bit, the rows of one draw of the whole
+ * batch.  cppflow_flow_train_batch is this call with first_row = 0. */
+int cppflow_flow_train_batch_rows(const cppflow_flow_train_desc* desc, const float* d_q, const float* d_poses,
+                                  int64_t n_data, int64_t batch, int64_t first_row, uint64_t seed,
+                                  float softflow_noise_scale, float* d_x, float* d_cond, int64_t* d_idx, float* d_noise,
+                                  void* stream);
+/* The optimizer tail of cppflow_flow_train_step on a gradient the caller supplies: d_grad fp32 [P] (the layout of
+ * d_params) -> finite check, skip decision and counters, Adam and the BF16 table rewrites, exactly as the step runs
+ * them (cppflow_flow_train_step calls the same code, so NO_UPDATE + this call is the one-call step bit for bit).
+ * d_workspace is a workspace of cppflow_flow_train_step for `batch` rows; the call uses only its flag and skip words,
+ * the activations are left alone.  No allocation, no host synchronisation; capturable in a CUDA graph. */
+int cppflow_flow_train_apply(const cppflow_flow_train_desc* desc, const float* d_grad, int64_t batch, void* d_workspace,
+                             size_t workspace_bytes, void* stream);
+/* Fixed-order sum of n equal FP32 slices, for data-parallel training whose result does not depend on how the shards
+ * map to GPUs: d_out[k] = scale * T(d_in[k], d_in[stride + k], ..., d_in[(n - 1) stride + k]) for k < len, with T the
+ * balanced pairwise tree in slice order, ((s0 + s1) + (s2 + s3)) + ..., every add and the final multiply rounded to
+ * nearest FP32.  n a power of two <= CPPFLOW_TREE_REDUCE_MAX; len and stride multiples of 4, stride >= len when n > 1;
+ * d_in and d_out 16-byte aligned.  d_out may be d_in (slice 0) and no other slice.  HBM-bound, no atomics. */
+#define CPPFLOW_TREE_REDUCE_MAX 32
+int cppflow_flow_grad_tree_reduce(const float* d_in, int n, int64_t len, int64_t stride, float scale, float* d_out,
+                                  void* stream);
 
 /* Exact inverse kinematics from IKFlow's samples: ikflow's IKFlowSolver.generate_exact_ik_solutions (sample the flow,
  * refine every sample with batched Levenberg-Marquardt IK, resample the targets that did not converge with more samples
