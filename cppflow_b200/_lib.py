@@ -163,6 +163,8 @@ class IkRefineDescC(C.Structure):
     ]
 
 
+LM_BATCHED_PINNED_BYTES = 64  # CPPFLOW_LM_BATCHED_PINNED_BYTES
+
 ABI_VERSION = 5  # CPPFLOW_ABI_VERSION of include/cppflow_b200.h
 
 _VP, _I, _I64, _SZ, _F, _DBL = C.c_void_p, C.c_int, C.c_int64, C.c_size_t, C.c_float, C.c_double
@@ -193,9 +195,14 @@ _PROTOTYPES = {
                                          _I64, c_float_p, c_float_p, _I, _I, _DBL, _I, _DBL, _VP, _SZ, _VP, _VP,
                                          C.POINTER(LmLoopResultC), _VP]),
     "cppflow_lm_alternating_loss_many": (_I, [_I, C.POINTER(LmLoopJobC)]),
+    "cppflow_lm_alternating_batched_workspace_bytes": (_SZ, [_I, _I64, _I64]),
+    "cppflow_lm_alternating_loss_batched": (_I, [_I, C.POINTER(LmParamsC), C.POINTER(LmParamsC), C.POINTER(ConstraintsC),
+                                                 _VP, _VP, _I64, _I64, c_float_p, c_float_p, _I, _I, _DBL, _I, _DBL, _VP,
+                                                 _SZ, _VP, _VP, C.POINTER(LmLoopResultC), _VP]),
     "cppflow_joint_limit_flags": (_I, [_I, _VP, _I64, _F, _F, _VP, _VP]),
     "cppflow_dp_search_workspace_bytes": (_SZ, [_I64, _I64]),
     "cppflow_dp_search": (_I, [_I, _VP, _VP, _VP, _I64, _I64, _VP, _SZ, _VP, _VP, _VP, _VP, _VP]),
+    "cppflow_dp_backtrack": (_I, [_VP, _VP, _I64, _I64, _I, _VP, _I64, _VP, _VP]),
     "cppflow_path_metrics": (_I, [_I, _VP, _VP, _I64, _I64, c_float_p, c_float_p, _I, _VP, _VP]),
     "cppflow_path_key_argmin": (_I, [_VP, _I64, C.POINTER(ConstraintsC), _I64, _VP, _VP]),
     "cppflow_path_metrics_ex": (_I, [_I, _VP, _VP, _I64, _I64, c_float_p, c_float_p, _I, _I, _VP, _VP]),

@@ -58,6 +58,10 @@ inline int make_obstacles(const float* h_cuboids, const float* h_Tcuboids, int n
     return CPPFLOW_OK;
 }
 
+// path_metrics_tagged flag (internal, above the public CPPFLOW_METRICS_* bits): take the kernel one path of T waypoints
+// gets (the clustered split, or one CTA per path when a path fits one CTA), whatever the number of paths
+constexpr int METRICS_AS_ONE_PATH = 1 << 16;
+
 // cppflow_path_metrics with a completion tag in column 7 of every row (k_metrics.cu)
 int path_metrics_tagged(int robot, const float* d_q, const float* d_target, int64_t P, int64_t T, const float* h_cuboids,
                         const float* h_Tcuboids, int n_obstacles, float* d_out, float tag, void* stream, int flags = 0);
@@ -66,6 +70,10 @@ int path_metrics_tagged(int robot, const float* d_q, const float* d_target, int6
 int pose_step_metrics_tagged(int robot, const cppflow_lm_params* params, const float* d_q, const float* d_target, int64_t T,
                              const float* h_cuboids, const float* h_Tcuboids, int n_obstacles, float* d_x_out, float* d_out,
                              float tag, void* stream);
+// the same for n_rows paths: path p is row rows[p] of d_q / d_x_out, its metrics go to d_out[p] (k_metrics.cu)
+int pose_step_metrics_rows(int robot, const cppflow_lm_params* params, const float* d_q, const float* d_target, int64_t T,
+                           const float* h_cuboids, const float* h_Tcuboids, int n_obstacles, const int* d_rows,
+                           int64_t n_rows, float* d_x_out, float* d_out, float tag, void* stream);
 
 inline unsigned grid_for(int64_t n, int block) { return (unsigned)((n + block - 1) / block); }
 

@@ -45,10 +45,13 @@ __device__ __forceinline__ float warp_sum(float v) {
 // are idempotent, the trajectory length is added by lane 0 of a group only).
 // FUSE (clustered, one pass over the path, one path): the kernel first takes the pose-only LM step of every waypoint
 // (lane 0 of a waypoint's group; pose_step.cuh) from `q` into `pf.x_out`, and then evaluates the metrics of the NEW path -
-// one launch per iteration of the single-path LM loop instead of two launch-bound ones.
+// one launch per iteration of the single-path LM loop instead of two launch-bound ones.  With `rows` set (the batched
+// loop, lm_loop_batched.cu) cluster p steps the path in row rows[p] of `q` / `x_out` (paths of T waypoints); its
+// metrics still go to out[p].  G and the cluster size depend on T only, so every path gets the single-path arithmetic.
 struct PoseFuse {
     float alpha_pos, alpha_rot, lambda;
     float* x_out;
+    const int* rows;
 };
 
 template <bool COHERENT>
@@ -72,21 +75,25 @@ path_metrics_kernel(const float* __restrict__ q_in, const float* __restrict__ ta
         csize = cluster.num_blocks();
     }
     const int64_t p = blockIdx.x / csize;
+    int64_t prow = p;  // row of `q` that holds path p
     float* sm = smem + threadIdx.x;
     const float* q = q_in;
     if constexpr (FUSE) {
+        prow = pf.rows ? __ldg(pf.rows + p) : p;
+        const float* xin = q_in + prow * T * D;
+        float* xout = pf.x_out + prow * T * D;
         static_assert(CLUSTERED, "the fused step needs the cluster-wide barrier");
         // every thread takes part in the shuffles and the barrier: threads beyond the path shadow its last waypoint
         const int64_t t0 = rank * (MBLOCK / G) + threadIdx.x / G;
         const bool act = t0 < T;
         const int64_t tc = act ? t0 : T - 1;
         float xs[D], tgs[7];
-        load_q<M>(q_in, tc, xs);
+        load_q<M>(xin, tc, xs);
 #pragma unroll
         for (int k = 0; k < 7; ++k) tgs[k] = __ldg(target + tc * 7 + k);
         if (threadIdx.x % G == 0) pose_lm_update<M>(xs, tgs, pf.alpha_pos, pf.alpha_rot, pf.lambda, 1, nullptr, nullptr, 0);
         __syncwarp();
-        if (threadIdx.x % G == 0 && act) store_q<M>(pf.x_out, tc, xs);
+        if (threadIdx.x % G == 0 && act) store_q<M>(xout, tc, xs);
         __threadfence();
         cg::this_cluster().sync();  // the new path is complete (neighbouring waypoints live in other CTAs)
         q = pf.x_out;
@@ -94,7 +101,7 @@ path_metrics_kernel(const float* __restrict__ q_in, const float* __restrict__ ta
     float m_pos = 0.f, m_rot = 0.f, m_rev = 0.f, m_pri = 0.f, tl = 0.f, d_self = INFINITY, d_env = INFINITY;
     const int gl = threadIdx.x % G;  // lane within the waypoint's group
     for (int64_t t = rank * (MBLOCK / G) + threadIdx.x / G; t < T; t += (int64_t)csize * (MBLOCK / G)) {
-        const int64_t i = p * T + t;
+        const int64_t i = prow * T + t;
         float x[D];
 #pragma unroll
         for (int d = 0; d < D; ++d) x[d] = ld_row<FUSE>(q + i * D + d);
@@ -449,7 +456,10 @@ int cppflow::path_metrics_tagged(int robot, const float* d_q, const float* d_tar
     const int G = T <= 8 * MBLOCK / 4 ? 4 : (T <= 8 * MBLOCK / 2 ? 2 : 1);
     const int64_t per_cta = MBLOCK / G;
     const int csize = (int)((T + per_cta - 1) / per_cta < 8 ? (T + per_cta - 1) / per_cta : 8);
-    const bool clustered = csize > 1 && P * csize <= 2 * 148;
+    // many paths: one CTA per path fills the GPU better, but its trajectory-length sum is added in another order.
+    // METRICS_AS_ONE_PATH keeps the kernel that ONE path of T waypoints gets, whatever P (the batched LM loop's
+    // convergence decisions must see the single-path loop's bits)
+    const bool clustered = csize > 1 && ((flags & METRICS_AS_ONE_PATH) != 0 || P * csize <= 2 * 148);
     CPPFLOW_DISPATCH_ROBOT(robot, {
         const size_t sh = sizeof(float) * MBLOCK * SmemLayout<M>::N_DIST;
         if (clustered) {
@@ -491,21 +501,26 @@ int cppflow::path_metrics_tagged(int robot, const float* d_q, const float* d_tar
     return CPPFLOW_OK;
 }
 
-// pose-only LM step (+ clamp) of ONE path of T <= 8 * MBLOCK waypoints and the metrics of the new path, one launch
-int cppflow::pose_step_metrics_tagged(int robot, const cppflow_lm_params* params, const float* d_q, const float* d_target,
-                                      int64_t T, const float* h_cuboids, const float* h_Tcuboids, int n_obstacles,
-                                      float* d_x_out, float* d_out, float tag, void* stream) {
+// pose-only LM step (+ clamp) of n_rows paths of T <= 8 * MBLOCK waypoints and the metrics of the new paths, one launch:
+// cluster p steps the path in row rows[p] of d_q into the same row of d_x_out and writes its metrics to d_out[p]
+// (rows = NULL: one path, row 0)
+int cppflow::pose_step_metrics_rows(int robot, const cppflow_lm_params* params, const float* d_q, const float* d_target,
+                                    int64_t T, const float* h_cuboids, const float* h_Tcuboids, int n_obstacles,
+                                    const int* d_rows, int64_t n_rows, float* d_x_out, float* d_out, float tag,
+                                    void* stream) {
     CPPFLOW_CHECK_ARG(params && d_q && d_target && d_x_out && d_out, "null pointer");
     CPPFLOW_CHECK_ARG(T > 0 && T <= 8 * MBLOCK, "T");
+    CPPFLOW_CHECK_ARG(n_rows >= 0 && (d_rows != nullptr || n_rows <= 1), "rows");
+    if (n_rows == 0) return CPPFLOW_OK;
     Obstacles ob;
     if (int rc = make_obstacles(h_cuboids, h_Tcuboids, n_obstacles, ob)) return rc;
     const int G = T <= 8 * MBLOCK / 4 ? 4 : (T <= 8 * MBLOCK / 2 ? 2 : 1);
     const int64_t per_cta = MBLOCK / G;
     const int csize = (int)((T + per_cta - 1) / per_cta);
-    const PoseFuse pf{params->alpha_position, params->alpha_rotation, params->lm_lambda, d_x_out};
+    const PoseFuse pf{params->alpha_position, params->alpha_rotation, params->lm_lambda, d_x_out, d_rows};
     CPPFLOW_DISPATCH_ROBOT(robot, {
         cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)csize);
+        cfg.gridDim = dim3((unsigned)(n_rows * csize));
         cfg.blockDim = dim3(MBLOCK);
         cfg.dynamicSmemBytes = sizeof(float) * MBLOCK * SmemLayout<M>::N_DIST;
         cfg.stream = (cudaStream_t)stream;
@@ -523,6 +538,13 @@ int cppflow::pose_step_metrics_tagged(int robot, const cppflow_lm_params* params
     });
     CPPFLOW_CHECK_LAUNCH();
     return CPPFLOW_OK;
+}
+
+int cppflow::pose_step_metrics_tagged(int robot, const cppflow_lm_params* params, const float* d_q, const float* d_target,
+                                      int64_t T, const float* h_cuboids, const float* h_Tcuboids, int n_obstacles,
+                                      float* d_x_out, float* d_out, float tag, void* stream) {
+    return pose_step_metrics_rows(robot, params, d_q, d_target, T, h_cuboids, h_Tcuboids, n_obstacles, nullptr, 1, d_x_out,
+                                  d_out, tag, stream);
 }
 
 extern "C" int cppflow_path_metrics(int robot, const float* d_q, const float* d_target, int64_t P, int64_t T,

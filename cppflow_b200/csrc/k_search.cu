@@ -444,3 +444,37 @@ extern "C" int cppflow_dp_search(int robot, const float* d_q, const uint8_t* d_s
     CPPFLOW_CHECK_LAUNCH();
     return CPPFLOW_OK;
 }
+
+// ----------------------------------------------------------------------------------------------------------------
+// Backtrack from chosen terminals (the planner's lm_seeds: the DP's best paths ending at its n cheapest terminals).
+// One warp per terminal walks memo from T - 1 to 0 exactly as dp_sweep_kernel's backtrack does (search.py:162-173) and
+// gathers the waypoints as it goes: lane d copies joint d of waypoint t of the chosen candidate.  A terminal is a
+// candidate index; memo entries are candidate indices, so every step stays inside [0, k).
+namespace cppflow {
+__global__ void __launch_bounds__(256)
+dp_backtrack_kernel(const float* __restrict__ q, const int32_t* __restrict__ memo, int k, int T, int D,
+                    const int32_t* __restrict__ terminals, int64_t n, float* __restrict__ out) {
+    const int64_t j = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (j >= n) return;
+    int i = __ldg(terminals + j);
+    float* o = out + j * (int64_t)T * D;
+    for (int t = T - 1; t >= 0; --t) {
+        if (lane < D) o[(int64_t)t * D + lane] = __ldg(q + ((int64_t)i * T + t) * D + lane);
+        i = __ldg(memo + (int64_t)i * T + t);
+    }
+}
+}  // namespace cppflow
+
+extern "C" int cppflow_dp_backtrack(const float* d_q, const int32_t* d_memo, int64_t k, int64_t T, int ndof,
+                                    const int32_t* d_terminals, int64_t n, float* d_out, void* stream) {
+    CPPFLOW_CHECK_ARG(k > 0 && T > 0 && n >= 0, "k, T, n");
+    CPPFLOW_CHECK_ARG(k <= 65535 && T <= 65535, "k, T must be <= 65535");
+    CPPFLOW_CHECK_ARG(ndof > 0 && ndof <= 32, "ndof");
+    if (n == 0) return CPPFLOW_OK;
+    CPPFLOW_CHECK_ARG(d_q && d_memo && d_terminals && d_out, "null pointer");
+    dp_backtrack_kernel<<<grid_for(n * 32, 256), 256, 0, (cudaStream_t)stream>>>(d_q, d_memo, (int)k, (int)T, ndof,
+                                                                                 d_terminals, n, d_out);
+    CPPFLOW_CHECK_LAUNCH();
+    return CPPFLOW_OK;
+}

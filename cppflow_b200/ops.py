@@ -303,6 +303,25 @@ def dp_search(rid: int, ndof: int, q: torch.Tensor, self_flags: torch.Tensor, en
     return best, memo, costs, chosen
 
 
+@_on_device
+def dp_backtrack(q: torch.Tensor, memo: torch.Tensor, terminals: torch.Tensor) -> torch.Tensor:
+    """The DP's best paths ending at the given terminal candidates: q [k, T, ndof], memo int32 [k, T] (dp_search's),
+    terminals int [n] -> [n, T, ndof], path j backtracked from candidate terminals[j] as dp_search backtracks."""
+    q = require_cuda(q, "q")
+    assert q.dim() == 3, f"q must be [k, T, ndof], is {tuple(q.shape)}"
+    k, T, ndof = q.shape
+    memo = require_cuda(memo, "memo", torch.int32)
+    assert memo.shape == (k, T), f"memo must be [{k}, {T}], is {tuple(memo.shape)}"
+    terminals = require_cuda(terminals.to(q.device), "terminals", torch.int32)
+    assert terminals.dim() == 1
+    if terminals.numel() and not bool(((terminals >= 0) & (terminals < k)).all()):
+        raise ValueError(f"terminals must be candidate indices in [0, {k})")
+    out = torch.empty((terminals.numel(), T, ndof), device=q.device, dtype=torch.float32)
+    check(_lib.load().cppflow_dp_backtrack(ptr(q), ptr(memo), k, T, ndof, ptr(terminals), terminals.numel(), ptr(out),
+                                           stream_ptr(q.device)))
+    return out
+
+
 METRIC_NAMES = ("max_pos_cm", "max_rot_deg", "mjac_deg", "mjac_cm", "tl", "min_self", "min_env")
 
 
@@ -436,6 +455,47 @@ def lm_alternating_loss_many(jobs):
         outs.append((x_out, res))
     check(lib.cppflow_lm_alternating_loss_many(n, arr))
     return [(x, int(r.n_steps_taken), bool(r.is_valid), r.schedule.decode(), list(r.last_metrics)) for x, r in outs]
+
+
+@_on_device
+def lm_alternating_loss_batched(rid: int, ndof: int, params_diff: LmParamsC, params_pose: LmParamsC, constraints,
+                                x_seeds: torch.Tensor, target: torch.Tensor, ob: Optional[Obstacles], max_n_steps: int,
+                                tmax_sec: float, return_if_valid_after_n_steps: int, convergence_threshold: float):
+    """run_lm_alternating_loss for N seed paths x_seeds [N, T, ndof] of one problem, driven by the library's batched loop
+    (csrc/lm_loop_batched.cu): every launch covers all unfinished seeds, one host round trip per iteration.  Seed i's
+    outcome is bit for bit that of lm_alternating_loss on seed i alone (last_metrics[7], no metric, is 0).
+    -> list of N (x_opt [T, ndof], n_steps_taken, is_valid, schedule, last_metrics list of 8)"""
+    x_seeds = require_cuda(x_seeds, "x_seeds")
+    assert x_seeds.dim() == 3 and x_seeds.shape[2] == ndof, f"x_seeds must be [N, T, {ndof}], is {tuple(x_seeds.shape)}"
+    N, T, _ = x_seeds.shape
+    assert T > 0, "x_seeds must have at least one waypoint"
+    target = require_cuda(target, "target_path")
+    assert target.shape == (T, 7), f"target_path must be [{T}, 7], is {tuple(target.shape)}"
+    x_out = torch.empty_like(x_seeds)
+    if N == 0:
+        return []
+    lib = _lib.load()
+    dev = x_seeds.device
+    ws = _workspace(dev, lib.cppflow_lm_alternating_batched_workspace_bytes(rid, N, T) + 256, "lm_loop_batched")
+    off = (-ws.data_ptr()) % 256
+    pkey = (str(dev), torch.cuda.current_stream(dev).cuda_stream, "batched")
+    pinned = _PINNED.get(pkey)
+    if pinned is None:
+        pinned = _PINNED[pkey] = torch.empty(_lib.LM_BATCHED_PINNED_BYTES // 4, dtype=torch.int32).pin_memory()
+    cons = _lib.ConstraintsC(constraints.max_allowed_position_error_cm, constraints.max_allowed_rotation_error_deg,
+                             constraints.max_allowed_mjac_deg, constraints.max_allowed_mjac_cm)
+    res = (_lib.LmLoopResultC * N)()
+    cu, tc, no = _obs(ob)
+    import ctypes as C
+
+    tmax = 1e30 if tmax_sec is None or tmax_sec == float("inf") else float(tmax_sec)
+    check(lib.cppflow_lm_alternating_loss_batched(
+        rid, params_diff, params_pose, cons, ptr(x_seeds), ptr(target), N, T, cu, tc, no,
+        int(min(max_n_steps, 2 ** 31 - 1)), tmax, int(min(return_if_valid_after_n_steps, 2 ** 31 - 1)),
+        float(convergence_threshold), C.c_void_p(ws.data_ptr() + off), ws.numel() - off, C.c_void_p(pinned.data_ptr()),
+        ptr(x_out), res, stream_ptr(dev)))
+    return [(x_out[i], int(r.n_steps_taken), bool(r.is_valid), r.schedule.decode(), list(r.last_metrics))
+            for i, r in enumerate(res)]
 
 
 FLOW_REVERSE, FLOW_CLAMP = 1, 2  # CPPFLOW_FLOW_REVERSE / _CLAMP (include/cppflow_b200.h)

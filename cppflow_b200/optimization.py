@@ -5,11 +5,12 @@
   run_lm_alternating_loss        :147-373  same control flow; one device->host read of 8 floats per iteration
   run_lm_optimization            :376-426
 Unlike the reference (`assert parallel_count == 1`, :128) the full step handles `parallel_count` stacked paths in
-one launch; `run_lm_fixed_schedule` runs a data-independent step sequence over thousands of paths (SURVEY 8d, config 5).
+one launch; `run_lm_fixed_schedule` runs a data-independent step sequence over thousands of paths (SURVEY 8d, config 5);
+`run_lm_optimization_batched` runs the alternating loop, with its per-path decisions, over many seeds of one problem.
 """
 from dataclasses import dataclass
 from time import time
-from typing import Dict, Optional
+from typing import Dict, List, Optional
 import warnings
 
 import torch
@@ -19,9 +20,6 @@ from .config import ENV_COLLISIONS_IGNORED, SELF_COLLISIONS_IGNORED
 from .data_types import Constraints, Problem
 from .lm_hyper_parameters import ALT_LOSS_V2_1_DIFF, ALT_LOSS_V2_1_POSE, OptimizationParameters, all_terms_parameters
 from .optimization_utils import LmResidualFns, clamp_to_joint_limits, path_metrics, x_is_valid
-
-
-_SEED_STREAMS: Dict[str, list] = {}
 
 
 @dataclass
@@ -242,26 +240,13 @@ def run_lm_optimization(problem: Problem, x_seed: torch.Tensor, tmax_sec: float,
     assert isinstance(max_n_steps, int), f"error: max_n_steps must be int, is {type(max_n_steps)}"
     if parallel_count > 1:
         # the reference stacks `parallel_count` seeds but its full LM step asserts parallel_count == 1 (:128); here
-        # every seed runs its own alternating loop, all in lock step on their own streams, and the first valid one
+        # every seed runs its own alternating loop (all of them in the library's batched loop) and the first valid one
         # (lowest seed index) is returned - the first seed's last iterate if none is valid
         assert mesh_validator is None, "parallel seeds run inside the library: no mesh callback"
         T = problem.n_timesteps
-        seeds = [x_seed[i * T:(i + 1) * T].contiguous() for i in range(parallel_count)]
-        pool = _SEED_STREAMS.setdefault(str(x_seed.device), [])
-        while len(pool) < parallel_count:
-            pool.append(torch.cuda.Stream(x_seed.device))
-        cur = torch.cuda.current_stream(x_seed.device)
-        for s in pool[:parallel_count]:
-            s.wait_stream(cur)
-        results = run_lm_optimization_many([problem] * parallel_count, seeds, pool[:parallel_count], tmax_sec, max_n_steps,
-                                           return_if_valid_after_n_steps, convergence_threshold)
-        for s in pool[:parallel_count]:
-            cur.wait_stream(s)
-        for i, r in enumerate(results):
-            if r.is_valid:
-                r.parallel_seed_idx = i
-                return r
-        return results[0]
+        results = run_lm_optimization_batched(problem, x_seed.reshape(parallel_count, T, problem.robot.ndof), tmax_sec,
+                                              max_n_steps, return_if_valid_after_n_steps, convergence_threshold)
+        return next((r for r in results if r.is_valid), results[0])
     opt_problem = OptimizationProblem(problem, problem.constraints, x_seed, stacked_target_path, verbosity,
                                       parallel_count, results_df)
     opt_state = OptimizationState(x_seed.clone(), 0, time())
@@ -271,6 +256,31 @@ def run_lm_optimization(problem: Problem, x_seed: torch.Tensor, tmax_sec: float,
         convergence_threshold=convergence_threshold, save_images=False, results_df=results_df,
         mesh_validator=mesh_validator, native=native,
     )
+
+
+def run_lm_optimization_batched(problem: Problem, x_seeds: torch.Tensor, tmax_sec: Optional[float],
+                                max_n_steps: Optional[int], return_if_valid_after_n_steps: int,
+                                convergence_threshold: float) -> List[OptimizationResult]:
+    """run_lm_optimization for N seed paths x_seeds [N, T, ndof] of one problem at once (csrc/lm_loop_batched.cu): every
+    kernel launch of an iteration covers all unfinished seeds and the host reads the iteration's outcome once, whatever
+    N.  Result i (parallel_seed_idx = i) is bit for bit that of run_lm_optimization(problem, x_seeds[i]); the time limit
+    is checked once per iteration for all seeds.  tmax_sec / max_n_steps = None as in run_lm_alternating_loss."""
+    robot = problem.robot
+    assert x_seeds.dim() == 3 and x_seeds.shape[1:] == (problem.n_timesteps, robot.ndof), \
+        f"x_seeds must be [N, {problem.n_timesteps}, {robot.ndof}], is {tuple(x_seeds.shape)}"
+    if tmax_sec is None:
+        assert (max_n_steps is not None) and (return_if_valid_after_n_steps is not None)
+        assert return_if_valid_after_n_steps <= max_n_steps
+        tmax_sec = float("inf")
+    if max_n_steps is None:
+        assert tmax_sec is not None
+        max_n_steps = int(1e9)
+    out = ops.lm_alternating_loss_batched(
+        robot.robot_id, robot.ndof, ops.make_params(ALT_LOSS_V2_1_DIFF), ops.make_params(ALT_LOSS_V2_1_POSE),
+        problem.constraints, x_seeds, problem.target_path, problem.obstacle_tables, max_n_steps, tmax_sec,
+        return_if_valid_after_n_steps, convergence_threshold)
+    return [OptimizationResult(x_opt=x, n_steps_taken=n, is_valid=v, parallel_seed_idx=i, schedule=s)
+            for i, (x, n, v, s, _) in enumerate(out)]
 
 
 def run_lm_optimization_many(problems, x_seeds, streams, tmax_sec: float, max_n_steps: int,

@@ -18,7 +18,7 @@ from .collision_detection import qpaths_batched_collisions
 from .config import DEVICE, OPTIMIZATION_CONVERGENCE_THRESHOLD, SUCCESS_THRESHOLD_initial_q_norm_dist
 from .data_types import PathReport, PlannerResult, PlannerSettings, Problem, TimingData
 from .evaluation_utils import get_mjacs
-from .optimization import run_lm_optimization
+from .optimization import run_lm_optimization, run_lm_optimization_batched
 from .optimization_utils import path_metrics
 from .search import dp_search
 from . import ops
@@ -364,15 +364,17 @@ class Planner:
     def name(self) -> str:
         return str(self.__class__.__name__)
 
-    def _run_pipeline(self, problem: Problem, **kwargs) -> Tuple[torch.Tensor, bool, TimingData, Dict, Tuple]:
-        """Candidates -> collision flags -> dp_search (planners.py:191-292)."""
+    def _run_pipeline(self, problem: Problem, search_details: bool = False, **kwargs) -> Tuple:
+        """Candidates -> collision flags -> dp_search (planners.py:191-292).  With `search_details` a sixth element
+        (memo [k, T], costs [k, T]) of the search follows."""
         existing_q_data = kwargs.get("rerun_data")
         t0 = time()
         k = self._cfg.k if existing_q_data is None else DEFAULT_RERUN_NEW_K
         qs = self._candidates(problem, k)  # [k, T, ndof]
         time_ikflow = time() - t0
         if self._cfg.return_only_1st_plan:
-            return qs[0], False, TimingData(-1, time_ikflow, 0.0, 0.0, 0.0, 0.0), {}, (qs[0], None, None)
+            first = (qs[0], False, TimingData(-1, time_ikflow, 0.0, 0.0, 0.0, 0.0), {}, (qs[0], None, None))
+            return first + (None,) if search_details else first
 
         t0 = time()
         k_current = qs.shape[0]
@@ -393,10 +395,13 @@ class Planner:
         time_coll = time() - t0
 
         t0 = time()
-        qpath_search = dp_search(self.robot, qs, self_v, env_v, verbosity=0)
+        qpath_search, memo, costs, _ = dp_search(self.robot, qs, self_v, env_v, verbosity=0, return_details=True)
         q_data = (qs, self_v, env_v)
         time_dp = time() - t0
-        return qpath_search, False, TimingData(-1, time_ikflow, time_coll, 0.0, time_dp, 0.0), {}, q_data
+        td = TimingData(-1, time_ikflow, time_coll, 0.0, time_dp, 0.0)
+        if search_details:
+            return qpath_search, False, td, {}, q_data, (memo, costs)
+        return qpath_search, False, td, {}, q_data
 
     def generate_plan(self, problem: Problem, **kwargs) -> PlannerResult:
         raise NotImplementedError()
@@ -415,12 +420,44 @@ class PlannerSearcher(Planner):
 
 
 class CppFlowPlanner(Planner):
-    """dp_search followed by LM optimisation (planners.py:339-468)."""
+    """dp_search followed by LM optimisation (planners.py:339-468).
+
+    `lm_seeds` = N > 1 refines the DP's best paths to its N cheapest terminals (ordered by final cost, then candidate
+    index; seed 0 is dp_search's own path) together in the batched LM loop, with the step budget of one refinement,
+    and returns the lowest-index valid seed's plan, seed 0's when none is valid.  A valid seed 0 gives the plan of
+    lm_seeds = 1.  debug_info["lm_seed_index"] names the seed used."""
+
+    def __init__(self, settings: PlannerSettings, robot, candidate_generator: Optional[CandidateGenerator] = None,
+                 lm_seeds: int = 1):
+        super().__init__(settings, robot, candidate_generator)
+        if int(lm_seeds) < 1:
+            raise ValueError(f"lm_seeds must be >= 1, is {lm_seeds}")
+        self._lm_seeds = int(lm_seeds)
+
+    @property
+    def lm_seeds(self) -> int:
+        return self._lm_seeds
+
+    def _search_seeds(self, q_data, search) -> torch.Tensor:
+        """[n, T, ndof]: the DP's best paths ending at its n = min(lm_seeds, k) cheapest terminals, in the order
+        (costs[:, T-1], index) - row 0 is dp_search's path, bit for bit."""
+        qs = q_data[0]
+        memo, costs = search
+        k, T = costs.shape
+        last = costs[:, T - 1]
+        # stable sort on the cost: ties keep the lower candidate index first, as dp_search's argmin does
+        order = torch.sort(last, stable=True).indices[: min(self._lm_seeds, k)]
+        return ops.dp_backtrack(qs.contiguous(), memo, order.to(torch.int32))
 
     def generate_plan(self, problem: Problem, **kwargs) -> PlannerResult:
         t0 = kwargs.get("t0", time())
         rerun_data = kwargs.get("rerun_data")
-        search_qpath, is_valid, td, debug_info, q_data = self._run_pipeline(problem, **kwargs)
+        search = None
+        if self._lm_seeds > 1:
+            search_qpath, is_valid, td, debug_info, q_data, search = self._run_pipeline(problem, search_details=True,
+                                                                                        **kwargs)
+        else:
+            search_qpath, is_valid, td, debug_info, q_data = self._run_pipeline(problem, **kwargs)
 
         def time_is_exceeded():
             return time() - t0 > self._cfg.tmax_sec
@@ -436,7 +473,11 @@ class CppFlowPlanner(Planner):
             mjac_deg, mjac_cm = get_mjacs(problem.robot, search_qpath)
             if mjac_deg > self._cfg.rerun_mjac_threshold_deg or mjac_cm > self._cfg.rerun_mjac_threshold_cm:
                 kwargs["rerun_data"] = q_data
-                search_qpath, is_valid, td, debug_info, q_data = self._run_pipeline(problem, **kwargs)
+                if self._lm_seeds > 1:
+                    search_qpath, is_valid, td, debug_info, q_data, search = self._run_pipeline(
+                        problem, search_details=True, **kwargs)
+                else:
+                    search_qpath, is_valid, td, debug_info, q_data = self._run_pipeline(problem, **kwargs)
         if time_is_exceeded():
             return return_(search_qpath)
         if (not self._cfg.anytime_mode_enabled) and is_valid:
@@ -444,14 +485,18 @@ class CppFlowPlanner(Planner):
 
         t0_opt = time()
         if self._cfg.anytime_mode_enabled:
-            result = run_lm_optimization(problem, search_qpath, max_n_steps=75, tmax_sec=self._cfg.tmax_sec - (time() - t0),
-                                         return_if_valid_after_n_steps=int(1e8),
-                                         convergence_threshold=OPTIMIZATION_CONVERGENCE_THRESHOLD,
-                                         verbosity=self._cfg.verbosity)
+            lm_kw = dict(max_n_steps=75, return_if_valid_after_n_steps=int(1e8),
+                         convergence_threshold=OPTIMIZATION_CONVERGENCE_THRESHOLD)
         else:
-            result = run_lm_optimization(problem, search_qpath, max_n_steps=20, tmax_sec=self._cfg.tmax_sec - (time() - t0),
-                                         return_if_valid_after_n_steps=0, convergence_threshold=1e6,
-                                         verbosity=self._cfg.verbosity)
+            lm_kw = dict(max_n_steps=20, return_if_valid_after_n_steps=0, convergence_threshold=1e6)
+        if search is None:
+            result = run_lm_optimization(problem, search_qpath, tmax_sec=self._cfg.tmax_sec - (time() - t0),
+                                         verbosity=self._cfg.verbosity, **lm_kw)
+        else:
+            seeds = self._search_seeds(q_data, search)
+            results = run_lm_optimization_batched(problem, seeds, tmax_sec=self._cfg.tmax_sec - (time() - t0), **lm_kw)
+            result = next((r for r in results if r.is_valid), results[0])
+            debug_info["lm_seed_index"] = result.parallel_seed_idx
         td.optimizer = time() - t0_opt
         debug_info["n_optimization_steps"] = result.n_steps_taken
         if result.is_valid:
@@ -495,8 +540,8 @@ def plan_many(planner_factory: Callable[[Problem], Planner], problems):
       3. the alternating LM loops of all problems advance in lock step inside the library
          (cppflow_lm_alternating_loss_many: the next step of every unfinished loop is enqueued before the host waits);
       4. the plan reports.
-    Results equal those of one `generate_plan` call per problem.  Planners with a rerun option or
-    `return_only_1st_plan` set (and non-CppFlowPlanner planners) are run one after the other instead.
+    Results equal those of one `generate_plan` call per problem.  Planners with a rerun option,
+    `return_only_1st_plan` or lm_seeds > 1 set (and non-CppFlowPlanner planners) are run one after the other instead.
     (Host threads do not help here: the stages are Python-bound and serialise on the GIL - 13 threads were 1.5x slower
     than the sequential loop.)  -> list of PlannerResult in order."""
     from .optimization import run_lm_optimization_many
@@ -505,7 +550,7 @@ def plan_many(planner_factory: Callable[[Problem], Planner], problems):
     planners = [planner_factory(p) for p in problems]
     if not problems:
         return []
-    batchable = all(isinstance(pl, CppFlowPlanner) and not pl._cfg.return_only_1st_plan
+    batchable = all(isinstance(pl, CppFlowPlanner) and pl.lm_seeds == 1 and not pl._cfg.return_only_1st_plan
                     and not pl._cfg.do_rerun_if_large_dp_search_mjac and not pl._cfg.do_rerun_if_optimization_fails
                     and pl._cfg.anytime_mode_enabled == planners[0]._cfg.anytime_mode_enabled for pl in planners)
     if not batchable:

@@ -236,6 +236,26 @@ typedef struct cppflow_lm_loop_job {
 } cppflow_lm_loop_job;
 int cppflow_lm_alternating_loss_many(int n_jobs, const cppflow_lm_loop_job* jobs);
 
+/* The same loop for n_seeds seed paths d_x_seeds [n_seeds, T, ndof] of ONE problem, with the per-seed state on the
+ * device: each kernel launch of an iteration covers every unfinished seed (pose-only steps in one clustered launch,
+ * differencing steps gathered into one cppflow_lm_full_step), a decision kernel takes every seed's decisions and
+ * compacts the unfinished seeds into the next iteration's lists, and the host reads 3 integers per iteration into
+ * `h_pinned` (CPPFLOW_LM_BATCHED_PINNED_BYTES of page-locked memory; polled tag, stream synchronisation as fallback),
+ * whatever n_seeds is.  Seed i's d_x_out row, decisions and results[i] are bit for bit those of
+ * cppflow_lm_alternating_loss on that seed alone, except last_metrics[7] (no metric: 0 here, the single loop's
+ * completion tag there); the time limit tmax_sec is checked once per iteration for all seeds.  BLOCKS like cppflow_lm_alternating_loss.  d_x_out [n_seeds, T, ndof]; results [n_seeds].
+ * Workspace: cppflow_lm_alternating_batched_workspace_bytes(robot, n_seeds, T) bytes, 256-byte aligned.
+ * n_seeds == 0 returns at once. */
+#define CPPFLOW_LM_BATCHED_PINNED_BYTES 64
+size_t cppflow_lm_alternating_batched_workspace_bytes(int robot, int64_t n_seeds, int64_t T);
+int cppflow_lm_alternating_loss_batched(int robot, const cppflow_lm_params* params_diff,
+                                        const cppflow_lm_params* params_pose, const cppflow_constraints* constraints,
+                                        const float* d_x_seeds, const float* d_target, int64_t n_seeds, int64_t T,
+                                        const float* h_cuboids, const float* h_Tcuboids, int n_obstacles, int max_n_steps,
+                                        double tmax_sec, int return_if_valid_after_n_steps, double convergence_threshold,
+                                        void* d_workspace, size_t workspace_bytes, int32_t* h_pinned, float* d_x_out,
+                                        cppflow_lm_loop_result* results, void* stream);
+
 /* joint_limit_almost_violations_3d(robot, qs, eps_revolute, eps_prismatic) -> float32 0/1 [n]  (search.py:25-52) */
 int cppflow_joint_limit_flags(int robot, const float* d_q, int64_t n, float eps_revolute, float eps_prismatic,
                               float* d_flags, void* stream);
@@ -248,6 +268,12 @@ size_t cppflow_dp_search_workspace_bytes(int64_t k, int64_t T);
 int cppflow_dp_search(int robot, const float* d_q, const uint8_t* d_self_flags, const uint8_t* d_env_flags, int64_t k,
                       int64_t T, void* d_workspace, size_t workspace_bytes, float* d_best_path, int32_t* d_memo,
                       float* d_costs, int32_t* d_chosen, void* stream);
+
+/* The backtrack of dp_search (search.py:162-173) from n chosen terminals: path j of d_out [n, T, ndof] ends at
+ * candidate d_terminals[j] and follows d_memo [k, T] (cppflow_dp_search's output) back to t = 0; waypoint t is
+ * d_q [k, T, ndof] row (chosen candidate, t).  The terminal argmin of the last cost column gives dp_search's path. */
+int cppflow_dp_backtrack(const float* d_q, const int32_t* d_memo, int64_t k, int64_t T, int ndof,
+                         const int32_t* d_terminals, int64_t n, float* d_out, void* stream);
 
 /* Per-path validity metrics (x_is_valid without the klampt calls: optimization_utils.py:836-886,
  * evaluation_utils.py:29-75,113-141; TL of optimization.py:173-175).  d_out [P,8] =

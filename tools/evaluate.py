@@ -8,13 +8,14 @@ visualisation, no results directory).
     python tools/evaluate.py --problem_file my_problem.yaml            # a problem yaml in the reference's layout
     python tools/evaluate.py --all --ikflow_checkpoint panda_sd.pt     # candidates from a trained IKFlow
     python tools/evaluate.py --all --ikflow_checkpoint panda_sd.pt --ikflow_refine   # ... refined by LM IK
+    python tools/evaluate.py --all --lm_seeds 16       # refine the DP's 16 best paths together, keep the first valid
 
 --ikflow_checkpoint takes a GraphINN state dict (tools/train_ikflow.py --state_dict, or an IKFlow checkpoint's); the
 planner then draws its candidates with IkflowCandidateGenerator.  The network's shape is read from the state dict,
 and problems of robots whose joint scale differs from the state dict's are skipped.  --ikflow_refine passes the
 flow's candidates through the per-waypoint LM refinement (IkRefineSettings: the 20-step damping schedule of
 LmIkCandidateGenerator, stopping at 0.1 mm / 0.1 deg); waypoints that do not converge count as violations in
-dp_search.
+dp_search.  --lm_seeds N (CppFlow only) refines the DP's best paths to its N cheapest terminals in the batched LM loop.
 
 Errors come from plan_from_qpath (FK of the returned path against the target path); the validity flag is the
 capsule-model one (the reference's klampt mesh check is out of scope)."""
@@ -40,9 +41,10 @@ CONSTRAINTS = Constraints(max_allowed_position_error_cm=0.01, max_allowed_rotati
                           max_allowed_mjac_cm=2.0)  # scripts/evaluate.py:51-56
 
 
-def evaluate(planner_name: str, problem, settings: PlannerSettings, warmup: bool = True, generator=None):
-    planner = (PLANNERS[planner_name](settings, problem.robot) if generator is None else
-               PLANNERS[planner_name](settings, problem.robot, generator))
+def evaluate(planner_name: str, problem, settings: PlannerSettings, warmup: bool = True, generator=None, lm_seeds: int = 1):
+    extra = {} if lm_seeds == 1 else {"lm_seeds": lm_seeds}
+    planner = (PLANNERS[planner_name](settings, problem.robot, **extra) if generator is None else
+               PLANNERS[planner_name](settings, problem.robot, generator, **extra))
     if warmup:
         planner.generate_plan(problem)  # first call: kernel attributes, workspaces
     torch.cuda.synchronize()
@@ -70,7 +72,13 @@ def main(argv=None):
     ap.add_argument("--no_warmup", action="store_true")
     ap.add_argument("--ikflow_checkpoint", default=None, help="GraphINN state dict: plan with IkflowCandidateGenerator")
     ap.add_argument("--ikflow_refine", action="store_true", help="LM-refine the IKFlow candidates (IkRefineSettings)")
+    ap.add_argument("--lm_seeds", type=int, default=1,
+                    help="CppFlow: refine the DP's best paths to its N cheapest terminals together (batched LM loop)")
     args = ap.parse_args(argv)
+    if args.lm_seeds < 1:
+        ap.error("--lm_seeds must be >= 1")
+    if args.lm_seeds > 1 and args.planner != "CppFlow":
+        ap.error("--lm_seeds needs --planner CppFlow")
     if args.ikflow_checkpoint and args.planner != "CppFlow":
         ap.error("--ikflow_checkpoint needs --planner CppFlow")
     if args.ikflow_refine and not args.ikflow_checkpoint:
@@ -100,7 +108,8 @@ def main(argv=None):
                 solvers[rob.name] = IkflowSolver(rob, params_from_state_dict(sd), state_dict=sd, device=args.device)
             generator = IkflowCandidateGenerator(solvers[rob.name], seed=0, refine=refine)
         try:
-            row, ok = evaluate(args.planner, problem, settings, warmup=not args.no_warmup, generator=generator)
+            row, ok = evaluate(args.planner, problem, settings, warmup=not args.no_warmup, generator=generator,
+                               lm_seeds=args.lm_seeds)
         except AssertionError as e:  # the reference's checks on the candidates, e.g. "too many env collisions"
             print(f"{problem.full_name}: the planner stopped: {e}")
             failed.append(problem.full_name)
